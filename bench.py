@@ -2,6 +2,7 @@
 """bench.py — frames/s of the Video-Depth-Anything hot path (BASELINE.json metric) on N B200s.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--encoder vitl] [--dtype bf16]
+                    [--dump-outputs DIR]
 
 A "step" is one forward pass of one 1x32x518x518 window (BASELINE.json configs[1]) per GPU.  N>1 is launched by
 torchrun (one rank per GPU, NCCL); windows are independent in model compute (SURVEY.md §3.2), so ranks process
@@ -17,6 +18,13 @@ Printed JSON (rank 0, one line):
   cpu_baseline the oracle port (oracle/vda_oracle.py, torch fp32 on the host cores) on a bounded sample
 `--impl reference` times that CPU port alone (the reference itself is Python/PyTorch on CPU; /root/reference does
 not exist on the GPU box, the oracle is its pinned restatement).
+
+`--dump-outputs DIR` (GPU arm, rank 0) writes what the timed calls returned in their last step, so that two builds can be
+compared output for output on the same seeded inputs (weights and inputs depend on the arguments only):
+  depth.npy        the whole float32 [1, 32, 518, 518] depth map of the last timed window (34 MB)
+  video_depth.npy  8 frames of the long-video result, picked with a fixed seed, in frame order: float32 [8, 518, 518]
+                   (9 MB; every frame of a video shorter than 8 frames; absent with --video-frames 0, and with a
+                   note on stderr if that arm failed)
 """
 from __future__ import annotations
 
@@ -163,7 +171,13 @@ def main():
     ap.add_argument("--no-other-configs", dest="other_configs", action="store_false",
                     help="skip the BASELINE configs[3]/[4] arms (metric 518x924, vits clips)")
     ap.add_argument("--profile-out", default=None, help="write the per-kernel-family time table (JSON) here")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="write the outputs of the last timed step as DIR/<name>.npy (GPU arm only)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to the GPU arm (--impl ours)")
     if args.impl == "reference":
         return run_reference(args)
 
@@ -215,6 +229,9 @@ def main():
         ev[i][1].record()
     t_end.record()
     barrier()
+    dumps = {}
+    if args.dump_outputs and rank == 0:    # the last timed step's depth map
+        dumps["depth"] = d.float().cpu().numpy()
     launches = ops.LAUNCHES - launches0
     clocks = sampler.stop() if sampler else None
     step_ms = [a.elapsed_time(b) for a, b in ev]
@@ -391,6 +408,9 @@ def main():
             # the result is bit-reproducible across GPU counts (fixed-order reductions, batch-invariant kernels): the
             # CRC of the depth bytes must be the same number in the N = 1, 2, 4, 8 lines (computed after the timed region)
             crc = zlib.crc32(memoryview(np.ascontiguousarray(depths)).cast("B")) & 0xFFFFFFFF
+            if args.dump_outputs:
+                pick = np.random.default_rng(0).choice(args.video_frames, min(8, args.video_frames), replace=False)
+                dumps["video_depth"] = np.ascontiguousarray(depths[np.sort(pick)], dtype=np.float32)
             return {"workload": f"{args.encoder} {args.video_frames}x518x518 uint8 video, 32-frame windows, overlap 10, "
                                  f"host frames -> host depths (upload, device preprocessing, feature reuse, alignment, "
                                  f"download all inside the timed region)",
@@ -427,10 +447,9 @@ def main():
                 for _ in range(3):
                     m2.forward(xx)
                 barrier()
-                k2 = max(3, min(K, 10))
                 a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
                 tsum = 0.0
-                for _ in range(k2):
+                for _ in range(K):
                     fl.zero_()
                     a.record()
                     dd = m2.forward(xx)
@@ -440,10 +459,10 @@ def main():
                 tt = torch.tensor([tsum], device=dev)
                 if world > 1:
                     dist.all_reduce(tt, op=dist.ReduceOp.MAX)
-                ms2 = tt.item() / k2
+                ms2 = tt.item() / K
                 tfl = {"metric924": 88.4, "vits8clips": ALGO_TFLOP_PER_WINDOW["vits"]}[name]
                 other[name] = {"workload": f"{enc}{' metric' if metric else ''} 1x32x{hh}x{ww} clip per GPU per step x{world} GPUs",
-                               "frames_per_s": world * 32 / (ms2 * 1e-3), "ms_per_clip": ms2, "steps": k2, "dtype": args.dtype,
+                               "frames_per_s": world * 32 / (ms2 * 1e-3), "ms_per_clip": ms2, "steps": K, "dtype": args.dtype,
                                "tflops_algorithmic_per_gpu": tfl / (ms2 * 1e-3), "timing": "CUDA events, max over ranks, L2 flushed"}
                 assert (dd > 0).float().mean().item() > 0.99
                 m2 = xx = fl = dd = None
@@ -491,6 +510,15 @@ def main():
                                             tflops=v["flops"] / (v["ms"] * 1e-3) / 1e12 if v["ms"] > 0 else 0)
                                        for k, v in sorted(shapes.items(), key=lambda kv: -kv[1]["ms"])],
                        "step_ms": step_ms, "eager_profiled_step_ms": prof_step_ms}, open(args.profile_out, "w"), indent=1)
+        if args.dump_outputs:
+            import numpy as np
+            assert sum(a.nbytes for a in dumps.values()) <= 64 << 20
+            os.makedirs(args.dump_outputs, exist_ok=True)
+            for name, a in dumps.items():
+                np.save(os.path.join(args.dump_outputs, name + ".npy"), a)
+            if args.video_frames > 0 and "video_depth" not in dumps:
+                print(f"bench.py: {os.path.join(args.dump_outputs, 'video_depth.npy')} not written: the long-video arm "
+                      f"failed ({(video or {}).get('error')})", file=sys.stderr, flush=True)
     if world > 1:
         dist.destroy_process_group()
 

@@ -60,6 +60,15 @@ def import_reference():
     return MetricVDA, metric_mod, top
 
 
+def ivd_frames() -> np.ndarray:
+    """The uint8 [50, 60, 80, 3] input video of the infer_video_depth golden cases, regenerated from its seed (the .npz
+    files store the reference's depths only): smooth-ish frames so the cubic resize is exercised on non-noise data too."""
+    rng = np.random.default_rng(0)
+    base = rng.integers(0, 256, (50, 15, 20, 3), dtype=np.uint8)
+    frames = np.repeat(np.repeat(base, 4, axis=1), 4, axis=2)
+    return (frames.astype(np.int32) + rng.integers(-20, 20, frames.shape)).clip(0, 255).astype(np.uint8)
+
+
 def build_ref(MetricVDA, enc, sd):
     from video_depth_anything_b200.synth import MODEL_CONFIGS
     m = MetricVDA(**MODEL_CONFIGS[enc]).eval()
@@ -77,14 +86,14 @@ def main():
     manifest = {"generator": "oracle/make_golden.py", "torch": torch.__version__, "cases": {}}
 
     fwd_cases = [
-        # name, encoder, seed, x shape, x seed, store stride
-        ("fwd_vits_T8_56x70", "vits", 0, (1, 8, 3, 56, 70), 1234, 1),
-        ("fwd_vits_T32_42x42", "vits", 1, (1, 32, 3, 42, 42), 1235, 1),
-        ("fwd_vitl_T4_28x42", "vitl", 0, (1, 4, 3, 28, 42), 1236, 1),
-        ("fwd_vits_T2_518x518", "vits", 0, (1, 2, 3, 518, 518), 1237, 2),
+        # name, encoder, seed, x shape, x seed, depth store stride, tap token stride (keeps every file under 1 MB)
+        ("fwd_vits_T8_56x70", "vits", 0, (1, 8, 3, 56, 70), 1234, 1, 8),
+        ("fwd_vits_T32_42x42", "vits", 1, (1, 32, 3, 42, 42), 1235, 1, 8),
+        ("fwd_vitl_T4_28x42", "vitl", 0, (1, 4, 3, 28, 42), 1236, 1, 8),
+        ("fwd_vits_T2_518x518", "vits", 0, (1, 2, 3, 518, 518), 1237, 2, 64),
     ]
     models = {}
-    for name, enc, seed, shape, xseed, stride in fwd_cases:
+    for name, enc, seed, shape, xseed, stride, tap_stride in fwd_cases:
         sd = synth_state_dict(**MODEL_CONFIGS[enc], seed=seed)
         ref = build_ref(MetricVDA, enc, sd)
         models[(enc, seed)] = (sd, ref)
@@ -108,21 +117,17 @@ def main():
               f"std {d_ref.std():.4f}; ref time {t_ref:.1f}s")
         assert diff < 5e-5, name
         assert frac_pos > 0.99, name
-        taps = {f"tap{i}": stages[f"tap{i}"][:, ::max(1, stride * 8)].numpy().astype(np.float32) for i in range(4)}
+        taps = {f"tap{i}": stages[f"tap{i}"][:, ::tap_stride].numpy().astype(np.float32) for i in range(4)}
         np.savez_compressed(os.path.join(GOLD, name + ".npz"),
                             depth=d_ref.numpy()[..., ::stride, ::stride].astype(np.float32), **taps)
         manifest["cases"][name] = dict(kind="forward", encoder=enc, seed=seed, x_shape=list(shape), x_seed=xseed,
-                                       stride=stride, tap_stride=max(1, stride * 8),
+                                       stride=stride, tap_stride=tap_stride,
                                        oracle_vs_ref_max_abs=diff, oracle_vs_ref_rel=rel,
                                        perm_sensitivity=sens, frac_positive=frac_pos)
 
     # ---- infer_video_depth: top-level (affine) and metric (identity) drivers ----
     sd, ref = models[("vits", 0)]
-    rng = np.random.default_rng(0)
-    # smooth-ish frames so the cubic resize is exercised on non-noise data too
-    base = rng.integers(0, 256, (50, 15, 20, 3), dtype=np.uint8)
-    frames = np.repeat(np.repeat(base, 4, axis=1), 4, axis=2)
-    frames = (frames.astype(np.int32) + rng.integers(-20, 20, frames.shape)).clip(0, 255).astype(np.uint8)
+    frames = ivd_frames()
     for name, mod, mode in (("ivd_affine_vits_50x60x80", top, "affine"),
                             ("ivd_identity_vits_50x60x80", metric_mod, "identity")):
         fn = mod.VideoDepthAnything.infer_video_depth
@@ -133,7 +138,7 @@ def main():
         diff = float(np.abs(d_or - d_ref).max())
         print(f"{name}: oracle-vs-ref max abs {diff:.3e}; out {d_ref.shape} mean {d_ref.mean():.4f}; ref {t_ref:.1f}s")
         assert diff < 5e-5, name
-        np.savez_compressed(os.path.join(GOLD, name + ".npz"), depth=d_ref.astype(np.float32), frames=frames)
+        np.savez_compressed(os.path.join(GOLD, name + ".npz"), depth=d_ref.astype(np.float32))
         manifest["cases"][name] = dict(kind="infer_video_depth", encoder="vits", seed=0, mode=mode, input_size=56,
                                        n_frames=50, oracle_vs_ref_max_abs=diff)
 

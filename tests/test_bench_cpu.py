@@ -5,6 +5,8 @@ import os
 import subprocess
 import sys
 
+import pytest
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
@@ -38,6 +40,13 @@ def test_reference_arm_sample_fits_the_budget_and_config_matches_the_gpu_arm():
     # the driver compares the two arms' config objects
     assert bench.workload_config("vitl", 4) == bench.workload_config("vitl", 4)
     assert "1x32x518x518" in bench.workload_config("vitl", 1)["workload"]
+
+
+@pytest.mark.parametrize("args", [["--steps", "0"], ["--impl", "reference", "--dump-outputs", "out"]])
+def test_bad_arguments_are_refused(args):
+    out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), *args], capture_output=True, text=True,
+                         timeout=120, env={**os.environ, "CUDA_VISIBLE_DEVICES": ""})
+    assert out.returncode == 2 and out.stdout == "", out.stderr[-2000:]
 
 
 def test_reference_arm_honours_steps_and_warmup():

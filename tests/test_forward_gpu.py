@@ -14,6 +14,7 @@ pytestmark = pytest.mark.gpu
 
 from e2e_checks import GOLD, build_model, golden_case, stage_report  # noqa: E402
 from oracle import vda_oracle as O  # noqa: E402
+from oracle.make_golden import ivd_frames  # noqa: E402
 
 TOL = 1e-2           # north_star: per-pixel relative depth error, every advertised dtype, on the MAX (no percentile escape)
 TOL_VALIDATION = 1e-3   # north_star: fp32-accumulate validation mode (`fp32=True`)
@@ -42,7 +43,7 @@ def test_infer_video_depth_vs_reference_golden(name):
     g = np.load(os.path.join(GOLD, name + ".npz"))
     m, _ = build_model(c["encoder"], c["seed"], torch.float16)
     m.metric = c["mode"] == "identity"
-    out, fps = m.infer_video_depth(g["frames"], 24, input_size=c["input_size"], device="cuda")
+    out, fps = m.infer_video_depth(ivd_frames(), 24, input_size=c["input_size"], device="cuda")
     assert fps == 24 and out.shape == g["depth"].shape and out.dtype == np.float32
     mx, p999, mean = O.rel_err(torch.from_numpy(out), torch.from_numpy(g["depth"]))
     assert mx <= TOL, f"{name}: rel err max {mx:.3e} p99.9 {p999:.3e} mean {mean:.3e}"
@@ -135,11 +136,11 @@ def test_sharded_driver_single_process_equals_plain():
     from video_depth_anything_b200.parallel import infer_video_depth_sharded
     name = IVD[0]
     c = MAN[name]
-    g = np.load(os.path.join(GOLD, name + ".npz"))
     m, _ = build_model(c["encoder"], c["seed"], torch.float16)
     m.metric = c["mode"] == "identity"
-    a, _ = m.infer_video_depth(g["frames"], 24, input_size=c["input_size"], device="cuda")
-    b, _ = infer_video_depth_sharded(m, g["frames"], 24, input_size=c["input_size"])
+    frames = ivd_frames()
+    a, _ = m.infer_video_depth(frames, 24, input_size=c["input_size"], device="cuda")
+    b, _ = infer_video_depth_sharded(m, frames, 24, input_size=c["input_size"])
     assert np.array_equal(a, b)
 
 

@@ -472,7 +472,10 @@ class Engine:
             launches = ops.LAUNCHES - n0
             torch.cuda.current_stream().synchronize()
             graph = torch.cuda.CUDAGraph()
-            with torch.cuda.graph(graph):
+            # thread-local capture: the video driver's drain thread waits on copy-stream events (cudaEventSynchronize)
+            # while a window's graph may be captured; in the default global mode that call from another thread
+            # invalidates the capture, although it never touches the capturing stream
+            with torch.cuda.graph(graph, capture_error_mode="thread_local"):
                 static_out = fn(*static_in)
             entry = self._graphs[key] = (graph, static_in, static_out, launches)
         graph, static_in, static_out, launches = entry
