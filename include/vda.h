@@ -144,6 +144,21 @@ int vda_attention_spatial(const void* qkv, void* out, int frames, int N, int hea
  * [q | k | v], each split in `heads` heads of C/heads.  out: h16 [T*hw, C]. */
 int vda_attention_temporal(const void* qkv, void* out, int T, int hw, int C, int heads, int dtype, void* stream);
 
+/* Streaming temporal attention: the current frame's query against the cached frames of the stream and itself.
+ *   qkv:   h16 [hw, 3*C], the current frame's q'|k'|v' (the q|k|v Linear applied to the LayerNorm output WITHOUT the
+ *          positional encoding);
+ *   cache: h16 [slots, hw, 2*C], per slot and position the row k'|v' of an earlier frame;
+ *   pe:    fp32 [32, 3*C], pe[p] @ [W_q | W_k | W_v]^T, the positional encoding's share of q|k|v at position p;
+ *   ctx:   device int32 [2 + n_ctx] = {n_ctx, write_slot, slot of context position 0, ..., n_ctx - 1}, n_ctx <= 31
+ *          (larger values are clamped to 31, slot indices to slots - 1).
+ * Keys / values are the n_ctx cached rows (position p: k' + pe_k[p], v' + pe_v[p]) followed by the current frame at
+ * position n_ctx, whose query is q' + pe_q[n_ctx]; out: h16 [hw, C] = softmax(q k^T / sqrt(C/heads)) v per head, fp32
+ * inside.  The current frame's k'|v' rows are also copied, unchanged, into slot `write_slot` of the cache, which must
+ * not be one of the slots read.  Everything that changes from step to step is in `ctx`, so a captured CUDA graph
+ * replays it. */
+int vda_attention_temporal_step(const void* qkv, void* cache, const float* pe, const int32_t* ctx, void* out, int hw,
+                                int C, int heads, int slots, int dtype, void* stream);
+
 /* Frame preprocessing of infer_video_depth (video_depth.py:173-185,197-198; util/transform.py:109-158): for every
  * i < n, frame idx[i] of the device-resident uint8 RGB video frames [*, H0, W0, 3] -> /255 -> cv2-style INTER_CUBIC
  * resize to (nh, nw) -> (x - mean) / std (float64) -> out fp32 [n, 3, nh, nw].  idx: device int32 [n]. */

@@ -1,0 +1,149 @@
+#!/usr/bin/env python
+"""Streaming inference on one GPU (VideoDepthAnything.stream / DepthStream.push); prints one JSON line and writes it to
+--out.
+
+Per config (vits 518x518, vitl 518x518, vitl 518x924 = a 1280x720 video, the metric config):
+  * push latency p50 / p99: host clock around `push` (H2D of the frame, graph replay, D2H of the depth, synchronised),
+    400 frames after 40 warm-up frames, so the context has been sliding for 8 frames before the first timed one;
+  * step device time p50 / p99: CUDA events around a replay of the step graph alone;
+  * the windowed forward of the same model (one 32-frame window, CUDA events) in frames/s, for comparison.
+Then the step kernel alone at every block shape of the configs with a full context (31 cached frames, 32 slots):
+median time over launches with the L2 overwritten in between, the bytes it must move (computed from shapes) over that
+time, and that rate's share of the HBM bound (7.7 TB/s, the HGX B200 data sheet's per-GPU figure).
+The card's name and power limit are read in the same run."""
+import argparse
+import json
+import os
+import subprocess
+import sys
+import time
+
+import numpy as np
+import torch
+
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, ROOT)
+from video_depth_anything_b200 import MODEL_CONFIGS, VideoDepthAnything, ops, synth_state_dict  # noqa: E402
+from video_depth_anything_b200.windows import get_resize_hw  # noqa: E402
+
+HBM_BYTES_PER_S = 7.7e12
+CONFIGS = [("vits", 518, 518), ("vitl", 518, 518), ("vitl", 720, 1280)]
+
+
+def card():
+    q = subprocess.run(["nvidia-smi", "--id=0", "--query-gpu=name,power.limit", "--format=csv,noheader"],
+                       capture_output=True, text=True, timeout=30).stdout.strip()
+    return {"card": q.split(",")[0].strip() if q else torch.cuda.get_device_name(0),
+            "power_limit": q.split(",")[1].strip() if "," in q else "unknown"}
+
+
+def pct(xs, p):
+    return float(np.percentile(np.asarray(xs), p))
+
+
+def model(enc, dtype):
+    m = VideoDepthAnything(**MODEL_CONFIGS[enc], dtype=dtype)
+    m.load_state_dict(synth_state_dict(**MODEL_CONFIGS[enc], seed=0))
+    return m.to("cuda")
+
+
+def bench_config(enc, h0, w0, warmup, frames, dtype):
+    m = model(enc, dtype)
+    pool = np.random.default_rng(0).integers(0, 256, (16, h0, w0, 3), dtype=np.uint8)
+    st = m.stream()
+    for t in range(warmup):
+        st.push(pool[t % 16])
+    host = []
+    for t in range(frames):
+        f = pool[t % 16]
+        t0 = time.perf_counter()
+        st.push(f)
+        host.append((time.perf_counter() - t0) * 1e3)
+    dev = []
+    for _ in range(100):                              # replays of the last step (idempotent: same inputs, same slot)
+        s, e = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+        s.record()
+        st.engine.stream_step_graphed(st.sid, st.frame_dev, st.ctx_dev, st.cache, st.nh, st.nw)
+        e.record()
+        e.synchronize()
+        dev.append(s.elapsed_time(e))
+    nh, nw = get_resize_hw(h0, w0)
+    x = torch.randn(1, 32, 3, nh, nw, device="cuda")
+    for _ in range(2):
+        m.forward(x)
+    win = []
+    for _ in range(5):
+        s, e = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+        s.record()
+        m.forward(x)
+        e.record()
+        e.synchronize()
+        win.append(s.elapsed_time(e))
+    eng = st.engine
+    hp, wp = nh // 14, nw // 14
+    shapes = [(c.shape[1], c.shape[2] // 2) for c in st.cache[::2]]   # (hw, C) of motion modules 0..3
+    launches = eng._graphs[("stream", st.sid, st.nh, st.nw, h0, w0, 3)][3]
+    st.close()
+    del st, m
+    torch.cuda.empty_cache()
+    return {"encoder": enc, "frame": [h0, w0], "network": [nh, nw], "dtype": str(dtype).split(".")[-1],
+            "push_ms_p50": round(pct(host, 50), 3), "push_ms_p99": round(pct(host, 99), 3),
+            "step_device_ms_p50": round(pct(dev, 50), 3), "step_device_ms_p99": round(pct(dev, 99), 3),
+            "push_fps_p50": round(1e3 / pct(host, 50), 1), "launches_per_step": launches,
+            "window_forward_ms": round(pct(win, 50), 2), "window_forward_fps": round(32e3 / pct(win, 50), 1),
+            "grid": [hp, wp]}, shapes
+
+
+def bench_kernel(hw, C, dtype, iters=30):
+    slots, n = 32, 31
+    g = torch.Generator(device="cuda").manual_seed(0)
+    qkv = torch.randn(hw, 3 * C, device="cuda", generator=g).to(dtype)
+    cache = torch.randn(slots, hw, 2 * C, device="cuda", generator=g).to(dtype)
+    pe = torch.randn(32, 3 * C, device="cuda", generator=g)
+    ctx = torch.tensor([n, 31] + list(range(31)), dtype=torch.int32, device="cuda")
+    out = torch.empty(hw, C, dtype=dtype, device="cuda")
+    flush = torch.empty(512 << 20, dtype=torch.uint8, device="cuda")
+    ops.attention_temporal_step(qkv, cache, pe, ctx, out)
+    ts = []
+    for _ in range(iters):
+        flush.zero_()                                  # 512 MB written: the cache rows come from HBM, not the 126 MB L2
+        s, e = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+        s.record()
+        ops.attention_temporal_step(qkv, cache, pe, ctx, out)
+        e.record()
+        e.synchronize()
+        ts.append(s.elapsed_time(e))
+    ms = pct(ts, 50)
+    nbytes = 2 * hw * (n * 2 * C + 3 * C + C + 2 * C)   # cached k'|v' read, q'|k'|v' read, out + write-slot row written
+    gbs = nbytes / (ms * 1e-3) / 1e9
+    return {"hw": hw, "C": C, "head_dim": C // 8, "us": round(ms * 1e3, 2), "MB": round(nbytes / 1e6, 2),
+            "GB_s": round(gbs, 1), "hbm_share": round(gbs * 1e9 / HBM_BYTES_PER_S, 3)}
+
+
+def main():
+    ap = argparse.ArgumentParser()
+    ap.add_argument("--warmup", type=int, default=40)
+    ap.add_argument("--frames", type=int, default=400)
+    ap.add_argument("--out", default=os.path.join(ROOT, "profiles", "stream_b200.json"))
+    a = ap.parse_args()
+    if not torch.cuda.is_available():
+        sys.exit("bench_stream.py needs a GPU")
+    res = {"what": "streaming push latency / step device time / step kernel", **card(), "configs": [], "step_kernel": []}
+    seen = set()
+    for enc, h0, w0 in CONFIGS:
+        r, shapes = bench_config(enc, h0, w0, a.warmup, a.frames, torch.bfloat16)
+        res["configs"].append(r)
+        for mm, (hw, C) in enumerate(shapes):
+            if (hw, C) not in seen:
+                seen.add((hw, C))
+                res["step_kernel"].append({"config": f"{enc} {r['network'][0]}x{r['network'][1]} mm{mm}",
+                                           **bench_kernel(hw, C, torch.bfloat16)})
+    line = json.dumps(res)
+    print(line)
+    os.makedirs(os.path.dirname(os.path.abspath(a.out)), exist_ok=True)
+    with open(a.out, "w") as f:
+        f.write(line + "\n")
+
+
+if __name__ == "__main__":
+    main()

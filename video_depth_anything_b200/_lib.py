@@ -51,6 +51,8 @@ _SIGS = {
                                 C.c_int, C.c_void_p, C.c_int, C.c_void_p]),
     "vda_attention_spatial": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p]),
     "vda_attention_temporal": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p]),
+    "vda_attention_temporal_step": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int,
+                                              C.c_int, C.c_int, C.c_int, C.c_void_p]),
     "vda_preprocess_frames": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int,
                                         C.c_void_p]),
     "vda_copy_frames": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int64, C.c_void_p]),

@@ -237,9 +237,191 @@ static int dispatch_temporal(const void* qkv, void* out, int T_, int hw, int C, 
   return launch_temporal<T, 128>(qkv, out, T_, hw, C, heads, st);
 }
 
+// ---------------------------------------------------------------------------------------------
+// Streaming step: one new frame's query against <= 31 cached frames + itself (vda.h, vda_attention_temporal_step).
+//
+// One warp owns (head, PPT adjacent positions).  Lane = (key split ks, chunk c): c < G holds 16-byte chunk c of the
+// head's dh columns (G = dh/8 rounded up to a power of two, the extra lanes hold zeros), and the KS = 32/G key splits
+// take keys ks, ks + KS, ... of the sequence, so a lane walks at most 32/KS keys and a warp has all its loads in
+// flight at once (the kernel is HBM-bound: the cached K'|V' rows are the traffic).  Scores are reduced over the G
+// lanes of a split with xor shuffles; every split keeps an online softmax (fp32) and the splits are merged at the
+// end (max, rescale, sum).  The PE projections are added as each row is loaded; a PE row is shared by the PPT
+// positions of a warp, which halves its (L1/L2) traffic.
+// ---------------------------------------------------------------------------------------------
+template <typename T>
+__device__ __forceinline__ void unpack8(const uint4& u, float (&f)[8]) {
+  const uint32_t w[4] = {u.x, u.y, u.z, u.w};
+#pragma unroll
+  for (int e = 0; e < 4; ++e) {
+    const float2 p = H16<T>::unpack2(w[e]);
+    f[2 * e] = p.x;
+    f[2 * e + 1] = p.y;
+  }
+}
+
+__device__ __forceinline__ void load_pe8(const float* p, float (&f)[8]) {
+  const float4 a = __ldg(reinterpret_cast<const float4*>(p));
+  const float4 b = __ldg(reinterpret_cast<const float4*>(p) + 1);
+  f[0] = a.x, f[1] = a.y, f[2] = a.z, f[3] = a.w, f[4] = b.x, f[5] = b.y, f[6] = b.z, f[7] = b.w;
+}
+
+template <typename T, int G, int PPT>
+__global__ void __launch_bounds__(256)
+temporal_step_kernel(const T* __restrict__ qkv, T* __restrict__ cache, const float* __restrict__ pe,
+                     const int32_t* __restrict__ ctx, T* __restrict__ out, int hw, int C, int heads, int slots) {
+  constexpr int KS = 32 / G;
+  const long long warp = (static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x) >> 5;
+  const int lane = threadIdx.x & 31, c = lane % G, ks = lane / G;
+  const int dh = C / heads;
+  const int h = static_cast<int>(warp % heads);
+  const long long p0 = warp / heads * PPT;          // (no early exit for p0 >= hw: the shuffles need the whole warp)
+  const bool act = c * 8 < dh;                       // lane holds a real chunk of the head
+  const int col = act ? h * dh + c * 8 : h * dh;
+  const int n = min(max(__ldg(ctx), 0), 31);
+  const int ws = min(max(__ldg(ctx + 1), 0), slots - 1);
+  const float sc = rsqrtf(static_cast<float>(dh)) * 1.4426950408889634f;
+  const long long row2 = 2LL * C;
+
+  float q[PPT][8], o[PPT][8], m[PPT], l[PPT];
+  {
+    float pq[8];
+    load_pe8(pe + static_cast<long long>(n) * 3 * C + col, pq);
+#pragma unroll
+    for (int i = 0; i < PPT; ++i) {
+      const long long pos = p0 + i;
+      uint4 uq = make_uint4(0, 0, 0, 0);
+      if (act && pos < hw) {
+        const T* r = qkv + pos * 3 * C + col;
+        uq = __ldg(reinterpret_cast<const uint4*>(r));
+        if (ks == 0) {                               // the current frame's k'|v' go to the write slot unchanged
+          T* w = cache + (static_cast<long long>(ws) * hw + pos) * row2 + col;
+          *reinterpret_cast<uint4*>(w) = __ldg(reinterpret_cast<const uint4*>(r + C));
+          *reinterpret_cast<uint4*>(w + C) = __ldg(reinterpret_cast<const uint4*>(r + 2 * C));
+        }
+      }
+      float fq[8];
+      unpack8<T>(uq, fq);
+#pragma unroll
+      for (int e = 0; e < 8; ++e) {
+        q[i][e] = act ? (fq[e] + pq[e]) * sc : 0.f;
+        o[i][e] = 0.f;
+      }
+      m[i] = -INFINITY;
+      l[i] = 0.f;
+    }
+  }
+  // ---- keys ks, ks + KS, ... of the sequence: context positions 0..n-1 (cache), then the current frame (position n) ----
+#pragma unroll 2
+  for (int jb = 0; jb <= n; jb += KS) {             // (warp-uniform trip count: the shuffles need every lane)
+    const int j = min(jb + ks, n);
+    const bool valid = jb + ks <= n, cur = j == n;
+    const int slot = cur ? 0 : min(max(__ldg(ctx + 2 + j), 0), slots - 1);
+    float pk[8], pv[8];
+    load_pe8(pe + static_cast<long long>(j) * 3 * C + C + col, pk);
+    load_pe8(pe + static_cast<long long>(j) * 3 * C + 2 * C + col, pv);
+    uint4 uk[PPT], uv[PPT];
+#pragma unroll
+    for (int i = 0; i < PPT; ++i) {
+      const long long pos = p0 + i;
+      uk[i] = uv[i] = make_uint4(0, 0, 0, 0);
+      if (act && pos < hw) {
+        const T* r = cur ? qkv + pos * 3 * C + C + col : cache + (static_cast<long long>(slot) * hw + pos) * row2 + col;
+        uk[i] = __ldg(reinterpret_cast<const uint4*>(r));
+        uv[i] = __ldg(reinterpret_cast<const uint4*>(r + C));
+      }
+    }
+#pragma unroll
+    for (int i = 0; i < PPT; ++i) {
+      float fk[8], fv[8];
+      unpack8<T>(uk[i], fk);
+      unpack8<T>(uv[i], fv);
+      float s = 0.f;
+#pragma unroll
+      for (int e = 0; e < 8; ++e) s = fmaf(q[i][e], fk[e] + pk[e], s);
+#pragma unroll
+      for (int x = 1; x < G; x <<= 1) s += __shfl_xor_sync(0xffffffffu, s, x);
+      if (valid) {
+        const float mn = fmaxf(m[i], s);
+        const float corr = exp2f(m[i] - mn), p = exp2f(s - mn);
+        m[i] = mn;
+        l[i] = fmaf(l[i], corr, p);
+#pragma unroll
+        for (int e = 0; e < 8; ++e) o[i][e] = fmaf(o[i][e], corr, p * (fv[e] + pv[e]));
+      }
+    }
+  }
+  // ---- merge the key splits (lanes c, c + G, c + 2G, ...); a split without keys has m = -inf, l = 0 ----
+#pragma unroll
+  for (int i = 0; i < PPT; ++i) {
+    float mx = m[i];
+#pragma unroll
+    for (int x = G; x < 32; x <<= 1) mx = fmaxf(mx, __shfl_xor_sync(0xffffffffu, mx, x));
+    const float f = exp2f(m[i] - mx);
+    float li = l[i] * f;
+#pragma unroll
+    for (int x = G; x < 32; x <<= 1) li += __shfl_xor_sync(0xffffffffu, li, x);
+#pragma unroll
+    for (int e = 0; e < 8; ++e) {
+      float v = o[i][e] * f;
+#pragma unroll
+      for (int x = G; x < 32; x <<= 1) v += __shfl_xor_sync(0xffffffffu, v, x);
+      o[i][e] = v;
+    }
+    const long long pos = p0 + i;
+    if (ks == 0 && act && pos < hw) {
+      const float inv = 1.f / li;
+      uint4 u;
+      u.x = H16<T>::pack2(o[i][0] * inv, o[i][1] * inv);
+      u.y = H16<T>::pack2(o[i][2] * inv, o[i][3] * inv);
+      u.z = H16<T>::pack2(o[i][4] * inv, o[i][5] * inv);
+      u.w = H16<T>::pack2(o[i][6] * inv, o[i][7] * inv);
+      *reinterpret_cast<uint4*>(out + pos * C + col) = u;
+    }
+  }
+}
+
+template <typename T, int G>
+static int launch_step(const void* qkv, void* cache, const float* pe, const int32_t* ctx, void* out, int hw, int C,
+                       int heads, int slots, cudaStream_t st) {
+  constexpr int PPT = 2;
+  const long long threads = static_cast<long long>((hw + PPT - 1) / PPT) * heads * 32;
+  const int blocks = static_cast<int>((threads + 255) / 256);
+  temporal_step_kernel<T, G, PPT><<<blocks, 256, 0, st>>>(static_cast<const T*>(qkv), static_cast<T*>(cache), pe, ctx,
+                                                          static_cast<T*>(out), hw, C, heads, slots);
+  VDA_CUDA(cudaGetLastError());
+  return 0;
+}
+
+template <typename T>
+static int dispatch_step(const void* qkv, void* cache, const float* pe, const int32_t* ctx, void* out, int hw, int C,
+                         int heads, int slots, cudaStream_t st) {
+  const int chunks = C / heads / 8;
+  if (chunks <= 1) return launch_step<T, 1>(qkv, cache, pe, ctx, out, hw, C, heads, slots, st);
+  if (chunks <= 2) return launch_step<T, 2>(qkv, cache, pe, ctx, out, hw, C, heads, slots, st);
+  if (chunks <= 4) return launch_step<T, 4>(qkv, cache, pe, ctx, out, hw, C, heads, slots, st);
+  if (chunks <= 8) return launch_step<T, 8>(qkv, cache, pe, ctx, out, hw, C, heads, slots, st);
+  return launch_step<T, 16>(qkv, cache, pe, ctx, out, hw, C, heads, slots, st);
+}
+
 }  // namespace vda
 
 using namespace vda;
+
+extern "C" int vda_attention_temporal_step(const void* qkv, void* cache, const float* pe, const int32_t* ctx, void* out,
+                                           int hw, int C, int heads, int slots, int dtype, void* stream) {
+  VDA_CHECK(dtype == VDA_BF16 || dtype == VDA_FP16, "bad dtype %d", dtype);
+  VDA_CHECK(hw > 0, "temporal step: hw must be positive, got %d", hw);
+  VDA_CHECK(C % 8 == 0 && C % heads == 0 && (C / heads) % 8 == 0 && heads <= 8 && C / heads <= 128,
+            "bad channel/head split C=%d heads=%d (head dim must be a multiple of 8, <= 128; heads <= 8)", C, heads);
+  VDA_CHECK(slots >= 2 && slots <= 32, "temporal step: the cache holds 2..32 frame slots, got %d", slots);
+  VDA_CHECK(qkv && cache && pe && ctx && out, "temporal step: null pointer");
+  VDA_CHECK(((reinterpret_cast<uintptr_t>(qkv) | reinterpret_cast<uintptr_t>(cache) | reinterpret_cast<uintptr_t>(pe) |
+              reinterpret_cast<uintptr_t>(out)) & 15) == 0,
+            "qkv/cache/pe/out must be 16-byte aligned");
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  if (dtype == VDA_BF16) return dispatch_step<__nv_bfloat16>(qkv, cache, pe, ctx, out, hw, C, heads, slots, st);
+  return dispatch_step<__half>(qkv, cache, pe, ctx, out, hw, C, heads, slots, st);
+}
 
 extern "C" int vda_attention_temporal(const void* qkv, void* out, int T, int hw, int C, int heads, int dtype,
                                       void* stream) {

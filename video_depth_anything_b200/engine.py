@@ -97,6 +97,8 @@ class Engine:
         self.w: Dict[str, torch.Tensor] = {}
         self._pos_cache: Dict[tuple, torch.Tensor] = {}
         self.loaded = False
+        self.generation = 0          # bumped by every load(): streams opened on older weights refuse to continue
+        self._stream_serial = 0
         # One CUDA graph per input shape: a forward is ~330 back-to-back kernel launches with no host decisions,
         # so it is captured once and replayed (removes launch gaps and the host-side descriptor encoding).
         self.use_graphs = os.environ.get("VDA_NO_GRAPH", "0") != "1"
@@ -206,6 +208,11 @@ class Engine:
                 w[f"mm{m}.a{a}.qkv.w"] = h16(torch.cat([sd[ab + "to_q.weight"], sd[ab + "to_k.weight"], sd[ab + "to_v.weight"]], 0))
                 w[f"mm{m}.a{a}.o.w"], w[f"mm{m}.a{a}.o.b"] = h16(sd[ab + "to_out.0.weight"]), f32(ab + "to_out.0.bias")
                 w[f"mm{m}.a{a}.pe"] = f32(ab + "pos_encoder.pe").reshape(-1, C)
+                # streaming: q|k|v = (n + pe[p]) W^T = n W^T + pe[p] W^T, so cached frames keep n W_k^T | n W_v^T and the
+                # step kernel adds this positional share (fp32, rounded once from double) at the position a frame has now
+                wqkv = torch.cat([sd[ab + "to_q.weight"], sd[ab + "to_k.weight"], sd[ab + "to_v.weight"]], 0)
+                pe32 = sd[ab + "pos_encoder.pe"].reshape(-1, C)[:32].double()
+                w[f"mm{m}.a{a}.pet"] = (pe32 @ wqkv.double().t()).to(dev, torch.float32).contiguous()
                 w[f"mm{m}.a{a}.ln.w"], w[f"mm{m}.a{a}.ln.b"] = f32(f"{blk}norms.{a}.weight"), f32(f"{blk}norms.{a}.bias")
             w[f"mm{m}.ffn.w"], w[f"mm{m}.ffn.b"] = f32(blk + "ff_norm.weight"), f32(blk + "ff_norm.bias")
             half = 128 if (4 * C) % 128 == 0 else 64
@@ -214,6 +221,7 @@ class Engine:
             w[f"mm{m}.ff0.w"], w[f"mm{m}.ff0.b"] = h16(wp), bp
             self.__dict__.setdefault("mm_half", {})[m] = half
             w[f"mm{m}.ff2.w"], w[f"mm{m}.ff2.b"] = h16(sd[blk + "ff.net.2.weight"]), f32(blk + "ff.net.2.bias")
+        self.generation += 1
         self.loaded = True
 
     # -------------------------------------------------------------------------------------------
@@ -344,8 +352,10 @@ class Engine:
         ops.bilinear_nhwc(o, up, n, H, W, oh, ow, F)
         return up
 
-    def _motion(self, m, x, B, T, hw):
-        """TemporalModule (motion_module.py:60-65, 102-126, 164-177).  x h16 [B*T*hw, C] rows (b, f, pos)."""
+    def _motion(self, m, x, B, T, hw, stream=None):
+        """TemporalModule (motion_module.py:60-65, 102-126, 164-177).  x h16 [B*T*hw, C] rows (b, f, pos).
+        `stream` = (caches, ctx): one streamed frame (B = T = 1) whose temporal attention reads the stream's cached
+        frames (stream_step)."""
         w, C = self.w, self.mm_c[m]
         M = B * T * hw
         p = f"mm{m}."
@@ -357,12 +367,17 @@ class Engine:
         qkv = self._hnew(M, 3 * C)
         o = self._hnew(M, C)
         for a in (0, 1):                                                                # :165-172
-            ops.layernorm(h, w[f"{p}a{a}.ln.w"], w[f"{p}a{a}.ln.b"], 1e-5, n, pe=w[f"{p}a{a}.pe"], pe_rows_per_frame=hw,
-                          pe_frames=T)                     # rows are (clip, frame, position): frame = (r // hw) % T
-            ops.gemm(n, w[f"{p}a{a}.qkv.w"], qkv, bias=self._const(0.0, 3 * C))   # zero bias: takes the specialised epilogue
-            for b in range(B):
-                s = slice(b * T * hw, (b + 1) * T * hw)
-                ops.attention_temporal(qkv[s], o[s], T, hw, C)
+            if stream is None:
+                ops.layernorm(h, w[f"{p}a{a}.ln.w"], w[f"{p}a{a}.ln.b"], 1e-5, n, pe=w[f"{p}a{a}.pe"], pe_rows_per_frame=hw,
+                              pe_frames=T)                 # rows are (clip, frame, position): frame = (r // hw) % T
+                ops.gemm(n, w[f"{p}a{a}.qkv.w"], qkv, bias=self._const(0.0, 3 * C))   # zero bias: takes the specialised epilogue
+                for b in range(B):
+                    s = slice(b * T * hw, (b + 1) * T * hw)
+                    ops.attention_temporal(qkv[s], o[s], T, hw, C)
+            else:                                          # positional encoding enters through the `pet` table
+                ops.layernorm(h, w[f"{p}a{a}.ln.w"], w[f"{p}a{a}.ln.b"], 1e-5, n)
+                ops.gemm(n, w[f"{p}a{a}.qkv.w"], qkv, bias=self._const(0.0, 3 * C))
+                ops.attention_temporal_step(qkv, stream[0][2 * m + a], w[f"{p}a{a}.pet"], stream[1], o)
             ops.gemm(o, w[f"{p}a{a}.o.w"], h, bias=w[f"{p}a{a}.o.b"], gamma=self._const(1.0, C), res1=h)   # unit LayerScale: ditto
         ops.layernorm(h, w[p + "ffn.w"], w[p + "ffn.b"], 1e-5, n)                        # :174
         g = self._hnew(M, 4 * C)
@@ -373,8 +388,8 @@ class Engine:
         ops.gemm(h16, w[p + "out.w"], out, bias=w[p + "out.b"], res1=x)                  # :120-125
         return out
 
-    def head(self, taps, B, T, hp, wp, stages=None) -> torch.Tensor:
-        """DPTHeadTemporal.forward (dpt_temporal.py:53-114) -> fp32 [B*T, 14hp, 14wp]."""
+    def head(self, taps, B, T, hp, wp, stages=None, stream=None) -> torch.Tensor:
+        """DPTHeadTemporal.forward (dpt_temporal.py:53-114) -> fp32 [B*T, 14hp, 14wp].  `stream`: see _motion."""
         w, F, oc = self.w, self.F, self.oc
         BT = B * T
         P = hp * wp
@@ -396,8 +411,8 @@ class Engine:
         del col
         if stages is not None:
             stages.update(layer_1=(l1, h1, w1), layer_2=(l2, h2, w2), layer_3=(l3, hp, wp), layer_4=(l4, h4, w4))
-        l3 = self._motion(0, l3, B, T, P)                                               # :75
-        l4 = self._motion(1, l4, B, T, h4 * w4)                                         # :76
+        l3 = self._motion(0, l3, B, T, P, stream)                                       # :75
+        l4 = self._motion(1, l4, B, T, h4 * w4, stream)                                 # :76
         if stages is not None:
             stages.update(mm0=(l3, hp, wp), mm1=(l4, h4, w4))
 
@@ -416,11 +431,11 @@ class Engine:
         p4 = self._fusion(4, None, l4r, l4rr, BT, h4, w4, hp, wp)                        # :83
         if stages is not None:
             stages["path_4_pre"] = (p4, hp, wp)
-        p4 = self._motion(2, p4, B, T, P)                                               # :84
+        p4 = self._motion(2, p4, B, T, P, stream)                                       # :84
         p3 = self._fusion(3, p4, l3r, l3rr, BT, hp, wp, h2, w2)                          # :85
         if stages is not None:
             stages.update(path_4=(p4, hp, wp), path_3_pre=(p3, h2, w2))
-        p3 = self._motion(3, p3, B, T, h2 * w2)                                         # :86
+        p3 = self._motion(3, p3, B, T, h2 * w2, stream)                                 # :86
         p2 = self._fusion(2, p3, l2r, l2rr, BT, h2, w2, h1, w1)                          # :90/103
         p1 = self._fusion(1, p2, l1r, l1rr, BT, h1, w1, 2 * h1, 2 * w1)                  # :91/104
         if stages is not None:
@@ -528,3 +543,43 @@ class Engine:
         depth = self.head(taps, B, T, hp, wp, stages)
         # video_depth.py:162-163: bilinear to (H,W) is the identity (14*hp == H) and the ReLU is already applied
         return depth.view(B, T, H, W)
+
+    # ------------------------------------------------------------------------------------------- streaming
+    def stream_cache(self, hp: int, wp: int, slots: int) -> List[torch.Tensor]:
+        """Per temporal-attention block (index 2 * motion module + attention block) the k'|v' rows of `slots` frames:
+        head dtype [slots, hw, 2C], row = k' (C) | v' (C) of one position, so one head's keys and values are contiguous
+        16-byte runs."""
+        hws = [hp * wp, ((hp - 1) // 2 + 1) * ((wp - 1) // 2 + 1), hp * wp, 4 * hp * wp]
+        return [self._hnew(slots, hws[m], 2 * self.mm_c[m]) for m in range(4) for _ in (0, 1)]
+
+    def stream_step(self, frame: torch.Tensor, ctx: torch.Tensor, cache: List[torch.Tensor], nh: int, nw: int) -> torch.Tensor:
+        """One streamed frame: uint8 [H0,W0,3] (device) -> fp32 depth [H0,W0] (>= 0).  Preprocessing as in
+        infer_video_depth, encoder and head at T = 1 with every temporal attention against `cache` as `ctx` describes
+        (vda_attention_temporal_step), bilinear resize to the frame size.  No host decisions: graph-capturable."""
+        h0, w0 = frame.shape[:2]
+        key = ("idx0",)
+        if key not in self._bufs:
+            self._bufs[key] = [torch.zeros(1, dtype=torch.int32, device=self.device)]
+        x = ops.preprocess_frames(frame.unsqueeze(0), self._bufs[key][0], nh, nw)
+        d = self.head(self.encode(x), 1, 1, nh // 14, nw // 14, stream=(cache, ctx))
+        if (nh, nw) != (h0, w0):
+            d = ops.bilinear_f32(d, h0, w0)
+        return d[0]
+
+    def new_stream_id(self) -> int:
+        self._stream_serial += 1
+        return self._stream_serial
+
+    def stream_step_graphed(self, sid: int, frame: torch.Tensor, ctx: torch.Tensor, cache: List[torch.Tensor], nh: int,
+                            nw: int) -> torch.Tensor:
+        """stream_step as a CUDA graph captured once per stream `sid` (its cache pointers are part of the graph); `frame`
+        and `ctx` are the stream's own long-lived input buffers.  Returns the graph's static output."""
+        if self.use_graphs and ops.PROFILE is None:
+            return self._graphed(("stream", sid, nh, nw) + tuple(frame.shape), lambda f, c: self.stream_step(f, c, cache, nh, nw),
+                                 [frame, ctx], adopt=True)
+        return self.stream_step(frame, ctx, cache, nh, nw)
+
+    def drop_stream(self, sid: int) -> None:
+        """Forget the graphs of stream `sid` (they hold its cache)."""
+        for k in [k for k in self._graphs if k[0] == "stream" and k[1] == sid]:
+            del self._graphs[k]

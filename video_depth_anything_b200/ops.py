@@ -199,6 +199,28 @@ def attention_temporal(qkv: torch.Tensor, out: torch.Tensor, T: int, hw: int, Cc
     return out
 
 
+def attention_temporal_step(qkv: torch.Tensor, cache: torch.Tensor, pe: torch.Tensor, ctx: torch.Tensor, out: torch.Tensor,
+                            heads: int = 8):
+    """Streaming temporal attention of one frame (vda.h vda_attention_temporal_step): qkv h16 [hw, 3C] (q'|k'|v', no
+    positional encoding), cache h16 [slots, hw, 2C] (k'|v' rows of earlier frames), pe fp32 [32, 3C] (positional share of
+    q|k|v), ctx device int32 [>= 2] = (n_ctx, write slot, context slots...) -> out h16 [hw, C]."""
+    lib = _lib.load()
+    hw, C3 = qkv.shape
+    Cc = C3 // 3
+    slots = cache.shape[0]
+    assert qkv.is_contiguous() and cache.is_contiguous() and pe.is_contiguous() and out.is_contiguous()
+    assert cache.shape[1:] == (hw, 2 * Cc) and cache.dtype == qkv.dtype and out.dtype == qkv.dtype
+    assert pe.dtype == torch.float32 and pe.shape[-1] == C3 and pe.shape[0] >= 32
+    assert ctx.dtype == torch.int32 and ctx.is_contiguous() and ctx.numel() >= 2
+    if PROFILE is not None:      # bytes of a full 31-frame context: cached k'|v' rows read, current q|k|v in, out + slot out
+        _INFO.update(kind="attention_temporal_step",
+                     bytes=float(qkv.element_size() * hw * (31 * 2 * Cc + 3 * Cc + Cc + 2 * Cc)))
+    check(lib.vda_attention_temporal_step(_p(qkv), _p(cache), _p(pe), _p(ctx), _p(out), hw, Cc, heads, slots,
+                                          dt_code(qkv.dtype), _stream()))
+    _count()
+    return out
+
+
 def preprocess_frames(frames_u8: torch.Tensor, idx: torch.Tensor, nh: int, nw: int) -> torch.Tensor:
     """uint8 RGB [N,H0,W0,3] (device) + int32 frame indices [n] (device) -> normalised fp32 [n,3,nh,nw]
     (util/transform.py Resize(INTER_CUBIC) / NormalizeImage / PrepareForNet)."""
@@ -351,7 +373,8 @@ def _profiled(fn, name):
     return wrapper
 
 
-for _n in ("preprocess_frames", "copy_frames", "gemm", "layernorm", "rowstats_cast", "groupnorm", "attention_spatial", "attention_temporal", "patch_im2col", "write_cls",
+for _n in ("preprocess_frames", "copy_frames", "gemm", "layernorm", "rowstats_cast", "groupnorm", "attention_spatial", "attention_temporal",
+           "attention_temporal_step", "patch_im2col", "write_cls",
            "pos_embed_bicubic", "im2col3x3_s2", "bilinear_nhwc", "tail_fused", "bilinear_f32", "add_h16", "lsq_scale_shift", "align_chain",
            "affine_clamp_blend"):
     globals()[_n] = _profiled(globals()[_n], _n)

@@ -26,7 +26,7 @@ from . import ops
 from .engine import Engine
 from .synth import ENCODER_DIMS, synth_state_dict
 from .windows import (INFER_LEN, INTERP_LEN, KEYFRAMES, OVERLAP, aligner_ring_len, aligner_ring_pos, get_resize_hw,
-                      plan_feature_cache, upload_ring_plan, window_source_indices)
+                      plan_feature_cache, stream_context, upload_ring_plan, window_source_indices)
 
 
 VALIDATION_DTYPE = torch.float16     # operand type of the `fp32=True` path (see _ensure_engine)
@@ -54,6 +54,7 @@ class VideoDepthAnything(nn.Module):
         self._engine: Optional[Engine] = None
         self._engine_val: Optional[Engine] = None        # fp32=True (validation precision), built on first use
         self._device = torch.device("cpu")
+        self._stream_one: Optional["DepthStream"] = None   # infer_video_depth_one's stream
 
     # ---- nn.Module surface -------------------------------------------------------------------
     def state_dict(self, *a, **k):
@@ -192,6 +193,111 @@ class VideoDepthAnything(nn.Module):
             if not own_aligner:
                 return None
             return aligner.result(), target_fps
+
+    # ---- streaming -----------------------------------------------------------------------------
+    def stream(self, input_size: int = 518, fp32: bool = False) -> "DepthStream":
+        """Open a depth stream on this model's device: `push` one uint8 frame, get its depth back at once.  Each frame
+        attends to frame 0 and the 30 frames before it (DepthStream).  Streams are independent of each other and of
+        `forward` / `infer_video_depth`; `fp32=True` selects the validation-precision engine as in infer_video_depth."""
+        return DepthStream(self, self._ensure_engine(validation=bool(fp32)), input_size)
+
+    @torch.no_grad()
+    def infer_video_depth_one(self, frame: np.ndarray, input_size: int = 518, device="cuda", fp32: bool = False) -> np.ndarray:
+        """Depth of the next frame of the model's own stream (the name of the upstream project's streaming entry
+        point): frame uint8 [H0,W0,3] -> float32 [H0,W0].  The stream is opened on the first call and reopened (its
+        temporal context starts over) when `input_size`, `fp32` or the device change or new weights were loaded."""
+        if torch.device(device).type != "cuda":
+            raise RuntimeError("infer_video_depth_one: the B200 engine has no CPU path (device must be 'cuda')")
+        self.to(device)
+        eng = self._ensure_engine(validation=bool(fp32))
+        st = self._stream_one
+        if st is None or st.engine is not eng or st.input_size != input_size or st.generation != eng.generation:
+            if st is not None:
+                st.close()
+            st = self._stream_one = self.stream(input_size, fp32)
+        return st.push(frame)
+
+
+class DepthStream:
+    """Streaming inference: one frame in, its depth out, with a cached temporal context.
+
+    Frame t is preprocessed as in infer_video_depth, encoded and run through the head with T = 1; in each of the 8
+    temporal-attention blocks its query attends to itself and to the context frames ctx(t) = [0] + the most recent
+    earlier frames (at most L = num_frames - 1 = 31 of them, windows.stream_context), frame 0 at position 0 and the
+    current frame last, each with the positional encoding of its position in that sequence.  So for t <= 31 the result is
+    the windowed forward of frames 0..t under a causal temporal mask.  (The upstream streaming script pads the early
+    context with copies of frame 0 instead; that breaks this equivalence and is not done here.)  No scale / shift
+    alignment between frames.
+
+    A cached frame is kept as its k'|v' = LayerNorm output @ [W_k | W_v]^T rows, without the positional encoding, whose
+    share is added by the step kernel at the frame's current position: a step never re-projects old frames.  Device
+    memory is bounded: L + 1 cache slots per block.  The whole step (preprocess, encoder, head, resize) is one CUDA graph
+    per stream; a push is one H2D of the frame and of the <= 33-int context, a replay and one D2H of the depth.
+    Frame size (and so the network size) is fixed by the first frame."""
+
+    def __init__(self, model: VideoDepthAnything, engine: Engine, input_size: int = 518):
+        self.model, self.engine, self.input_size = model, engine, int(input_size)
+        self.device = engine.device
+        self.generation = engine.generation
+        self.L = model.num_frames - 1
+        if not 1 <= self.L <= INFER_LEN - 1:
+            raise ValueError(f"streaming needs num_frames in 2..{INFER_LEN}, got {model.num_frames}")
+        self.sid = engine.new_stream_id()
+        self.t = 0                                   # frames pushed so far
+        self.size = None                             # (h0, w0), fixed by the first frame
+        self.cache = None
+        self.closed = False
+
+    def _open(self, h0: int, w0: int) -> None:
+        eng = self.engine
+        self.nh, self.nw = get_resize_hw(h0, w0, self.input_size)
+        with torch.cuda.device(self.device):
+            self.cache = eng.stream_cache(self.nh // 14, self.nw // 14, self.L + 1)
+            self.frame_dev = torch.empty(h0, w0, 3, dtype=torch.uint8, device=self.device)
+            self.ctx_dev = torch.zeros(2 + self.L, dtype=torch.int32, device=self.device)
+            self.frame_host = torch.empty(h0, w0, 3, dtype=torch.uint8).pin_memory()
+            self.ctx_host = torch.zeros(2 + self.L, dtype=torch.int32).pin_memory()
+            self.out_host = torch.empty(h0, w0, dtype=torch.float32).pin_memory()
+        self.size = (h0, w0)
+
+    @torch.no_grad()
+    def push(self, frame: np.ndarray) -> np.ndarray:
+        """frame uint8 RGB [H0,W0,3] -> its depth float32 [H0,W0] (>= 0); a fresh array on every call."""
+        if not isinstance(frame, np.ndarray) or frame.ndim != 3 or frame.shape[2] != 3 or frame.dtype != np.uint8:
+            raise ValueError("frame must be a uint8 numpy array [H0,W0,3]")
+        if self.closed:
+            raise RuntimeError("push on a closed DepthStream")
+        if self.engine.generation != self.generation or not self.engine.loaded:
+            raise RuntimeError("the model's weights changed since this stream was opened; open a new stream")
+        if self.size is None:
+            self._open(*frame.shape[:2])
+        elif tuple(frame.shape[:2]) != self.size:
+            raise ValueError(f"frame size {tuple(frame.shape[:2])} differs from the stream's {self.size}")
+        _, slots, write = stream_context(self.t, self.L)
+        ctx = self.ctx_host.numpy()
+        ctx[0], ctx[1] = len(slots), write
+        ctx[2:2 + len(slots)] = slots
+        np.copyto(self.frame_host.numpy(), frame)
+        with torch.cuda.device(self.device):
+            self.frame_dev.copy_(self.frame_host, non_blocking=True)
+            self.ctx_dev.copy_(self.ctx_host, non_blocking=True)
+            d = self.engine.stream_step_graphed(self.sid, self.frame_dev, self.ctx_dev, self.cache, self.nh, self.nw)
+            self.out_host.copy_(d, non_blocking=True)
+            torch.cuda.current_stream().synchronize()   # (also: the pinned inputs are free for the next push)
+        self.t += 1
+        return self.out_host.numpy().copy()
+
+    def close(self) -> None:
+        """Release the stream's graph and cache (also done when the object is collected)."""
+        self.engine.drop_stream(self.sid)
+        self.cache = None
+        self.closed = True
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:                                # noqa: BLE001  (interpreter shutdown)
+            pass
 
 
 class FeatureCache:

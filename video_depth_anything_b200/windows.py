@@ -130,3 +130,25 @@ def upload_ring_plan(n_needed: int, chunk: int = 64, ring_chunks: int = 4):
     slots = [0] + [1 + (j - 1) % cap for j in range(1, n_needed)]
     chunks = [(0, 1)] + [(lo, min(lo + chunk, n_needed)) for lo in range(1, n_needed, chunk)]
     return True, 1 + cap, slots, chunks
+
+
+# ------------------------------------------------------------------------------------------------
+# streaming (video_depth.DepthStream): temporal context and cache slots of frame t
+# ------------------------------------------------------------------------------------------------
+STREAM_CONTEXT = INFER_LEN - 1          # L: cached frames a streamed frame attends to (32 positions with itself)
+
+
+def stream_context(t: int, L: int = STREAM_CONTEXT):
+    """Context of streamed frame t: (frame ids, their cache slots, slot frame t is written to).  Frame 0 is a permanent
+    anchor at position 0 (as slot 0 of every offline window), followed by the most recent earlier frames:
+    ctx(0) = [], ctx(t) = [0] + [max(1, t - L + 1) .. t - 1].  Frame 0 owns slot 0, frames j >= 1 share a ring of L slots
+    (slot 1 + (j - 1) % L), so a stream holds at most L + 1 slots however long it runs.  The frame a write replaces
+    (t - L) has just left the context, so the write slot is never read in the same step."""
+    if t < 0 or L < 1:
+        raise ValueError(f"bad stream step t={t} L={L}")
+
+    def slot(j):
+        return 0 if j == 0 else 1 + (j - 1) % L
+
+    ids = [] if t == 0 else [0] + list(range(max(1, t - L + 1), t))
+    return ids, [slot(j) for j in ids], slot(t)
