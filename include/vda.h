@@ -155,9 +155,21 @@ int vda_attention_temporal(const void* qkv, void* out, int T, int hw, int C, int
  * position n_ctx, whose query is q' + pe_q[n_ctx]; out: h16 [hw, C] = softmax(q k^T / sqrt(C/heads)) v per head, fp32
  * inside.  The current frame's k'|v' rows are also copied, unchanged, into slot `write_slot` of the cache, which must
  * not be one of the slots read.  Everything that changes from step to step is in `ctx`, so a captured CUDA graph
- * replays it. */
+ * replays it.  The B = 1 case of vda_attention_temporal_step_batched on pool entry 0. */
 int vda_attention_temporal_step(const void* qkv, void* cache, const float* pe, const int32_t* ctx, void* out, int hw,
                                 int C, int heads, int slots, int dtype, void* stream);
+
+/* The streaming step of B frames of different streams in one launch (a group of streams pushing together):
+ *   qkv:  h16 [B*hw, 3*C], row block b = batch row b's q'|k'|v';
+ *   pool: h16 [S, slots, hw, 2*C], one cache as above per stream;
+ *   rows: device int32 [B], the pool entry of batch row b; -1 marks a pad row;
+ *   ctx:  device int32 [B, ctx_stride], row b laid out as ctx above (n_ctx is also clamped to ctx_stride - 2).
+ * A real row does exactly what vda_attention_temporal_step does against pool[rows[b]], including the write of its k'|v'
+ * into its write slot.  A row whose pool index is outside 0..S-1 (a pad row) attends to itself only (n_ctx = 0) and
+ * reads and writes no pool byte; pool entries no row names are not touched.  out: h16 [B*hw, C]. */
+int vda_attention_temporal_step_batched(const void* qkv, void* pool, const float* pe, const int32_t* rows,
+                                        const int32_t* ctx, void* out, int B, int S, int ctx_stride, int hw, int C,
+                                        int heads, int slots, int dtype, void* stream);
 
 /* Frame preprocessing of infer_video_depth (video_depth.py:173-185,197-198; util/transform.py:109-158): for every
  * i < n, frame idx[i] of the device-resident uint8 RGB video frames [*, H0, W0, 3] -> /255 -> cv2-style INTER_CUBIC

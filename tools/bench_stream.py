@@ -9,7 +9,11 @@ Per config (vits 518x518, vitl 518x518, vitl 518x924 = a 1280x720 video, the met
   * the windowed forward of the same model (one 32-frame window, CUDA events) in frames/s, for comparison.
 Then the step kernel alone at every block shape of the configs with a full context (31 cached frames, 32 slots):
 median time over launches with the L2 overwritten in between, the bytes it must move (computed from shapes) over that
-time, and that rate's share of the HBM bound (7.7 TB/s, the HGX B200 data sheet's per-GPU figure).
+time, and that rate's share of the HBM bound (7.7 TB/s, the HGX B200 data sheet's per-GPU figure); for the ViT-L 518x518
+shapes also the batched kernel at B = 8 (8 streams' frames in one launch).
+Then stream groups (VideoDepthAnything.stream_group) of each --streams count for ViT-S and ViT-L at 518x518: every push
+names every stream, push latency p50 / p99 over --group-pushes pushes after 40 warm-up pushes, and aggregate frames/s
+(streams / p50 push).
 The card's name and power limit are read in the same run."""
 import argparse
 import json
@@ -63,7 +67,7 @@ def bench_config(enc, h0, w0, warmup, frames, dtype):
     for _ in range(100):                              # replays of the last step (idempotent: same inputs, same slot)
         s, e = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         s.record()
-        st.engine.stream_step_graphed(st.sid, st.frame_dev, st.ctx_dev, st.cache, st.nh, st.nw)
+        st.group._step(1)
         e.record()
         e.synchronize()
         dev.append(s.elapsed_time(e))
@@ -81,8 +85,8 @@ def bench_config(enc, h0, w0, warmup, frames, dtype):
         win.append(s.elapsed_time(e))
     eng = st.engine
     hp, wp = nh // 14, nw // 14
-    shapes = [(c.shape[1], c.shape[2] // 2) for c in st.cache[::2]]   # (hw, C) of motion modules 0..3
-    launches = eng._graphs[("stream", st.sid, st.nh, st.nw, h0, w0, 3)][3]
+    shapes = [(c.shape[2], c.shape[3] // 2) for c in st.group.pool[::2]]   # (hw, C) of motion modules 0..3
+    launches = st.group.graphs[1][3]
     st.close()
     del st, m
     torch.cuda.empty_cache()
@@ -94,43 +98,78 @@ def bench_config(enc, h0, w0, warmup, frames, dtype):
             "grid": [hp, wp]}, shapes
 
 
-def bench_kernel(hw, C, dtype, iters=30):
+def bench_kernel(hw, C, dtype, B=1, iters=30):
     slots, n = 32, 31
     g = torch.Generator(device="cuda").manual_seed(0)
-    qkv = torch.randn(hw, 3 * C, device="cuda", generator=g).to(dtype)
-    cache = torch.randn(slots, hw, 2 * C, device="cuda", generator=g).to(dtype)
+    qkv = torch.randn(B * hw, 3 * C, device="cuda", generator=g).to(dtype)
+    cache = torch.randn(B, slots, hw, 2 * C, device="cuda", generator=g).to(dtype)
     pe = torch.randn(32, 3 * C, device="cuda", generator=g)
-    ctx = torch.tensor([n, 31] + list(range(31)), dtype=torch.int32, device="cuda")
-    out = torch.empty(hw, C, dtype=dtype, device="cuda")
+    ctx = torch.tensor([[n, 31] + list(range(31))] * B, dtype=torch.int32, device="cuda")
+    rows = torch.arange(B, dtype=torch.int32, device="cuda")
+    out = torch.empty(B * hw, C, dtype=dtype, device="cuda")
     flush = torch.empty(512 << 20, dtype=torch.uint8, device="cuda")
-    ops.attention_temporal_step(qkv, cache, pe, ctx, out)
+
+    def launch():
+        if B == 1:
+            ops.attention_temporal_step(qkv, cache[0], pe, ctx[0], out)
+        else:
+            ops.attention_temporal_step(qkv, cache, pe, ctx, out, rows=rows)
+    launch()
     ts = []
     for _ in range(iters):
         flush.zero_()                                  # 512 MB written: the cache rows come from HBM, not the 126 MB L2
         s, e = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         s.record()
-        ops.attention_temporal_step(qkv, cache, pe, ctx, out)
+        launch()
         e.record()
         e.synchronize()
         ts.append(s.elapsed_time(e))
     ms = pct(ts, 50)
-    nbytes = 2 * hw * (n * 2 * C + 3 * C + C + 2 * C)   # cached k'|v' read, q'|k'|v' read, out + write-slot row written
+    nbytes = B * 2 * hw * (n * 2 * C + 3 * C + C + 2 * C)   # cached k'|v' read, q'|k'|v' read, out + write-slot row written
     gbs = nbytes / (ms * 1e-3) / 1e9
-    return {"hw": hw, "C": C, "head_dim": C // 8, "us": round(ms * 1e3, 2), "MB": round(nbytes / 1e6, 2),
+    return {"B": B, "hw": hw, "C": C, "head_dim": C // 8, "us": round(ms * 1e3, 2), "MB": round(nbytes / 1e6, 2),
             "GB_s": round(gbs, 1), "hbm_share": round(gbs * 1e9 / HBM_BYTES_PER_S, 3)}
+
+
+def bench_group(enc, h0, w0, S, warmup, pushes, dtype):
+    m = model(enc, dtype)
+    pool = np.random.default_rng(0).integers(0, 256, (16, h0, w0, 3), dtype=np.uint8)
+    g = m.stream_group(max_streams=S)
+    hs = [g.open() for _ in range(S)]
+    host = []
+    for t in range(warmup + pushes):
+        batch = {h: pool[(t + i) % 16] for i, h in enumerate(hs)}
+        t0 = time.perf_counter()
+        g.push(batch)
+        if t >= warmup:
+            host.append((time.perf_counter() - t0) * 1e3)
+    (bk, entry), = g.graphs.items()
+    g.close()
+    del g, m
+    torch.cuda.empty_cache()
+    p50 = pct(host, 50)
+    return {"encoder": enc, "frame": [h0, w0], "streams": S, "bucket": bk, "launches_per_push": entry[3],
+            "push_ms_p50": round(p50, 3), "push_ms_p99": round(pct(host, 99), 3),
+            "aggregate_fps": round(S * 1e3 / p50, 1)}
 
 
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--warmup", type=int, default=40)
     ap.add_argument("--frames", type=int, default=400)
+    ap.add_argument("--streams", default="", help="comma-separated stream counts for the group sweep, e.g. 1,2,4,8,16")
+    ap.add_argument("--group-pushes", type=int, default=100)
+    ap.add_argument("--skip-single", action="store_true", help="only the group sweep and the batched kernel")
     ap.add_argument("--out", default=os.path.join(ROOT, "profiles", "stream_b200.json"))
     a = ap.parse_args()
+    counts = [int(x) for x in a.streams.split(",") if x]
     if not torch.cuda.is_available():
         sys.exit("bench_stream.py needs a GPU")
     res = {"what": "streaming push latency / step device time / step kernel", **card(), "configs": [], "step_kernel": []}
     seen = set()
     for enc, h0, w0 in CONFIGS:
+        if a.skip_single:
+            break
         r, shapes = bench_config(enc, h0, w0, a.warmup, a.frames, torch.bfloat16)
         res["configs"].append(r)
         for mm, (hw, C) in enumerate(shapes):
@@ -138,6 +177,14 @@ def main():
                 seen.add((hw, C))
                 res["step_kernel"].append({"config": f"{enc} {r['network'][0]}x{r['network'][1]} mm{mm}",
                                            **bench_kernel(hw, C, torch.bfloat16)})
+    if counts:
+        res["what"] += " / stream groups / batched step kernel at B = 8"
+        hp = 518 // 14
+        vitl = [(hp * hp, 1024), ((hp + 1) // 2 * ((hp + 1) // 2), 1024), (hp * hp, 256), (4 * hp * hp, 256)]
+        res["step_kernel_b8"] = [{"config": f"vitl 518x518 mm{mm}", **bench_kernel(hw, C, torch.bfloat16, B=8)}
+                                 for mm, (hw, C) in enumerate(vitl)]
+        res["groups"] = [bench_group(enc, 518, 518, S, a.warmup, a.group_pushes, torch.bfloat16)
+                         for enc in ("vits", "vitl") for S in counts]
     line = json.dumps(res)
     print(line)
     os.makedirs(os.path.dirname(os.path.abspath(a.out)), exist_ok=True)

@@ -53,6 +53,7 @@ _SIGS = {
     "vda_attention_temporal": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p]),
     "vda_attention_temporal_step": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int,
                                               C.c_int, C.c_int, C.c_int, C.c_void_p]),
+    "vda_attention_temporal_step_batched": (C.c_int, [C.c_void_p] * 6 + [C.c_int] * 8 + [C.c_void_p]),
     "vda_preprocess_frames": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int,
                                         C.c_void_p]),
     "vda_copy_frames": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int64, C.c_void_p]),

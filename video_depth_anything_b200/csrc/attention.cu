@@ -238,15 +238,18 @@ static int dispatch_temporal(const void* qkv, void* out, int T_, int hw, int C, 
 }
 
 // ---------------------------------------------------------------------------------------------
-// Streaming step: one new frame's query against <= 31 cached frames + itself (vda.h, vda_attention_temporal_step).
+// Streaming step: each batch row's query (one new frame of one stream) against <= 31 cached frames of that stream's
+// pool entry + itself (vda.h, vda_attention_temporal_step_batched; vda_attention_temporal_step is its B = 1 case).
 //
-// One warp owns (head, PPT adjacent positions).  Lane = (key split ks, chunk c): c < G holds 16-byte chunk c of the
-// head's dh columns (G = dh/8 rounded up to a power of two, the extra lanes hold zeros), and the KS = 32/G key splits
-// take keys ks, ks + KS, ... of the sequence, so a lane walks at most 32/KS keys and a warp has all its loads in
-// flight at once (the kernel is HBM-bound: the cached K'|V' rows are the traffic).  Scores are reduced over the G
-// lanes of a split with xor shuffles; every split keeps an online softmax (fp32) and the splits are merged at the
-// end (max, rescale, sum).  The PE projections are added as each row is loaded; a PE row is shared by the PPT
-// positions of a warp, which halves its (L1/L2) traffic.
+// A CTA owns (batch row b, head h, 8 warps x PPT adjacent positions).  It first stages the k | v positional rows of
+// head h at positions 0..n (fp32, n + 1 rows of 2 dh) in shared memory: they depend only on key position and column,
+// so every warp of the CTA reads them from there instead of each lane loading 64 bytes of PE table per 32 bytes of
+// cache from L2.  In a warp, lane = (key split ks, chunk c): c < G holds 16-byte chunk c of the head's dh columns
+// (G = dh/8 rounded up to a power of two, the extra lanes hold zeros), and the KS = 32/G key splits take keys ks,
+// ks + KS, ... of the sequence, so a lane walks at most 32/KS keys and a warp has all its loads in flight at once (the
+// kernel is HBM-bound: the cached K'|V' rows are the traffic).  Scores are reduced over the G lanes of a split with
+// xor shuffles; every split keeps an online softmax (fp32) and the splits are merged at the end (max, rescale, sum).
+// A row whose pool index is outside 0..S-1 (-1: a pad row) attends to itself only and touches no pool byte.
 // ---------------------------------------------------------------------------------------------
 template <typename T>
 __device__ __forceinline__ void unpack8(const uint4& u, float (&f)[8]) {
@@ -265,22 +268,49 @@ __device__ __forceinline__ void load_pe8(const float* p, float (&f)[8]) {
   f[0] = a.x, f[1] = a.y, f[2] = a.z, f[3] = a.w, f[4] = b.x, f[5] = b.y, f[6] = b.z, f[7] = b.w;
 }
 
+__device__ __forceinline__ void lds_pe8(const float* p, float (&f)[8]) {
+  const float4 a = reinterpret_cast<const float4*>(p)[0];
+  const float4 b = reinterpret_cast<const float4*>(p)[1];
+  f[0] = a.x, f[1] = a.y, f[2] = a.z, f[3] = a.w, f[4] = b.x, f[5] = b.y, f[6] = b.z, f[7] = b.w;
+}
+
+constexpr int STEP_WARPS = 8;
+
+// (min. 2 CTAs per SM: without it ptxas caps one instantiation at 64 registers and spills)
 template <typename T, int G, int PPT>
-__global__ void __launch_bounds__(256)
-temporal_step_kernel(const T* __restrict__ qkv, T* __restrict__ cache, const float* __restrict__ pe,
-                     const int32_t* __restrict__ ctx, T* __restrict__ out, int hw, int C, int heads, int slots) {
+__global__ void __launch_bounds__(STEP_WARPS * 32, 2)
+temporal_step_kernel(const T* __restrict__ qkv, T* __restrict__ pool, const float* __restrict__ pe,
+                     const int32_t* __restrict__ rows, const int32_t* __restrict__ ctx, T* __restrict__ out, int hw,
+                     int C, int heads, int S, int slots, int ctx_stride) {
+  extern __shared__ float4 spe4[];                   // [n + 1][pe_k (dh) | pe_v (dh)] of head h
+  float* spe = reinterpret_cast<float*>(spe4);
   constexpr int KS = 32 / G;
-  const long long warp = (static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x) >> 5;
+  const int b = blockIdx.y;
+  const int h = static_cast<int>(blockIdx.x % heads);
   const int lane = threadIdx.x & 31, c = lane % G, ks = lane / G;
   const int dh = C / heads;
-  const int h = static_cast<int>(warp % heads);
-  const long long p0 = warp / heads * PPT;          // (no early exit for p0 >= hw: the shuffles need the whole warp)
+  // (no early exit for p0 >= hw: the shuffles need the whole warp, the staging the whole CTA)
+  const long long p0 = (static_cast<long long>(blockIdx.x / heads) * STEP_WARPS + (threadIdx.x >> 5)) * PPT;
   const bool act = c * 8 < dh;                       // lane holds a real chunk of the head
   const int col = act ? h * dh + c * 8 : h * dh;
-  const int n = min(max(__ldg(ctx), 0), 31);
-  const int ws = min(max(__ldg(ctx + 1), 0), slots - 1);
+  const int sco = act ? c * 8 : 0;                   // the lane's column in a staged PE row
+  const int32_t* cx = ctx + static_cast<long long>(b) * ctx_stride;
+  const int r = rows ? __ldg(rows + b) : 0;
+  const bool real = r >= 0 && r < S;                 // a pad row (r = -1) or a bad index reads / writes no pool byte
+  const int n = real ? min(min(max(__ldg(cx), 0), 31), ctx_stride - 2) : 0;
+  const int ws = min(max(__ldg(cx + 1), 0), slots - 1);
   const float sc = rsqrtf(static_cast<float>(dh)) * 1.4426950408889634f;
   const long long row2 = 2LL * C;
+  const long long hwl = hw;
+  T* cache = pool + (real ? static_cast<long long>(r) * slots * hwl * row2 : 0LL);
+  const T* cq = qkv + static_cast<long long>(b) * hwl * 3 * C;
+  T* co = out + static_cast<long long>(b) * hwl * C;
+
+  for (int i = threadIdx.x; i < (n + 1) * dh / 2; i += blockDim.x) {   // float4 i of the staged rows
+    const int j = i / (dh / 2), w = (i % (dh / 2)) * 4;
+    const int src = w < dh ? C + h * dh + w : 2 * C + h * dh + (w - dh);
+    spe4[i] = __ldg(reinterpret_cast<const float4*>(pe + static_cast<long long>(j) * 3 * C + src));
+  }
 
   float q[PPT][8], o[PPT][8], m[PPT], l[PPT];
   {
@@ -291,12 +321,12 @@ temporal_step_kernel(const T* __restrict__ qkv, T* __restrict__ cache, const flo
       const long long pos = p0 + i;
       uint4 uq = make_uint4(0, 0, 0, 0);
       if (act && pos < hw) {
-        const T* r = qkv + pos * 3 * C + col;
-        uq = __ldg(reinterpret_cast<const uint4*>(r));
-        if (ks == 0) {                               // the current frame's k'|v' go to the write slot unchanged
+        const T* rq = cq + pos * 3 * C + col;
+        uq = __ldg(reinterpret_cast<const uint4*>(rq));
+        if (ks == 0 && real) {                       // the current frame's k'|v' go to the write slot unchanged
           T* w = cache + (static_cast<long long>(ws) * hw + pos) * row2 + col;
-          *reinterpret_cast<uint4*>(w) = __ldg(reinterpret_cast<const uint4*>(r + C));
-          *reinterpret_cast<uint4*>(w + C) = __ldg(reinterpret_cast<const uint4*>(r + 2 * C));
+          *reinterpret_cast<uint4*>(w) = __ldg(reinterpret_cast<const uint4*>(rq + C));
+          *reinterpret_cast<uint4*>(w + C) = __ldg(reinterpret_cast<const uint4*>(rq + 2 * C));
         }
       }
       float fq[8];
@@ -310,24 +340,25 @@ temporal_step_kernel(const T* __restrict__ qkv, T* __restrict__ cache, const flo
       l[i] = 0.f;
     }
   }
+  __syncthreads();
   // ---- keys ks, ks + KS, ... of the sequence: context positions 0..n-1 (cache), then the current frame (position n) ----
 #pragma unroll 2
   for (int jb = 0; jb <= n; jb += KS) {             // (warp-uniform trip count: the shuffles need every lane)
     const int j = min(jb + ks, n);
     const bool valid = jb + ks <= n, cur = j == n;
-    const int slot = cur ? 0 : min(max(__ldg(ctx + 2 + j), 0), slots - 1);
+    const int slot = cur ? 0 : min(max(__ldg(cx + 2 + j), 0), slots - 1);
     float pk[8], pv[8];
-    load_pe8(pe + static_cast<long long>(j) * 3 * C + C + col, pk);
-    load_pe8(pe + static_cast<long long>(j) * 3 * C + 2 * C + col, pv);
+    lds_pe8(spe + j * 2 * dh + sco, pk);
+    lds_pe8(spe + j * 2 * dh + dh + sco, pv);
     uint4 uk[PPT], uv[PPT];
 #pragma unroll
     for (int i = 0; i < PPT; ++i) {
       const long long pos = p0 + i;
       uk[i] = uv[i] = make_uint4(0, 0, 0, 0);
       if (act && pos < hw) {
-        const T* r = cur ? qkv + pos * 3 * C + C + col : cache + (static_cast<long long>(slot) * hw + pos) * row2 + col;
-        uk[i] = __ldg(reinterpret_cast<const uint4*>(r));
-        uv[i] = __ldg(reinterpret_cast<const uint4*>(r + C));
+        const T* rk = cur ? cq + pos * 3 * C + C + col : cache + (static_cast<long long>(slot) * hw + pos) * row2 + col;
+        uk[i] = __ldg(reinterpret_cast<const uint4*>(rk));
+        uv[i] = __ldg(reinterpret_cast<const uint4*>(rk + C));
       }
     }
 #pragma unroll
@@ -375,52 +406,78 @@ temporal_step_kernel(const T* __restrict__ qkv, T* __restrict__ cache, const flo
       u.y = H16<T>::pack2(o[i][2] * inv, o[i][3] * inv);
       u.z = H16<T>::pack2(o[i][4] * inv, o[i][5] * inv);
       u.w = H16<T>::pack2(o[i][6] * inv, o[i][7] * inv);
-      *reinterpret_cast<uint4*>(out + pos * C + col) = u;
+      *reinterpret_cast<uint4*>(co + pos * C + col) = u;
     }
   }
 }
 
+struct StepArgs {
+  const void* qkv;
+  void* pool;
+  const float* pe;
+  const int32_t* rows;
+  const int32_t* ctx;
+  void* out;
+  int B, S, ctx_stride, hw, C, heads, slots;
+};
+
 template <typename T, int G>
-static int launch_step(const void* qkv, void* cache, const float* pe, const int32_t* ctx, void* out, int hw, int C,
-                       int heads, int slots, cudaStream_t st) {
+static int launch_step(const StepArgs& a, cudaStream_t st) {
   constexpr int PPT = 2;
-  const long long threads = static_cast<long long>((hw + PPT - 1) / PPT) * heads * 32;
-  const int blocks = static_cast<int>((threads + 255) / 256);
-  temporal_step_kernel<T, G, PPT><<<blocks, 256, 0, st>>>(static_cast<const T*>(qkv), static_cast<T*>(cache), pe, ctx,
-                                                          static_cast<T*>(out), hw, C, heads, slots);
+  const int tiles = (a.hw + STEP_WARPS * PPT - 1) / (STEP_WARPS * PPT);
+  const dim3 grid(static_cast<unsigned>(tiles * a.heads), static_cast<unsigned>(a.B));
+  const size_t smem = static_cast<size_t>(32) * 2 * (a.C / a.heads) * sizeof(float);   // <= 32 KB (dh <= 128)
+  temporal_step_kernel<T, G, PPT><<<grid, STEP_WARPS * 32, smem, st>>>(
+      static_cast<const T*>(a.qkv), static_cast<T*>(a.pool), a.pe, a.rows, a.ctx, static_cast<T*>(a.out), a.hw, a.C,
+      a.heads, a.S, a.slots, a.ctx_stride);
   VDA_CUDA(cudaGetLastError());
   return 0;
 }
 
 template <typename T>
-static int dispatch_step(const void* qkv, void* cache, const float* pe, const int32_t* ctx, void* out, int hw, int C,
-                         int heads, int slots, cudaStream_t st) {
-  const int chunks = C / heads / 8;
-  if (chunks <= 1) return launch_step<T, 1>(qkv, cache, pe, ctx, out, hw, C, heads, slots, st);
-  if (chunks <= 2) return launch_step<T, 2>(qkv, cache, pe, ctx, out, hw, C, heads, slots, st);
-  if (chunks <= 4) return launch_step<T, 4>(qkv, cache, pe, ctx, out, hw, C, heads, slots, st);
-  if (chunks <= 8) return launch_step<T, 8>(qkv, cache, pe, ctx, out, hw, C, heads, slots, st);
-  return launch_step<T, 16>(qkv, cache, pe, ctx, out, hw, C, heads, slots, st);
+static int dispatch_step(const StepArgs& a, cudaStream_t st) {
+  const int chunks = a.C / a.heads / 8;
+  if (chunks <= 1) return launch_step<T, 1>(a, st);
+  if (chunks <= 2) return launch_step<T, 2>(a, st);
+  if (chunks <= 4) return launch_step<T, 4>(a, st);
+  if (chunks <= 8) return launch_step<T, 8>(a, st);
+  return launch_step<T, 16>(a, st);
+}
+
+static int temporal_step(const StepArgs& a, int dtype, void* stream) {
+  VDA_CHECK(dtype == VDA_BF16 || dtype == VDA_FP16, "bad dtype %d", dtype);
+  VDA_CHECK(a.hw > 0, "temporal step: hw must be positive, got %d", a.hw);
+  VDA_CHECK(a.C % 8 == 0 && a.C % a.heads == 0 && (a.C / a.heads) % 8 == 0 && a.heads <= 8 && a.C / a.heads <= 128,
+            "bad channel/head split C=%d heads=%d (head dim must be a multiple of 8, <= 128; heads <= 8)", a.C, a.heads);
+  VDA_CHECK(a.slots >= 2 && a.slots <= 32, "temporal step: the cache holds 2..32 frame slots, got %d", a.slots);
+  VDA_CHECK(a.B >= 1 && a.B <= 65535, "temporal step: 1..65535 batch rows, got %d", a.B);
+  VDA_CHECK(a.S >= 1, "temporal step: the pool needs at least one entry, got %d", a.S);
+  VDA_CHECK(a.ctx_stride >= 2, "temporal step: a context row holds at least {n_ctx, write slot}, got stride %d",
+            a.ctx_stride);
+  VDA_CHECK(a.qkv && a.pool && a.pe && a.ctx && a.out, "temporal step: null pointer");
+  VDA_CHECK(((reinterpret_cast<uintptr_t>(a.qkv) | reinterpret_cast<uintptr_t>(a.pool) |
+              reinterpret_cast<uintptr_t>(a.pe) | reinterpret_cast<uintptr_t>(a.out)) & 15) == 0,
+            "qkv/cache/pe/out must be 16-byte aligned");
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  if (dtype == VDA_BF16) return dispatch_step<__nv_bfloat16>(a, st);
+  return dispatch_step<__half>(a, st);
 }
 
 }  // namespace vda
 
 using namespace vda;
 
+extern "C" int vda_attention_temporal_step_batched(const void* qkv, void* pool, const float* pe, const int32_t* rows,
+                                                   const int32_t* ctx, void* out, int B, int S, int ctx_stride, int hw,
+                                                   int C, int heads, int slots, int dtype, void* stream) {
+  VDA_CHECK(rows, "temporal step: null row table");
+  return temporal_step({qkv, pool, pe, rows, ctx, out, B, S, ctx_stride, hw, C, heads, slots}, dtype, stream);
+}
+
 extern "C" int vda_attention_temporal_step(const void* qkv, void* cache, const float* pe, const int32_t* ctx, void* out,
                                            int hw, int C, int heads, int slots, int dtype, void* stream) {
-  VDA_CHECK(dtype == VDA_BF16 || dtype == VDA_FP16, "bad dtype %d", dtype);
-  VDA_CHECK(hw > 0, "temporal step: hw must be positive, got %d", hw);
-  VDA_CHECK(C % 8 == 0 && C % heads == 0 && (C / heads) % 8 == 0 && heads <= 8 && C / heads <= 128,
-            "bad channel/head split C=%d heads=%d (head dim must be a multiple of 8, <= 128; heads <= 8)", C, heads);
-  VDA_CHECK(slots >= 2 && slots <= 32, "temporal step: the cache holds 2..32 frame slots, got %d", slots);
-  VDA_CHECK(qkv && cache && pe && ctx && out, "temporal step: null pointer");
-  VDA_CHECK(((reinterpret_cast<uintptr_t>(qkv) | reinterpret_cast<uintptr_t>(cache) | reinterpret_cast<uintptr_t>(pe) |
-              reinterpret_cast<uintptr_t>(out)) & 15) == 0,
-            "qkv/cache/pe/out must be 16-byte aligned");
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
-  if (dtype == VDA_BF16) return dispatch_step<__nv_bfloat16>(qkv, cache, pe, ctx, out, hw, C, heads, slots, st);
-  return dispatch_step<__half>(qkv, cache, pe, ctx, out, hw, C, heads, slots, st);
+  // one row, pool entry 0; a stride of 2 + 31 keeps n_ctx's clamp at 31
+  return temporal_step({qkv, cache, pe, nullptr, ctx, out, 1, 1, 33, hw, C, heads, slots}, dtype, stream);
 }
 
 extern "C" int vda_attention_temporal(const void* qkv, void* out, int T, int hw, int C, int heads, int dtype,

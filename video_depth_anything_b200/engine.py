@@ -98,7 +98,6 @@ class Engine:
         self._pos_cache: Dict[tuple, torch.Tensor] = {}
         self.loaded = False
         self.generation = 0          # bumped by every load(): streams opened on older weights refuse to continue
-        self._stream_serial = 0
         # One CUDA graph per input shape: a forward is ~330 back-to-back kernel launches with no host decisions,
         # so it is captured once and replayed (removes launch gaps and the host-side descriptor encoding).
         self.use_graphs = os.environ.get("VDA_NO_GRAPH", "0") != "1"
@@ -354,8 +353,8 @@ class Engine:
 
     def _motion(self, m, x, B, T, hw, stream=None):
         """TemporalModule (motion_module.py:60-65, 102-126, 164-177).  x h16 [B*T*hw, C] rows (b, f, pos).
-        `stream` = (caches, ctx): one streamed frame (B = T = 1) whose temporal attention reads the stream's cached
-        frames (stream_step)."""
+        `stream` = (pool, rows, ctx): one streamed frame per batch row (T = 1) whose temporal attention reads its
+        stream's cached frames (stream_group_step)."""
         w, C = self.w, self.mm_c[m]
         M = B * T * hw
         p = f"mm{m}."
@@ -377,7 +376,7 @@ class Engine:
             else:                                          # positional encoding enters through the `pet` table
                 ops.layernorm(h, w[f"{p}a{a}.ln.w"], w[f"{p}a{a}.ln.b"], 1e-5, n)
                 ops.gemm(n, w[f"{p}a{a}.qkv.w"], qkv, bias=self._const(0.0, 3 * C))
-                ops.attention_temporal_step(qkv, stream[0][2 * m + a], w[f"{p}a{a}.pet"], stream[1], o)
+                ops.attention_temporal_step(qkv, stream[0][2 * m + a], w[f"{p}a{a}.pet"], stream[2], o, rows=stream[1])
             ops.gemm(o, w[f"{p}a{a}.o.w"], h, bias=w[f"{p}a{a}.o.b"], gamma=self._const(1.0, C), res1=h)   # unit LayerScale: ditto
         ops.layernorm(h, w[p + "ffn.w"], w[p + "ffn.b"], 1e-5, n)                        # :174
         g = self._hnew(M, 4 * C)
@@ -474,13 +473,18 @@ class Engine:
         return self._forward_eager(x, stages)
 
     def _graphed(self, key: tuple, fn, inputs: List[torch.Tensor], adopt: bool = False):
+        """Run `fn(*inputs)` as a CUDA graph captured once per `key` in the engine's own bounded cache (run_graphed)."""
+        if key not in self._graphs and len(self._graphs) >= 6:   # bound the memory held by private graph pools
+            self._graphs.pop(next(iter(self._graphs)))
+        return self.run_graphed(self._graphs, key, fn, inputs, adopt)
+
+    @staticmethod
+    def run_graphed(graphs: Dict[tuple, tuple], key: tuple, fn, inputs: List[torch.Tensor], adopt: bool = False):
         """Run `fn(*inputs)` (a fixed sequence of libvda launches, no host decisions) as a CUDA graph captured once
-        per `key`; returns the graph's static outputs (valid until the next call with the same key).  `adopt`: the
-        caller's tensors are long-lived buffers and become the graph's inputs themselves (no staging copy)."""
-        entry = self._graphs.get(key)
+        per `key` into `graphs`; returns the graph's static outputs (valid until the next call with the same key).
+        `adopt`: the caller's tensors are long-lived buffers and become the graph's inputs themselves (no staging copy)."""
+        entry = graphs.get(key)
         if entry is None:
-            if len(self._graphs) >= 6:                      # bound the memory held by private graph pools
-                self._graphs.pop(next(iter(self._graphs)))
             static_in = list(inputs) if adopt else [t.clone() for t in inputs]
             n0 = ops.LAUNCHES
             fn(*static_in)                                  # warm-up: lazy caches, kernel attributes
@@ -492,7 +496,7 @@ class Engine:
             # invalidates the capture, although it never touches the capturing stream
             with torch.cuda.graph(graph, capture_error_mode="thread_local"):
                 static_out = fn(*static_in)
-            entry = self._graphs[key] = (graph, static_in, static_out, launches)
+            entry = graphs[key] = (graph, static_in, static_out, launches)
         graph, static_in, static_out, launches = entry
         for s, t in zip(static_in, inputs):
             if s.data_ptr() != t.data_ptr():
@@ -545,41 +549,23 @@ class Engine:
         return depth.view(B, T, H, W)
 
     # ------------------------------------------------------------------------------------------- streaming
-    def stream_cache(self, hp: int, wp: int, slots: int) -> List[torch.Tensor]:
-        """Per temporal-attention block (index 2 * motion module + attention block) the k'|v' rows of `slots` frames:
-        head dtype [slots, hw, 2C], row = k' (C) | v' (C) of one position, so one head's keys and values are contiguous
-        16-byte runs."""
+    def stream_pool(self, S: int, hp: int, wp: int, slots: int) -> List[torch.Tensor]:
+        """Temporal context of S streams.  Per temporal-attention block (index 2 * motion module + attention block) the
+        k'|v' rows of `slots` frames of every stream: head dtype [S, slots, hw, 2C], row = k' (C) | v' (C) of one
+        position, so one head's keys and values are contiguous 16-byte runs."""
         hws = [hp * wp, ((hp - 1) // 2 + 1) * ((wp - 1) // 2 + 1), hp * wp, 4 * hp * wp]
-        return [self._hnew(slots, hws[m], 2 * self.mm_c[m]) for m in range(4) for _ in (0, 1)]
+        return [self._hnew(S, slots, hws[m], 2 * self.mm_c[m]) for m in range(4) for _ in (0, 1)]
 
-    def stream_step(self, frame: torch.Tensor, ctx: torch.Tensor, cache: List[torch.Tensor], nh: int, nw: int) -> torch.Tensor:
-        """One streamed frame: uint8 [H0,W0,3] (device) -> fp32 depth [H0,W0] (>= 0).  Preprocessing as in
-        infer_video_depth, encoder and head at T = 1 with every temporal attention against `cache` as `ctx` describes
-        (vda_attention_temporal_step), bilinear resize to the frame size.  No host decisions: graph-capturable."""
-        h0, w0 = frame.shape[:2]
-        key = ("idx0",)
-        if key not in self._bufs:
-            self._bufs[key] = [torch.zeros(1, dtype=torch.int32, device=self.device)]
-        x = ops.preprocess_frames(frame.unsqueeze(0), self._bufs[key][0], nh, nw)
-        d = self.head(self.encode(x), 1, 1, nh // 14, nw // 14, stream=(cache, ctx))
+    def stream_group_step(self, frames: torch.Tensor, idx: torch.Tensor, rows: torch.Tensor, ctx: torch.Tensor,
+                          pool: List[torch.Tensor], nh: int, nw: int) -> torch.Tensor:
+        """One streamed frame of each of B streams: frames uint8 [*,H0,W0,3] (device), batch row b takes frame idx[b]
+        (int32 [B]), pool entry rows[b] (int32 [B], -1: pad row) and context row ctx[b] (int32 [B, stride], see
+        vda_attention_temporal_step_batched) -> fp32 depth [B,H0,W0] (>= 0).  Preprocessing as in infer_video_depth,
+        encoder and head on the B frames at T = 1 with every temporal attention against the rows' pool entries,
+        bilinear resize to the frame size.  The launches do not depend on B.  No host decisions: graph-capturable."""
+        h0, w0 = frames.shape[1:3]
+        x = ops.preprocess_frames(frames, idx, nh, nw)
+        d = self.head(self.encode(x), idx.numel(), 1, nh // 14, nw // 14, stream=(pool, rows, ctx))
         if (nh, nw) != (h0, w0):
             d = ops.bilinear_f32(d, h0, w0)
-        return d[0]
-
-    def new_stream_id(self) -> int:
-        self._stream_serial += 1
-        return self._stream_serial
-
-    def stream_step_graphed(self, sid: int, frame: torch.Tensor, ctx: torch.Tensor, cache: List[torch.Tensor], nh: int,
-                            nw: int) -> torch.Tensor:
-        """stream_step as a CUDA graph captured once per stream `sid` (its cache pointers are part of the graph); `frame`
-        and `ctx` are the stream's own long-lived input buffers.  Returns the graph's static output."""
-        if self.use_graphs and ops.PROFILE is None:
-            return self._graphed(("stream", sid, nh, nw) + tuple(frame.shape), lambda f, c: self.stream_step(f, c, cache, nh, nw),
-                                 [frame, ctx], adopt=True)
-        return self.stream_step(frame, ctx, cache, nh, nw)
-
-    def drop_stream(self, sid: int) -> None:
-        """Forget the graphs of stream `sid` (they hold its cache)."""
-        for k in [k for k in self._graphs if k[0] == "stream" and k[1] == sid]:
-            del self._graphs[k]
+        return d

@@ -200,23 +200,35 @@ def attention_temporal(qkv: torch.Tensor, out: torch.Tensor, T: int, hw: int, Cc
 
 
 def attention_temporal_step(qkv: torch.Tensor, cache: torch.Tensor, pe: torch.Tensor, ctx: torch.Tensor, out: torch.Tensor,
-                            heads: int = 8):
-    """Streaming temporal attention of one frame (vda.h vda_attention_temporal_step): qkv h16 [hw, 3C] (q'|k'|v', no
-    positional encoding), cache h16 [slots, hw, 2C] (k'|v' rows of earlier frames), pe fp32 [32, 3C] (positional share of
-    q|k|v), ctx device int32 [>= 2] = (n_ctx, write slot, context slots...) -> out h16 [hw, C]."""
+                            heads: int = 8, rows: Optional[torch.Tensor] = None):
+    """Streaming temporal attention (vda.h vda_attention_temporal_step[_batched]).  One frame: qkv h16 [hw, 3C] (q'|k'|v',
+    no positional encoding), cache h16 [slots, hw, 2C] (k'|v' rows of earlier frames), pe fp32 [32, 3C] (positional share
+    of q|k|v), ctx device int32 [>= 2] = (n_ctx, write slot, context slots...) -> out h16 [hw, C].
+    B frames of different streams (`rows` device int32 [B], pool index per batch row, -1 = pad row): qkv [B*hw, 3C],
+    cache = the pool h16 [S, slots, hw, 2C], ctx [B, stride] one row as above per batch row -> out [B*hw, C]."""
     lib = _lib.load()
-    hw, C3 = qkv.shape
+    C3 = qkv.shape[1]
     Cc = C3 // 3
-    slots = cache.shape[0]
+    B = 1 if rows is None else rows.numel()
+    hw = qkv.shape[0] // B
     assert qkv.is_contiguous() and cache.is_contiguous() and pe.is_contiguous() and out.is_contiguous()
-    assert cache.shape[1:] == (hw, 2 * Cc) and cache.dtype == qkv.dtype and out.dtype == qkv.dtype
+    assert cache.shape[-2:] == (hw, 2 * Cc) and cache.dtype == qkv.dtype and out.dtype == qkv.dtype
+    assert qkv.shape[0] == B * hw and out.shape == (B * hw, Cc)
     assert pe.dtype == torch.float32 and pe.shape[-1] == C3 and pe.shape[0] >= 32
     assert ctx.dtype == torch.int32 and ctx.is_contiguous() and ctx.numel() >= 2
     if PROFILE is not None:      # bytes of a full 31-frame context: cached k'|v' rows read, current q|k|v in, out + slot out
         _INFO.update(kind="attention_temporal_step",
-                     bytes=float(qkv.element_size() * hw * (31 * 2 * Cc + 3 * Cc + Cc + 2 * Cc)))
-    check(lib.vda_attention_temporal_step(_p(qkv), _p(cache), _p(pe), _p(ctx), _p(out), hw, Cc, heads, slots,
-                                          dt_code(qkv.dtype), _stream()))
+                     bytes=float(qkv.element_size() * B * hw * (31 * 2 * Cc + 3 * Cc + Cc + 2 * Cc)))
+    if rows is None:
+        assert cache.dim() == 3
+        check(lib.vda_attention_temporal_step(_p(qkv), _p(cache), _p(pe), _p(ctx), _p(out), hw, Cc, heads,
+                                              cache.shape[0], dt_code(qkv.dtype), _stream()))
+    else:
+        assert cache.dim() == 4 and rows.dtype == torch.int32 and rows.is_contiguous() and ctx.dim() == 2
+        assert ctx.shape[0] == B
+        check(lib.vda_attention_temporal_step_batched(_p(qkv), _p(cache), _p(pe), _p(rows), _p(ctx), _p(out), B,
+                                                      cache.shape[0], ctx.shape[1], hw, Cc, heads, cache.shape[1],
+                                                      dt_code(qkv.dtype), _stream()))
     _count()
     return out
 

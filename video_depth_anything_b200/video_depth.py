@@ -26,7 +26,8 @@ from . import ops
 from .engine import Engine
 from .synth import ENCODER_DIMS, synth_state_dict
 from .windows import (INFER_LEN, INTERP_LEN, KEYFRAMES, OVERLAP, aligner_ring_len, aligner_ring_pos, get_resize_hw,
-                      plan_feature_cache, stream_context, upload_ring_plan, window_source_indices)
+                      StreamGroupPlan, plan_feature_cache, split_group_table, upload_ring_plan,
+                      window_source_indices)
 
 
 VALIDATION_DTYPE = torch.float16     # operand type of the `fp32=True` path (see _ensure_engine)
@@ -201,6 +202,12 @@ class VideoDepthAnything(nn.Module):
         `forward` / `infer_video_depth`; `fp32=True` selects the validation-precision engine as in infer_video_depth."""
         return DepthStream(self, self._ensure_engine(validation=bool(fp32)), input_size)
 
+    def stream_group(self, max_streams: int = 8, input_size: int = 518, fp32: bool = False) -> "DepthStreamGroup":
+        """Open a group of up to `max_streams` depth streams (several cameras) on this model's device: each `push` takes
+        one frame of any subset of the group's open streams and runs them as one batched step (DepthStreamGroup).  Every
+        stream behaves as a DepthStream of its own; `fp32=True` selects the validation-precision engine."""
+        return DepthStreamGroup(self, self._ensure_engine(validation=bool(fp32)), max_streams, input_size)
+
     @torch.no_grad()
     def infer_video_depth_one(self, frame: np.ndarray, input_size: int = 518, device="cuda", fp32: bool = False) -> np.ndarray:
         """Depth of the next frame of the model's own stream (the name of the upstream project's streaming entry
@@ -218,6 +225,116 @@ class VideoDepthAnything(nn.Module):
         return st.push(frame)
 
 
+class DepthStreamGroup:
+    """Streaming inference for many live streams (cameras) on one model: every push runs the frames of all the streams
+    it names as one batched step.
+
+    Each stream follows DepthStream's semantics exactly, with its own step counter t and its own temporal context
+    (windows.stream_context over its own row of a pooled k'|v' cache).  A push names any subset of the open streams,
+    each at most once; a stream left out does not advance.  The batch is padded up to a bucket (the powers of two below
+    `max_streams`, then `max_streams`; windows.stream_buckets): pad rows take the first frame and pool row -1, which
+    reads and writes no pool byte.  One CUDA graph per bucket, captured on first use and owned by the group (the
+    engine's forward / video graphs neither evict nor are evicted by them).  A push is one H2D of the frames, one H2D of
+    the int32 rows | ctx | idx table, a replay and one D2H of [bucket, H0, W0].
+
+    Device memory: the pool holds max_streams x (L + 1) = 32 frame slots per temporal-attention block, allocated at the
+    first push: 903 MB per stream for ViT-L at 518x518 (214 MB for ViT-S), plus one graph's activations per bucket used.
+    Frame size (and so the network size) is fixed by the first push, for every stream of the group."""
+
+    def __init__(self, model: VideoDepthAnything, engine: Engine, max_streams: int = 8, input_size: int = 518):
+        self.engine, self.input_size = engine, int(input_size)
+        self.device = engine.device
+        self.generation = engine.generation
+        L = model.num_frames - 1
+        if not 1 <= L <= INFER_LEN - 1:
+            raise ValueError(f"streaming needs num_frames in 2..{INFER_LEN}, got {model.num_frames}")
+        self.plan = StreamGroupPlan(int(max_streams), L)
+        self.max_streams = self.plan.max_streams
+        self.size = None                             # (h0, w0), fixed by the first push
+        self.pool = None
+        self.graphs = {}                             # bucket -> captured step (Engine.run_graphed)
+        self.closed = False
+
+    def open(self) -> int:
+        """A new stream starting at t = 0; returns its handle.  ValueError beyond `max_streams` open streams."""
+        if self.closed:
+            raise RuntimeError("open on a closed DepthStreamGroup")
+        return self.plan.open()
+
+    def close_stream(self, handle: int) -> None:
+        """Close one stream; its pool row is free for a later open (which starts over at t = 0)."""
+        self.plan.close(handle)
+
+    def _alloc(self, h0: int, w0: int) -> None:
+        eng, S, L = self.engine, self.max_streams, self.plan.L
+        self.nh, self.nw = get_resize_hw(h0, w0, self.input_size)
+        with torch.cuda.device(self.device):
+            self.pool = eng.stream_pool(S, self.nh // 14, self.nw // 14, L + 1)
+            self.frames_dev = torch.empty(S, h0, w0, 3, dtype=torch.uint8, device=self.device)
+            self.table_dev = torch.zeros(S * (L + 4), dtype=torch.int32, device=self.device)
+            self.frames_host = torch.empty(S, h0, w0, 3, dtype=torch.uint8).pin_memory()
+            self.table_host = torch.zeros(S * (L + 4), dtype=torch.int32).pin_memory()
+            self.out_host = torch.empty(S, h0, w0, dtype=torch.float32).pin_memory()
+        self.size = (h0, w0)
+
+    def _step(self, bk: int) -> torch.Tensor:
+        eng = self.engine
+        rows, ctx, idx = split_group_table(self.table_dev, bk, self.plan.L)
+        inputs = [self.frames_dev, idx, rows, ctx]
+
+        def fn(frames, idx, rows, ctx):
+            return eng.stream_group_step(frames, idx, rows, ctx, self.pool, self.nh, self.nw)
+        if eng.use_graphs and ops.PROFILE is None:
+            return eng.run_graphed(self.graphs, bk, fn, inputs, adopt=True)
+        return fn(*inputs)
+
+    @torch.no_grad()
+    def push(self, frames) -> dict:
+        """frames: {handle: uint8 RGB [H0,W0,3]} (or (handle, frame) pairs) -> {handle: depth float32 [H0,W0] (>= 0)},
+        fresh arrays."""
+        if self.closed:
+            raise RuntimeError("push on a closed DepthStreamGroup")
+        if self.engine.generation != self.generation or not self.engine.loaded:
+            raise RuntimeError("the model's weights changed since this stream group was opened; open a new one")
+        items = list(frames.items()) if isinstance(frames, dict) else list(frames)
+        size = self.size
+        for _, f in items:
+            if not isinstance(f, np.ndarray) or f.ndim != 3 or f.shape[2] != 3 or f.dtype != np.uint8:
+                raise ValueError("a frame must be a uint8 numpy array [H0,W0,3]")
+            size = size or tuple(f.shape[:2])
+            if tuple(f.shape[:2]) != size:
+                raise ValueError(f"frame size {tuple(f.shape[:2])} differs from the group's {size}")
+        handles = [h for h, _ in items]
+        bk, table = self.plan.step(handles)          # ValueError: empty push, unknown / closed / repeated handle
+        if self.size is None:
+            self._alloc(*size)
+        n = len(items)
+        np.copyto(self.table_host.numpy()[:table.size], table)
+        fh = self.frames_host.numpy()
+        for i, (_, f) in enumerate(items):
+            np.copyto(fh[i], f)
+        with torch.cuda.device(self.device):
+            self.frames_dev[:n].copy_(self.frames_host[:n], non_blocking=True)
+            self.table_dev[:table.size].copy_(self.table_host[:table.size], non_blocking=True)
+            d = self._step(bk)
+            self.out_host[:bk].copy_(d, non_blocking=True)
+            torch.cuda.current_stream().synchronize()   # (also: the pinned inputs are free for the next push)
+        out = self.out_host.numpy()
+        return {h: out[i].copy() for i, h in enumerate(handles)}
+
+    def close(self) -> None:
+        """Release the group's graphs and pool (also done when the object is collected)."""
+        self.graphs = {}
+        self.pool = None
+        self.closed = True
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:                                # noqa: BLE001  (interpreter shutdown)
+            pass
+
+
 class DepthStream:
     """Streaming inference: one frame in, its depth out, with a cached temporal context.
 
@@ -231,73 +348,22 @@ class DepthStream:
 
     A cached frame is kept as its k'|v' = LayerNorm output @ [W_k | W_v]^T rows, without the positional encoding, whose
     share is added by the step kernel at the frame's current position: a step never re-projects old frames.  Device
-    memory is bounded: L + 1 cache slots per block.  The whole step (preprocess, encoder, head, resize) is one CUDA graph
-    per stream; a push is one H2D of the frame and of the <= 33-int context, a replay and one D2H of the depth.
-    Frame size (and so the network size) is fixed by the first frame."""
+    memory is bounded: L + 1 cache slots per block.  A DepthStream is a DepthStreamGroup of one stream: the whole step
+    (preprocess, encoder, head, resize) is one CUDA graph; a push is one H2D of the frame and of the context, a replay
+    and one D2H of the depth.  Frame size (and so the network size) is fixed by the first frame."""
 
     def __init__(self, model: VideoDepthAnything, engine: Engine, input_size: int = 518):
-        self.model, self.engine, self.input_size = model, engine, int(input_size)
-        self.device = engine.device
-        self.generation = engine.generation
-        self.L = model.num_frames - 1
-        if not 1 <= self.L <= INFER_LEN - 1:
-            raise ValueError(f"streaming needs num_frames in 2..{INFER_LEN}, got {model.num_frames}")
-        self.sid = engine.new_stream_id()
-        self.t = 0                                   # frames pushed so far
-        self.size = None                             # (h0, w0), fixed by the first frame
-        self.cache = None
-        self.closed = False
+        self.group = DepthStreamGroup(model, engine, 1, input_size)
+        self.engine, self.input_size, self.generation = engine, self.group.input_size, self.group.generation
+        self.handle = self.group.open()
 
-    def _open(self, h0: int, w0: int) -> None:
-        eng = self.engine
-        self.nh, self.nw = get_resize_hw(h0, w0, self.input_size)
-        with torch.cuda.device(self.device):
-            self.cache = eng.stream_cache(self.nh // 14, self.nw // 14, self.L + 1)
-            self.frame_dev = torch.empty(h0, w0, 3, dtype=torch.uint8, device=self.device)
-            self.ctx_dev = torch.zeros(2 + self.L, dtype=torch.int32, device=self.device)
-            self.frame_host = torch.empty(h0, w0, 3, dtype=torch.uint8).pin_memory()
-            self.ctx_host = torch.zeros(2 + self.L, dtype=torch.int32).pin_memory()
-            self.out_host = torch.empty(h0, w0, dtype=torch.float32).pin_memory()
-        self.size = (h0, w0)
-
-    @torch.no_grad()
     def push(self, frame: np.ndarray) -> np.ndarray:
         """frame uint8 RGB [H0,W0,3] -> its depth float32 [H0,W0] (>= 0); a fresh array on every call."""
-        if not isinstance(frame, np.ndarray) or frame.ndim != 3 or frame.shape[2] != 3 or frame.dtype != np.uint8:
-            raise ValueError("frame must be a uint8 numpy array [H0,W0,3]")
-        if self.closed:
-            raise RuntimeError("push on a closed DepthStream")
-        if self.engine.generation != self.generation or not self.engine.loaded:
-            raise RuntimeError("the model's weights changed since this stream was opened; open a new stream")
-        if self.size is None:
-            self._open(*frame.shape[:2])
-        elif tuple(frame.shape[:2]) != self.size:
-            raise ValueError(f"frame size {tuple(frame.shape[:2])} differs from the stream's {self.size}")
-        _, slots, write = stream_context(self.t, self.L)
-        ctx = self.ctx_host.numpy()
-        ctx[0], ctx[1] = len(slots), write
-        ctx[2:2 + len(slots)] = slots
-        np.copyto(self.frame_host.numpy(), frame)
-        with torch.cuda.device(self.device):
-            self.frame_dev.copy_(self.frame_host, non_blocking=True)
-            self.ctx_dev.copy_(self.ctx_host, non_blocking=True)
-            d = self.engine.stream_step_graphed(self.sid, self.frame_dev, self.ctx_dev, self.cache, self.nh, self.nw)
-            self.out_host.copy_(d, non_blocking=True)
-            torch.cuda.current_stream().synchronize()   # (also: the pinned inputs are free for the next push)
-        self.t += 1
-        return self.out_host.numpy().copy()
+        return self.group.push([(self.handle, frame)])[self.handle]
 
     def close(self) -> None:
         """Release the stream's graph and cache (also done when the object is collected)."""
-        self.engine.drop_stream(self.sid)
-        self.cache = None
-        self.closed = True
-
-    def __del__(self):
-        try:
-            self.close()
-        except Exception:                                # noqa: BLE001  (interpreter shutdown)
-            pass
+        self.group.close()
 
 
 class FeatureCache:

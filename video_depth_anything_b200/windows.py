@@ -152,3 +152,76 @@ def stream_context(t: int, L: int = STREAM_CONTEXT):
 
     ids = [] if t == 0 else [0] + list(range(max(1, t - L + 1), t))
     return ids, [slot(j) for j in ids], slot(t)
+
+
+# ------------------------------------------------------------------------------------------------
+# stream groups (video_depth.DepthStreamGroup): handles, pool rows, per-stream steps, buckets and the per-push table
+# ------------------------------------------------------------------------------------------------
+def stream_buckets(max_streams: int):
+    """Batch sizes a group of at most `max_streams` streams runs at: the powers of two below it, then itself."""
+    if max_streams < 1:
+        raise ValueError(f"a stream group needs max_streams >= 1, got {max_streams}")
+    return [1 << i for i in range(max_streams.bit_length()) if 1 << i < max_streams] + [max_streams]
+
+
+class StreamGroupPlan:
+    """Host state of a stream group.  Every open stream has a handle (never reused), a pool row (the lowest free one;
+    reused after close) and its own step counter t, which only a push that names it advances.  `step(handles)` returns
+    the push's bucket and its int32 table rows [bucket] | ctx [bucket, 2 + L] | idx [bucket]: batch row i < len(handles)
+    is stream handles[i] with pool row, stream_context(t, L) as {n_ctx, write slot, context slots...} and frame i;
+    the pad rows behind it take pool row -1, n_ctx = 0 and frame 0."""
+
+    def __init__(self, max_streams: int, L: int = STREAM_CONTEXT):
+        self.buckets = stream_buckets(max_streams)
+        self.max_streams, self.L = max_streams, L
+        self.stride = 2 + L
+        self.row, self.t = {}, {}                      # handle -> pool row, handle -> frames pushed so far
+        self._next = 0
+
+    def open(self) -> int:
+        if len(self.row) >= self.max_streams:
+            raise ValueError(f"the group already holds its max_streams={self.max_streams} streams")
+        used = set(self.row.values())
+        h = self._next
+        self._next += 1
+        self.row[h] = min(r for r in range(self.max_streams) if r not in used)
+        self.t[h] = 0
+        return h
+
+    def check(self, h) -> None:
+        if h not in self.row:
+            raise ValueError(f"unknown or closed stream handle {h!r}")
+
+    def close(self, h) -> None:
+        self.check(h)
+        del self.row[h], self.t[h]
+
+    def bucket(self, n: int) -> int:
+        return next(b for b in self.buckets if b >= n)
+
+    def step(self, handles):
+        """Table of one push of `handles` (distinct open streams, in batch-row order); advances their t."""
+        for h in handles:
+            self.check(h)
+        if len(set(handles)) != len(handles):
+            raise ValueError("a stream is named more than once in one push")
+        if not handles:
+            raise ValueError("a push names at least one stream")
+        bk = self.bucket(len(handles))
+        rows = np.full(bk, -1, np.int32)
+        ctx = np.zeros((bk, self.stride), np.int32)
+        idx = np.zeros(bk, np.int32)
+        for i, h in enumerate(handles):
+            _, slots, write = stream_context(self.t[h], self.L)
+            rows[i], idx[i] = self.row[h], i
+            ctx[i, 0], ctx[i, 1] = len(slots), write
+            ctx[i, 2:2 + len(slots)] = slots
+        for h in handles:
+            self.t[h] += 1
+        return bk, np.concatenate([rows, ctx.ravel(), idx])
+
+
+def split_group_table(table, bk: int, L: int = STREAM_CONTEXT):
+    """Views (rows [bk], ctx [bk, 2 + L], idx [bk]) of a StreamGroupPlan table (numpy array or tensor)."""
+    s = 2 + L
+    return table[:bk], table[bk:bk + bk * s].reshape(bk, s), table[bk + bk * s:bk * (s + 2)]
