@@ -66,31 +66,11 @@ def run_temporal(T, hw, C, dt, iters=10):
     print(f"temporal attn T={T} hw={hw} C={C} {dt}: {ms * 1e3:.1f} us  {gb / ms * 1e3:.0f} GB/s (q,k,v,o)  max abs err {err:.3e}", flush=True)
 
 
-def timing_report(steps):
-    """Per-phase cycle sums of CTA 0's softmax warps (only in a -DVDA_SA_TIMING build)."""
-    import ctypes as C
-    from video_depth_anything_b200 import _lib
-    lib = C.CDLL(_lib.LIB_PATH)
-    if not hasattr(lib, "vda_debug_sa_timing"):
-        return
-    buf = (C.c_ulonglong * 24)()
-    lib.vda_debug_sa_timing(buf)
-    names = ["wait S", "ld S+max", "rescale chk", "exp rest", "exp0+o_done", "st P tail", "epilogue", "loop"]
-    for t in range(2):
-        tot = sum(buf[t * 8 + k] for k in range(8))
-        print(f"  WG{t}: total {tot} cyc, per step {tot / steps:.0f}: " +
-              ", ".join(f"{n} {buf[t * 8 + k] / steps:.0f}" for k, n in enumerate(names)))
-
 if __name__ == "__main__":
     if len(sys.argv) > 1 and sys.argv[1] == "temporal":
         for hw, C in ((1369, 1024), (361, 1024), (1369, 256), (5476, 256), (1369, 192), (361, 384), (5476, 64)):
             run_temporal(32, hw, C, torch.bfloat16)
         run_temporal(8, 100, 256, torch.float16)
-        sys.exit(0)
-    if len(sys.argv) > 1 and sys.argv[1] == "timing":
-        run(8, 1370, 16, torch.bfloat16, iters=1, check=False)
-        # CTA 0 of 148 handles items 0,148,...: 768 items -> 6 items (5 full + 1 half) -> 66 / 55 steps
-        timing_report(61)   # (5 pairs x 11 + the split item's 6 / 5 steps)
         sys.exit(0)
     if len(sys.argv) > 1 and sys.argv[1] == "prof32":    # the benchmarked shape, one warm-up + one launch (ncu -s 1 -c 1)
         run(32, 1370, 16, torch.bfloat16, iters=1, check=False)

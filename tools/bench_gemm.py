@@ -1,6 +1,6 @@
 #!/usr/bin/env python
 """Micro-benchmark of the tcgen05 GEMM / implicit-conv kernel on the shapes of the ViT-L window (CUDA events, L2
-flushed between launches, median of `iters`).  VDA_GEMM_STAGED=0|1 forces the epilogue variant (debug hook)."""
+flushed between launches, median of `iters`)."""
 import os
 import sys
 import torch

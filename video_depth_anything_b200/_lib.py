@@ -6,7 +6,7 @@ import ctypes as C
 import os
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-# VDA_LIB: debug hook (tools/attn_variants.sh) -- another build of the same library, e.g. with different -D switches
+# VDA_LIB: debug hook (tools/build_variant.sh) -- another build of the same library, e.g. with different nvcc flags
 LIB_PATH = os.environ.get("VDA_LIB") or os.path.join(HERE, "libvda.so")
 
 VDA_BF16, VDA_FP16 = 0, 1

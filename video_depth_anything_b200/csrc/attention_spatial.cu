@@ -20,7 +20,7 @@
 //           divided between the streams (stream 0: tiles 0..ja-1, stream 1: ja..n_kv-1, loaded interleaved); the two
 //           partial results (m, l, O) are merged through shared memory by warpgroup 0 (standard split-KV flash merge).
 //           Round 1 ran these items on one stream with the other idle (8 % of the kernel's time)
-//   SINGLE  the same odd tile on stream 0 only (when there is just one key tile, or -DVDA_SA_NO_SPLIT)
+//   SINGLE  the same odd tile on stream 0 only (when there is just one key tile)
 // Every `empty` barrier (K / V slots, Q buffers) expects TWO arrivals per use: one tcgen05.commit from each stream that
 // consumes the use; for a use only one stream consumes, the PRODUCER arrives in place of the other stream right after
 // issuing the load.  A stream therefore never waits on, or acknowledges, a slot it does not read -- it only counts
@@ -35,10 +35,6 @@
 // The kernel is bound by the instruction issue of the softmax warps (MUFU.EX2: 16/clk/SM), see DESIGN.md.
 #include "../../include/vda.h"
 #include "common.cuh"
-
-#ifndef VDA_SA_DEFAULT_KERNEL
-#define VDA_SA_DEFAULT_KERNEL 2
-#endif
 
 namespace vda {
 
@@ -55,6 +51,7 @@ constexpr uint32_t SMEM_BYTES = (4 + KS + VS) * TILE_BYTES + XCH_FLOATS * 4 + 10
 // TMEM columns
 constexpr uint32_t COL_S = 0, COL_O = 256, COL_P = 384;
 constexpr float RESCALE_LOG2 = 8.0f;
+constexpr int POLY_MASK = 3;       // pair p of a score row takes exp2_poly2 when (p & POLY_MASK) == POLY_MASK: 25 %
 enum { PAIR = 0, SPLIT = 1, SINGLE = 2 };
 enum { BAR_XCH_FULL = 1, BAR_XCH_EMPTY = 2 };   // named barriers (0 is __syncthreads)
 }  // namespace sa
@@ -110,21 +107,10 @@ __device__ __forceinline__ int sa_kv_cols(const SaParams& p, int j) {   // colum
   return valid >= sa::BN ? sa::BN : ((valid + 31) & ~31);
 }
 
-#ifdef VDA_SA_TIMING
-// debug build only: per-phase cycle sums of the softmax warps of CTA 0 (tools/bench_attention.py timing)
-__device__ unsigned long long g_sa_timing[3][8];
-#define SA_T(i) do { const long long _t = clock64(); tacc[i] += _t - tprev; tprev = _t; } while (0)
-#else
-#define SA_T(i) do { } while (0)
-#endif
-
 // exp2 on the FMA / ALU pipes for a pair of values (Cody-Waite: x = j + f, j = round(x), f in [-0.5, 0.5];
 // 2^f by a degree-3 minimax polynomial, max rel. error 7.7e-5 -- below the 16-bit rounding of P; 2^j by adding j
 // to the exponent field).  A quarter of the exponentials of a score tile take this path so that the MUFU (16 ex2/clk/SM)
 // is no longer the only unit that can produce them.
-#ifndef VDA_SA_POLY_MASK
-#define VDA_SA_POLY_MASK 3     // pair p of a row uses the polynomial when (p & MASK) == MASK; 1: 50%, 3: 25%, 7: 12.5%, 255: none
-#endif
 __device__ __forceinline__ float2 exp2_poly2(float2 x) {
   x.x = fmaxf(x.x, -126.f);
   x.y = fmaxf(x.y, -126.f);
@@ -317,9 +303,6 @@ spatial_attention_tc_kernel(const __grid_constant__ CUtensorMap tmQKV, const SaP
     uint32_t cnt = 0;                                 // running key-tile counter of this stream
     T* outp = reinterpret_cast<T*>(p.out);
     float* xch = reinterpret_cast<float*>(smem_gen + offX);
-#ifdef VDA_SA_TIMING
-    long long tacc[8] = {0, 0, 0, 0, 0, 0, 0, 0}, tprev = clock64();
-#endif
 
     for (int i = 0; i < n_my; ++i) {
       const SaItem it = sa_decode(p, blockIdx.x + i * gridDim.x);
@@ -334,10 +317,8 @@ spatial_attention_tc_kernel(const __grid_constant__ CUtensorMap tmQKV, const SaP
         const int valid = p.N - j * BN;
         uint32_t s[BN];
         float mx0 = -INFINITY, mx1 = -INFINITY, mx2 = -INFINITY, mx3 = -INFINITY;
-        SA_T(7);
         mbar_wait(&s_ready[t], cnt & 1u);
         tc_fence_after();
-        SA_T(0);
         if (valid >= BN) {
           // full key tile: the row maximum of chunk c is computed while chunk c+1 is still in flight from TMEM
           tmem_ld32(tS, s);
@@ -380,7 +361,6 @@ spatial_attention_tc_kernel(const __grid_constant__ CUtensorMap tmQKV, const SaP
             }
           }
         }
-        SA_T(1);
         const float mx = fmaxf(fmaxf(mx0, mx1), fmaxf(mx2, mx3));
         // O += P(j-1) V(j-1) was issued by this stream's own issuer as soon as P(j-1) was complete; P and O are ours
         // again once it has retired.  Normally that wait is taken as late as possible (in front of the first P store,
@@ -414,7 +394,6 @@ spatial_attention_tc_kernel(const __grid_constant__ CUtensorMap tmQKV, const SaP
             tmem_st_wait();
           }
         }
-        SA_T(2);
         // ---- exp phase: P = exp2(s*sc - m*sc), row sum, pack to 16 bit, store to TMEM ----
         const float nmb = -m_run * sc;
         const float2 nmb2 = make_float2(nmb, nmb);
@@ -425,9 +404,9 @@ spatial_attention_tc_kernel(const __grid_constant__ CUtensorMap tmQKV, const SaP
             float2 x0 = __ffma2_rn(make_float2(__uint_as_float(s[c + k]), __uint_as_float(s[c + k + 1])), sc2, nmb2);
             float2 x1 =
                 __ffma2_rn(make_float2(__uint_as_float(s[c + k + 2]), __uint_as_float(s[c + k + 3])), sc2, nmb2);
-            if ((((c + k) >> 1) & VDA_SA_POLY_MASK) == VDA_SA_POLY_MASK) x0 = exp2_poly2(x0);
+            if ((((c + k) >> 1) & POLY_MASK) == POLY_MASK) x0 = exp2_poly2(x0);
             else { x0.x = exp2f(x0.x); x0.y = exp2f(x0.y); }
-            if (((((c + k) >> 1) + 1) & VDA_SA_POLY_MASK) == VDA_SA_POLY_MASK) x1 = exp2_poly2(x1);
+            if (((((c + k) >> 1) + 1) & POLY_MASK) == POLY_MASK) x1 = exp2_poly2(x1);
             else { x1.x = exp2f(x1.x); x1.y = exp2f(x1.y); }
             la = __fadd2_rn(la, x0);
             lb = __fadd2_rn(lb, x1);
@@ -444,7 +423,6 @@ spatial_attention_tc_kernel(const __grid_constant__ CUtensorMap tmQKV, const SaP
           }
           tmem_st16(tP, pk);
         }
-        SA_T(4);
         if (cols == BN) {   // straight-line code for full key tiles: the scheduler hides the FMAs behind the MUFU
 #pragma unroll
           for (int c = 32; c < BN; c += 32) {
@@ -462,12 +440,10 @@ spatial_attention_tc_kernel(const __grid_constant__ CUtensorMap tmQKV, const SaP
             }
           }
         }
-        SA_T(3);
         l_run += (la.x + la.y) + (lb.x + lb.y);
         tmem_st_wait();
         tc_fence_before();
         mbar_arrive(&p_ready[t]);
-        SA_T(5);
       }
       // ---- epilogue: O / l -> 16 bit -> global ----
       mbar_wait(&o_done[t], (cnt - 1u) & 1u);
@@ -533,12 +509,7 @@ spatial_attention_tc_kernel(const __grid_constant__ CUtensorMap tmQKV, const SaP
         tc_fence_before();   // the O reads above are ordered before this thread's next p_ready arrive
         if (it.kind == SPLIT && i + 1 < n_my) named_bar_arrive(BAR_XCH_EMPTY, 256);   // (split items are the tail of the list)
       }
-      SA_T(6);
     }
-#ifdef VDA_SA_TIMING
-    if (blockIdx.x == 0 && quad == 0 && lane == 0)
-      for (int k = 0; k < 8; ++k) g_sa_timing[t][k] = static_cast<unsigned long long>(tacc[k]);
-#endif
   }
 
   tc_fence_before();
@@ -551,18 +522,7 @@ spatial_attention_tc_kernel(const __grid_constant__ CUtensorMap tmQKV, const SaP
 
 }  // namespace vda
 
-namespace vda {
-int sa4_launch(const void* qkv, void* out, int frames, int N, int heads, int dtype, cudaStream_t st);   // attention_spatial4.cu
-}
-
 using namespace vda;
-
-#ifdef VDA_SA_TIMING
-extern "C" int vda_debug_sa_timing(unsigned long long* host_out) {
-  VDA_CUDA(cudaMemcpyFromSymbol(host_out, g_sa_timing, sizeof(unsigned long long) * 24));
-  return 0;
-}
-#endif
 
 extern "C" int vda_attention_spatial(const void* qkv, void* out, int frames, int N, int heads, int dtype,
                                      void* stream) {
@@ -570,11 +530,6 @@ extern "C" int vda_attention_spatial(const void* qkv, void* out, int frames, int
   VDA_CHECK(dtype == VDA_BF16 || dtype == VDA_FP16, "bad dtype %d", dtype);
   VDA_CHECK((reinterpret_cast<uintptr_t>(qkv) & 15) == 0 && (reinterpret_cast<uintptr_t>(out) & 15) == 0,
             "qkv/out must be 16-byte aligned");
-  {
-    // VDA_SA_KERNEL=4: four streams x 64-key tiles (attention_spatial4.cu); 2: two streams x 128-key tiles (this file)
-    static const int which = []() { const char* e = getenv("VDA_SA_KERNEL"); return e ? atoi(e) : VDA_SA_DEFAULT_KERNEL; }();
-    if (which == 4) return sa4_launch(qkv, out, frames, N, heads, dtype, static_cast<cudaStream_t>(stream));
-  }
   // qkv is [frames, N, 3, heads, 64]: a 4-D tensor (d, which*heads + head, token, frame); token rows beyond N are
   // zero-filled by TMA instead of running into the next frame
   CUtensorMap tm;
@@ -592,11 +547,7 @@ extern "C" int vda_attention_spatial(const void* qkv, void* out, int frames, int
   p.n_items = frames * heads * p.n_pairs + ((p.n_qt & 1) ? frames * heads : 0);
   p.n_kv = (N + sa::BN - 1) / sa::BN;
   p.ja = (p.n_kv + 1) / 2;
-#ifdef VDA_SA_NO_SPLIT
-  p.split = 0;
-#else
   p.split = p.n_kv >= 2 ? 1 : 0;
-#endif
   p.out = out;
   const int grid = p.n_items < sm_count() ? p.n_items : sm_count();
   cudaStream_t st = static_cast<cudaStream_t>(stream);

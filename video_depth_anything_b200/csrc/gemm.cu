@@ -1029,11 +1029,8 @@ static int dispatch(const vda_gemm_params* p, const Maps& tm, const GemmDev& d, 
         case 6: return launch<T, VDA_EPI_LINEAR, false, true, 6>(tm, d, smem, st);
         default: break;
       }
-      if (d.staged)
-        return conv ? launch<T, VDA_EPI_LINEAR, true, true>(tm, d, smem, st)
-                    : launch<T, VDA_EPI_LINEAR, false, true>(tm, d, smem, st);
-      return conv ? launch<T, VDA_EPI_LINEAR, true, false>(tm, d, smem, st)
-                  : launch<T, VDA_EPI_LINEAR, false, false>(tm, d, smem, st);
+      return conv ? launch<T, VDA_EPI_LINEAR, true, true>(tm, d, smem, st)
+                  : launch<T, VDA_EPI_LINEAR, false, true>(tm, d, smem, st);
     case VDA_EPI_GEGLU:
       VDA_CHECK(!conv, "GEGLU epilogue is only defined for plain GEMMs");
       return launch<T, VDA_EPI_GEGLU, false, true>(tm, d, smem, st);
@@ -1050,7 +1047,7 @@ static int dispatch(const vda_gemm_params* p, const Maps& tm, const GemmDev& d, 
 
 // Which compile-time specialised epilogue serves this problem (0 = generic).  block_n is known.
 static int pick_spec(const vda_gemm_params* p, const GemmDev& d) {
-  if (p->epilogue != VDA_EPI_LINEAR || !d.staged || p->a_mode == VDA_A_CONV3) return 0;
+  if (p->epilogue != VDA_EPI_LINEAR || p->a_mode == VDA_A_CONV3) return 0;
   const bool plain16 = p->bias && !p->res1 && !p->res2 && !p->out_f32 && !p->out_relu && !p->gamma && p->row_group == 0;
   if (plain16 && p->row_stats_in) return p->act == VDA_ACT_GELU ? 6 : (p->act == VDA_ACT_NONE ? 5 : 0);
   if (plain16 && p->act == VDA_ACT_NONE) return 1;
@@ -1058,10 +1055,9 @@ static int pick_spec(const vda_gemm_params* p, const GemmDev& d) {
   if (p->bias && p->gamma && p->res1 && p->res1_f32 && !p->res2 && p->out_f32 && !p->out_relu && p->act == VDA_ACT_NONE &&
       p->row_group == 0) {
     // fp32 residual stream: all tile traffic by TMA when the residual is updated in place and the tile geometry allows
-    // 32-column boxes (SPEC 4); VDA_GEMM_TMA_EPI=0 keeps the register-staged epilogue (SPEC 3) for A/B runs
-    static const char* e = getenv("VDA_GEMM_TMA_EPI");
-    const bool tma_ok = !(e && e[0] == '0') && p->res1 == p->out && p->ldr1 == p->ldo && d.block_n % 64 == 0 &&
-                        p->N % d.block_n == 0 && (p->ldo % 4) == 0;
+    // 32-column boxes (SPEC 4); otherwise the register-staged epilogue (SPEC 3)
+    const bool tma_ok = p->res1 == p->out && p->ldr1 == p->ldo && d.block_n % 64 == 0 && p->N % d.block_n == 0 &&
+                        (p->ldo % 4) == 0;
     if (tma_ok) return 4;
     return (p->out16 || p->row_stats_out) ? -1 : 3;
   }
@@ -1086,10 +1082,7 @@ extern "C" int vda_gemm(const vda_gemm_params* p, void* stream) {
   GemmDev d = {};
   d.M = p->M; d.N = p->N; d.K = p->K;
   d.num_k_blocks = (p->K + BLOCK_K - 1) / BLOCK_K;
-  {
-    static const char* pf = getenv("VDA_GEMM_PREFETCH_KB");     // debug hook (tools/bench_gemm.py)
-    d.prefetch_max_kb = pf ? atoi(pf) : 32;
-  }
+  d.prefetch_max_kb = 32;
   Maps tm;
   CUtensorMap& tmA = tm.a;
   CUtensorMap& tmB = tm.b;
@@ -1154,10 +1147,6 @@ extern "C" int vda_gemm(const vda_gemm_params* p, void* stream) {
   // (not for K <= 256: those GEMMs are bound by their output stream, measured slower in pair mode)
   d.pair = (p->epilogue != VDA_EPI_TAIL && d.block_n % 32 == 0 && d.tiles_m >= 2 && d.num_k_blocks >= 8 &&
             ((d.tiles_m + 1) / 2) * d.tiles_n >= sm_count() / 2) ? 1 : 0;
-  {
-    static const char* force = getenv("VDA_GEMM_PAIR");    // debug hook (tools/bench_gemm.py)
-    if (force && force[0] == '0') d.pair = 0;
-  }
   if (d.pair) d.num_tiles = ((d.tiles_m + 1) / 2) * d.tiles_n;
   const uint32_t b_rows = d.pair ? d.block_n / 2 : d.block_n;   // B rows loaded (and stored) per CTA and stage
   {
@@ -1173,12 +1162,8 @@ extern "C" int vda_gemm(const vda_gemm_params* p, void* stream) {
   // 227 KB per CTA: 1 KB alignment slack + static barriers, the epilogue staging tiles, the rest for the operand ring
   // LINEAR epilogue variant (measured with tools/bench_gemm.py): the shared-memory transpose (coalesced row segments
   // for every residual load and store) wins for all LINEAR epilogues, 16-bit residuals included (RCU conv @148^2:
-  // 703 -> 627 us); the row-per-thread path remains for CONVT and as a debug variant.
+  // 703 -> 627 us); the row-per-thread path remains for CONVT.
   d.staged = (p->epilogue == VDA_EPI_GEGLU || p->epilogue == VDA_EPI_LINEAR) ? 1 : 0;
-  if (p->epilogue == VDA_EPI_LINEAR) {   // debug hook (tools/bench_gemm.py): force the epilogue variant
-    static const char* force = getenv("VDA_GEMM_STAGED");
-    if (force && (force[0] == '0' || force[0] == '1')) d.staged = force[0] - '0';
-  }
   const int spec = pick_spec(p, d);
   VDA_CHECK(spec >= 0, "out16 / row_stats_out need the in-place fp32 residual epilogue with N %% block_n == 0 and "
                        "block_n %% 64 == 0 (N=%d block_n=%d)", p->N, d.block_n);

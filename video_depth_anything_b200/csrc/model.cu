@@ -458,12 +458,6 @@ extern "C" int vda_create(const char* encoder, int features, const int32_t* out_
   m->num_frames = num_frames;
   m->dtype = dtype;
   m->hdtype = VDA_FP16;          // the DPT head runs on fp16 operands (engine.py: Engine.hdtype)
-  {
-    const char* e = getenv("VDA_HEAD_DTYPE");
-    if (e && strcmp(e, "fp16") != 0) m->hdtype = dtype;
-    const char* f = getenv("VDA_LN_FOLD");
-    m->ln_fold = !(f && f[0] == '0');
-  }
   m->device = device;
   m->c_l1 = pad_to(m->oc[0], 64);
   m->c_l2 = pad_to(m->oc[1], 64);

@@ -292,9 +292,9 @@ def _infer_two_phase(model, frames, target_fps, input_size, device, group):
             share = len(os.sched_getaffinity(0))
         except AttributeError:
             share = (os.cpu_count() or 8) // world
-        direct = os.environ.get("VDA_DIRECT_D2H", "1") != "0"      # GPU writes into the page-locked result rows
+        # direct: the GPU writes into the page-locked result rows
         drain = HostDrain(host, dev, touch=slice(lo, hi), copy_threads=max(2, min(6, share - 1)), touch_threads=1,
-                          direct=direct)
+                          direct=True)
         raws = model.infer_video_depth(frames, target_fps, input_size=input_size, device=dev,
                                        window_ids=list(parts[rank]), raw_only=True)          # [k_r,32,h0,w0]
         stamp("windows computed")

@@ -451,7 +451,7 @@ class FrameUploader:
     waits for the kernels that read it (`reads_done`).  `ring=False` (windows not in increasing order): everything stays."""
 
     CHUNK = 64
-    RING_CHUNKS = 4 if os.environ.get("VDA_VIDEO_RINGS", "1") != "0" else 1 << 20    # VDA_VIDEO_RINGS=0: keep everything
+    RING_CHUNKS = 4
 
     def __init__(self, frames: np.ndarray, needed: List[int], device, ring: bool = True):
         self.frames, self.needed, self.device = frames, needed, device
@@ -745,7 +745,7 @@ class WindowAligner:
     segment is only overwritten after the D2H copies that read it have completed (events of HostDrain.send)."""
 
     SEG = INFER_LEN - OVERLAP          # 22 new frames per window
-    RING_SEGS = 4 if os.environ.get("VDA_VIDEO_RINGS", "1") != "0" else 1 << 20
+    RING_SEGS = 4
 
     def __init__(self, n_frames: int, h0: int, w0: int, device, mode: str = "affine"):
         self.n, self.h0, self.w0, self.device, self.mode = n_frames, h0, w0, device, mode
