@@ -1,6 +1,7 @@
-"""N>1 host logic on CPU (gloo, world_size 2): window partition + gather of per-window depths to rank 0 reproduces
+"""N>1 host logic on CPU (gloo, world sizes 1-4): window partition + gather of per-window depths to rank 0 reproduces
 the single-process window stack bit-for-bit, and the sequential alignment (oracle restatement of
-video_depth.py:216-252) gives the same video from the gathered stack."""
+video_depth.py:216-252) gives the same video from the gathered stack; the two-phase exchange + finalisation gives it
+too, also when some ranks hold no window."""
 import os
 import socket
 import sys
@@ -64,12 +65,13 @@ def test_windows_depend_on_input_frames_only():
     assert wins[2][:3] == [0, 34, 46] and wins[4][-1] == 99
 
 
-@pytest.mark.parametrize("n_frames", [23, 70, 131])
-def test_gather_world2_matches_single_process(tmp_path, n_frames):
+@pytest.mark.parametrize("world,n_frames", [(2, 23), (2, 70), (2, 131), (3, 23)])
+def test_gather_matches_single_process(tmp_path, world, n_frames):
+    """The exchange of ranks on several hosts; (3, 23) has a rank with no window."""
     from oracle import vda_oracle as O
     port = _free_port()
     out = str(tmp_path / "gathered.npy")
-    mp.spawn(_worker, args=(2, port, n_frames, out), nprocs=2, join=True)
+    mp.spawn(_worker, args=(world, port, n_frames, out), nprocs=world, join=True)
     got = np.load(out)
     k = num_windows(n_frames)
     ref = torch.stack([fake_raw(i) for i in range(k)]).numpy()
@@ -78,41 +80,6 @@ def test_gather_world2_matches_single_process(tmp_path, n_frames):
     a = O.align_windows([w[i].copy() for w in got for i in range(INFER_LEN)], n_frames, "affine")
     b = O.align_windows([w[i].copy() for w in ref for i in range(INFER_LEN)], n_frames, "affine")
     assert np.array_equal(a, b) and a.shape[0] == n_frames
-
-
-def _stream_worker(rank, world, port, n_frames, out_path):
-    from video_depth_anything_b200.parallel import stream_window_depths
-    os.environ.update(MASTER_ADDR="127.0.0.1", MASTER_PORT=str(port))
-    dist.init_process_group("gloo", rank=rank, world_size=world)
-    try:
-        parts = partition_windows(num_windows(n_frames), world)
-        counts = [len(p) for p in parts]
-        mine = [fake_raw(k) for k in parts[rank]]
-        local = torch.stack(mine) if mine else torch.empty(0, INFER_LEN, 6, 5)
-        got = [local] if rank == 0 else []
-        order = []
-        for r, stack in stream_window_depths(local if rank else None, counts, (6, 5), torch.float32, "cpu", dst=0):
-            order.append(r)
-            got.append(stack.clone())
-        if rank == 0:
-            assert order == [r for r in range(1, world) if counts[r] > 0]
-            np.save(out_path, torch.cat(got).numpy())
-        else:
-            assert got == []
-    finally:
-        dist.destroy_process_group()
-
-
-@pytest.mark.parametrize("world,n_frames", [(2, 70), (3, 131), (3, 23)])
-def test_stream_collect_matches_single_process(tmp_path, world, n_frames):
-    """The point-to-point streaming collection (rank 0 keeps its own block, the others send) yields every other
-    rank's window stack in window order; (3, 23) has ranks with no windows at all."""
-    port = _free_port()
-    out = str(tmp_path / "streamed.npy")
-    mp.spawn(_stream_worker, args=(world, port, n_frames, out), nprocs=world, join=True)
-    got = np.load(out)
-    ref = torch.stack([fake_raw(i) for i in range(num_windows(n_frames))]).numpy()
-    assert got.shape == ref.shape and np.array_equal(got, ref)
 
 
 def test_frame_spans_tile_the_video():
@@ -183,14 +150,13 @@ def _two_phase_worker(rank, world, port, n_frames, mode, out_dir):
 
 
 @pytest.mark.parametrize("world,n_frames,mode", [(1, 70, "affine"), (2, 70, "affine"), (2, 131, "identity"),
-                                                 (3, 200, "affine"), (3, 100, "affine")])
+                                                 (3, 200, "affine"), (3, 100, "affine"), (3, 23, "affine"),
+                                                 (4, 50, "identity")])
 def test_two_phase_finalise_matches_sequential_alignment(tmp_path, world, n_frames, mode):
     """The scalable driver's exchange (halo point-to-point, anchor all-gather) + per-rank finalisation, run with gloo on
     CPU tensors, emits every video frame exactly once and equals the reference's sequential alignment of the full
-    window stack (oracle restatement of video_depth.py:216-252)."""
+    window stack (oracle restatement of video_depth.py:216-252).  (3, 23) and (4, 50) have ranks with no window."""
     from oracle import vda_oracle as O
-    if min(len(p) for p in partition_windows(num_windows(n_frames), world)) == 0:
-        pytest.skip("the two-phase form needs a window on every rank (the driver falls back otherwise)")
     port = _free_port()
     if world == 1:
         _two_phase_worker(0, 1, port, n_frames, mode, str(tmp_path))

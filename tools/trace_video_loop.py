@@ -1,6 +1,7 @@
 #!/usr/bin/env python
 """Host-side time per phase of the long-video loop (debug): monkeypatches the phases of infer_video_depth with wall-clock
-accumulators for a block of windows computed with raw_only (the non-aligning ranks' path) or with alignment."""
+accumulators for a block of windows computed with raw_only (the sharded driver's per-rank path) or aligned by the
+driver's own WindowAligner."""
 import os
 import sys
 import time
@@ -41,11 +42,7 @@ for ids, raw in ((range(0, 47), True), (range(47, 94), True), (range(47, 94), Fa
     acc.clear()
     torch.cuda.synchronize()
     t0 = time.perf_counter()
-    if raw:
-        out = m.infer_video_depth(frames, 24, window_ids=list(ids), raw_only=True)
-    else:
-        al = video_depth.WindowAligner(2048, 518, 518, torch.device("cuda"), "affine")
-        m.infer_video_depth(frames, 24, window_ids=list(ids), aligner=al)
+    out = m.infer_video_depth(frames, 24, window_ids=list(ids), raw_only=raw)
     t1 = time.perf_counter()
     torch.cuda.synchronize()
     t2 = time.perf_counter()

@@ -4,11 +4,14 @@ The reference has no multi-GPU inference path at all (SURVEY.md §2.1).  Its lon
 (video_depth_anything/video_depth.py:166-254) computes K = ceil(N/22) overlapping 32-frame windows whose model
 inputs depend on input frames only (closed form in windows.window_source_indices), followed by a cheap
 *sequential* scale/shift alignment (:216-252).  So the windows are sharded in contiguous blocks over the ranks with
-no data-path collective; the only exchange is a gather of the raw per-window depths to one rank (NCCL send/recv
-over NVLink, 34 MB per 32x518x518 fp32 window), which then runs the alignment recurrence on its GPU.
+no data-path collective; what remains is the exchange that feeds the alignment:
+  * ranks on one host: the two-phase form (`_infer_two_phase`): halo + anchor all-gather, every rank runs the
+    alignment chain itself and downloads its own frames into a shared-memory result returned on rank `dst`;
+  * ranks on several hosts: a gather of the raw per-window depths to rank `dst` (NCCL send/recv, 34 MB per
+    32x518x518 fp32 window), which then runs the alignment recurrence on its GPU.
 
-Host-side pieces (`partition_windows`, `gather_window_depths`) work on CPU tensors with the gloo backend too;
-that is how tests/test_parallel_cpu.py covers the N>1 logic without GPUs.
+Host-side pieces (`partition_windows`, `gather_window_depths`, `two_phase_finalise`) work on CPU tensors with the
+gloo backend too; that is how tests/test_parallel_cpu.py covers the N>1 logic without GPUs.
 """
 from __future__ import annotations
 
@@ -67,31 +70,6 @@ def gather_window_depths(local: torch.Tensor, counts: Sequence[int], dst: int = 
     if rank != dst:
         return None
     return torch.cat([bufs[r][:counts[r]] for r in range(world)], dim=0)
-
-
-def stream_window_depths(local: Optional[torch.Tensor], counts: Sequence[int], shape_hw, dtype, device, dst: int = 0,
-                         group=None):
-    """Point-to-point variant of the gather for the streaming driver: every rank other than `dst` sends its raw
-    window stack `[counts[rank], 32, H, W]` to `dst` (NCCL send over NVLink); on `dst` this is a generator that
-    posts all receives up front and yields `(rank, stack)` in rank order (= window order), so the caller aligns
-    rank r's windows while rank r+1's are still in flight.  `dst`'s own windows are not part of the stream."""
-    rank, world = _world(group)
-    if world == 1:
-        return
-    if rank != dst:
-        if counts[rank] > 0:
-            assert local is not None and local.shape[0] == counts[rank]
-            dist.send(local.contiguous(), dst=dst, group=group)
-        return
-    h, w = shape_hw
-    bufs, works = {}, {}
-    for r in range(world):
-        if r != dst and counts[r] > 0:
-            bufs[r] = torch.empty(counts[r], INFER_LEN, h, w, dtype=dtype, device=device)
-            works[r] = dist.irecv(bufs[r], src=r, group=group)
-    for r in sorted(bufs):
-        works[r].wait()
-        yield r, bufs[r]
 
 
 def frame_span(k0: int, k1: int, n_windows: int, n_frames: int):
@@ -242,15 +220,16 @@ def two_phase_finalise(raws: torch.Tensor, counts: Sequence[int], K: int, n: int
 
 
 @torch.no_grad()
-def _infer_two_phase(model, frames, target_fps, input_size, device, group):
-    """Scalable form for one node (SURVEY.md §8e option 2), the default.  Every rank computes its block of windows
+def _infer_two_phase(model, frames, target_fps, input_size, device, dst, group):
+    """Scalable form for ranks on one host (SURVEY.md §8e option 2).  Every rank computes its block of windows
     with no data-path collective; then
       1. the last 8 raw slots of every block travel to the next rank (cross-fade halo; NCCL batch_isend_irecv),
       2. the three anchor frames of every window (slots 0, 1, 12) are all-gathered (NCCL over NVLink, 3.2 MB / window),
       3. every rank walks the sequential (scale, shift) recurrence itself in ONE cooperative kernel
          (ops.align_chain: bit-identical to WindowAligner.push's per-window kernels),
       4. each rank clamps / cross-fades ITS frames in place and downloads them into a POSIX shared-memory array owned
-         by rank 0 -- PCIe, host copies and page faults are spread over all ranks instead of funnelled through one.
+         by rank `dst` -- PCIe, host copies and page faults are spread over all ranks instead of funnelled through one.
+    A rank without windows (more ranks than windows) takes part in every collective and downloads nothing.
     The result is bit-identical to the single-GPU `infer_video_depth`."""
     from multiprocessing import resource_tracker, shared_memory
     from .video_depth import HostDrain
@@ -263,16 +242,16 @@ def _infer_two_phase(model, frames, target_fps, input_size, device, group):
     k0, k1 = (parts[rank][0], parts[rank][-1] + 1) if counts[rank] else (0, 0)
     lo, hi = frame_span(k0, k1, K, n)
     _pin_cores(rank, world)
-    # shared result array: created by rank 0, attached by the others, first-touched per slice in the background
+    # shared result array: created by rank dst, attached by the others, first-touched per slice in the background
     nbytes = n * h0 * w0 * 4
     box = [None]
-    if rank == 0:
+    if rank == dst:
         shm = shared_memory.SharedMemory(create=True, size=nbytes)
         box[0] = shm.name
-    dist.broadcast_object_list(box, src=0, group=group)
-    if rank != 0:
+    dist.broadcast_object_list(box, src=dst, group=group)
+    if rank != dst:
         shm = shared_memory.SharedMemory(name=box[0])
-        resource_tracker.unregister(shm._name, "shared_memory")     # rank 0 owns the segment's lifetime
+        resource_tracker.unregister(shm._name, "shared_memory")     # rank dst owns the segment's lifetime
     host = np.ndarray((n, h0, w0), dtype=np.float32, buffer=shm.buf)
     trace = os.environ.get("VDA_TRACE_VIDEO") == "1"
     stamps = [("start", time.perf_counter())]
@@ -292,9 +271,10 @@ def _infer_two_phase(model, frames, target_fps, input_size, device, group):
             share = len(os.sched_getaffinity(0))
         except AttributeError:
             share = (os.cpu_count() or 8) // world
-        # direct: the GPU writes into the page-locked result rows
+        # direct: the GPU writes into the page-locked result rows.  A rank without rows (lo == hi) has nothing to drain:
+        # the staged path page-locks nothing and allocates its pinned buffers only on a first send, which never comes
         drain = HostDrain(host, dev, touch=slice(lo, hi), copy_threads=max(2, min(6, share - 1)), touch_threads=1,
-                          direct=True)
+                          direct=hi > lo)
         raws = model.infer_video_depth(frames, target_fps, input_size=input_size, device=dev,
                                        window_ids=list(parts[rank]), raw_only=True)          # [k_r,32,h0,w0]
         stamp("windows computed")
@@ -310,7 +290,7 @@ def _infer_two_phase(model, frames, target_fps, input_size, device, group):
     stamp("barrier")
     if trace:
         print(f"video trace rank {rank}: " + ", ".join(f"{a} +{(t - stamps[0][1]) * 1e3:.0f} ms" for a, t in stamps[1:]), flush=True)
-    if rank != 0:
+    if rank != dst:
         del host
         drain.unregister_later(close_after=shm)   # page lock released in the background, THEN the attachment is closed
         return None, target_fps
@@ -328,63 +308,20 @@ def infer_video_depth_sharded(model, frames: np.ndarray, target_fps, input_size:
                               dst: int = 0, group=None):
     """Drop-in for `model.infer_video_depth(frames, target_fps, input_size, device)` under torchrun: every rank
     passes the same `frames`; rank `dst` returns `(depths float32 [N,H0,W0], target_fps)`, the others `(None,
-    target_fps)`.  With one process (no process group) it is exactly `model.infer_video_depth`."""
+    target_fps)`.  With one process (no process group) it is exactly `model.infer_video_depth`.  Ranks on one host
+    use the two-phase form (_infer_two_phase); ranks on several hosts, which cannot share one result array, send their
+    raw window stacks to `dst` in one gather, and `dst` aligns them."""
     from .video_depth import WindowAligner
     rank, world = _world(group)
     if device is None:
         device = torch.device("cuda", torch.cuda.current_device())
     if world == 1:
         return model.infer_video_depth(frames, target_fps, input_size=input_size, device=device)
+    if _same_host(group):
+        return _infer_two_phase(model, frames, target_fps, input_size, device, dst, group)
     n, h0, w0 = frames.shape[:3]
     parts = partition_windows(num_windows(n), world)
     counts = [len(p) for p in parts]
-    # Default on one host: the two-phase form (every rank downloads its own frames; the (scale, shift) chain is one
-    # cooperative kernel).  Round 1 defaulted to the streaming form below: rank 0 pulled the other ranks' raw stacks
-    # (unbatched point-to-point) and funnelled all N frames through its one PCIe link -- 70 ms of a 650 ms call at 8
-    # GPUs.  VDA_SHARD_MODE=stream selects it again; it is also the form for ranks spread over several hosts.
-    mode = os.environ.get("VDA_SHARD_MODE", "two_phase")
-    if dst == 0 and min(counts) > 0 and mode == "two_phase" and _same_host(group):
-        return _infer_two_phase(model, frames, target_fps, input_size, device, group)
-    if dst == 0:
-        # streaming form: rank 0 owns the first block of windows, so it aligns them (and streams the finished frames
-        # to the host) while it computes; the other ranks' stacks arrive point-to-point and are aligned in rank order
-        if rank != 0:
-            t0 = time.perf_counter()
-            raw = model.infer_video_depth(frames, target_fps, input_size=input_size, device=device,
-                                          window_ids=list(parts[rank]), raw_only=True)
-            if os.environ.get("VDA_TRACE_VIDEO") == "1":
-                t1 = time.perf_counter()
-                torch.cuda.synchronize(raw.device)
-                print(f"video trace rank {rank}: enqueued +{(t1 - t0) * 1e3:.0f} ms, computed "
-                      f"+{(time.perf_counter() - t0) * 1e3:.0f} ms", flush=True)
-            for _ in stream_window_depths(raw, counts, (h0, w0), torch.float32, raw.device, dst=0, group=group):
-                pass
-            return None, target_fps
-        dev = torch.device(device)
-        trace = os.environ.get("VDA_TRACE_VIDEO") == "1"       # debug: synchronising wall-clock stamps of the phases
-        stamps = [("start", time.perf_counter())]
-
-        def stamp(name):
-            if trace:
-                torch.cuda.synchronize(dev)
-                stamps.append((name, time.perf_counter()))
-
-        with torch.cuda.device(dev):
-            aligner = WindowAligner(n, h0, w0, dev, "identity" if model.metric else "affine")
-            stamp("aligner allocated")
-            model.infer_video_depth(frames, target_fps, input_size=input_size, device=dev, window_ids=list(parts[0]),
-                                    aligner=aligner)
-            stamp("own windows computed + aligned")
-            for r, stack in stream_window_depths(None, counts, (h0, w0), torch.float32, dev, dst=0, group=group):
-                stamp(f"received rank {r}")
-                for k in range(stack.shape[0]):
-                    aligner.push(stack[k])
-                stamp(f"aligned rank {r}")
-            out = aligner.result()
-            stamp("drained to host")
-            if trace:
-                print("video trace: " + ", ".join(f"{a} +{(t - stamps[0][1]) * 1e3:.0f} ms" for a, t in stamps[1:]), flush=True)
-            return out, target_fps
     raw = model.infer_video_depth(frames, target_fps, input_size=input_size, device=device,
                                   window_ids=list(parts[rank]), raw_only=True)         # [k_r,32,h0,w0] on device
     allraw = gather_window_depths(raw, counts, dst=dst, group=group)
@@ -397,5 +334,5 @@ def infer_video_depth_sharded(model, frames: np.ndarray, target_fps, input_size:
         return aligner.result(), target_fps
 
 
-__all__ = ["two_phase_finalise", "partition_windows", "gather_window_depths", "stream_window_depths", "frame_span", "rank_core_slice",
+__all__ = ["two_phase_finalise", "partition_windows", "gather_window_depths", "frame_span", "rank_core_slice",
            "infer_video_depth_sharded", "INFER_LEN"]

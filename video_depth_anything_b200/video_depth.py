@@ -125,8 +125,7 @@ class VideoDepthAnything(nn.Module):
     # ---- long-video driver -------------------------------------------------------------------
     @torch.no_grad()
     def infer_video_depth(self, frames: np.ndarray, target_fps, input_size=518, device="cuda", fp32=False,
-                          window_ids: Optional[Sequence[int]] = None, raw_only=False, reuse_features: bool = True,
-                          aligner: Optional["WindowAligner"] = None):
+                          window_ids: Optional[Sequence[int]] = None, raw_only=False, reuse_features: bool = True):
         """frames uint8 [N,H0,W0,3] -> (float32 [N,H0,W0], target_fps)   (video_depth.py:166-254).
 
         Everything after the upload of the uint8 frames runs on the device: per-window gather + cv2-style
@@ -138,8 +137,7 @@ class VideoDepthAnything(nn.Module):
         statistics and softmax (<= 1e-3 of the fp32 reference on full vitl AND vits windows, tests/test_forward_gpu.py),
         whatever the model's own dtype; the flag is not silently ignored.
         `window_ids` / `raw_only` are the multi-GPU hooks (parallel.py): compute only those windows and return
-        the raw, resized per-window depths [len(window_ids),32,H0,W0] on the device, skipping alignment; with
-        `aligner` the windows are pushed into that WindowAligner instead (the caller finishes it) and None is returned.
+        the raw, resized per-window depths [len(window_ids),32,H0,W0] on the device, skipping alignment.
         `reuse_features`: the DINOv2 encoder is per-frame and 10 of a window's 32 slots repeat frames of earlier
         windows (:200-201), so each source frame is encoded once and its four tap features are kept on the device
         until no later window needs them (FeatureCache); every kernel is batch-invariant, so the result is
@@ -157,8 +155,6 @@ class VideoDepthAnything(nn.Module):
         ids = list(range(len(wins))) if window_ids is None else list(window_ids)
         with torch.cuda.device(self._device):
             if not ids:
-                if aligner is not None:
-                    return None
                 return torch.empty(0, INFER_LEN, h0, w0, device=self._device) if raw_only else \
                     (np.empty((0, h0, w0), np.float32), target_fps)
             needed = sorted({i for k in ids for i in wins[k]})
@@ -167,9 +163,7 @@ class VideoDepthAnything(nn.Module):
             up = FrameUploader(frames, needed, self._device, ring=not raw_only and all(a < b for a, b in zip(ids, ids[1:])))
             # raw stack allocated once: a fresh 34 MB block per window costs a cudaMalloc each (~10 ms at 518x518)
             raws = torch.empty(len(ids), INFER_LEN, h0, w0, dtype=torch.float32, device=self._device) if raw_only else None
-            own_aligner = aligner is None and not raw_only
-            if own_aligner:
-                aligner = WindowAligner(n, h0, w0, self._device, "identity" if self.metric else "affine")
+            aligner = None if raw_only else WindowAligner(n, h0, w0, self._device, "identity" if self.metric else "affine")
             cache = FeatureCache(eng, up, nh, nw, [wins[k] for k in ids]) if reuse_features else None
             if cache is None:     # all index lists in one upload (a per-window pageable H2D would sync the stream)
                 idx_all = torch.tensor([[up.slot[i] for i in wins[k]] for k in ids], dtype=torch.int32).pin_memory() \
@@ -191,8 +185,6 @@ class VideoDepthAnything(nn.Module):
             up.close()
             if raw_only:
                 return raws
-            if not own_aligner:
-                return None
             return aligner.result(), target_fps
 
     # ---- streaming -----------------------------------------------------------------------------
@@ -465,7 +457,7 @@ class FrameUploader:
         self.read_ev = [None] * (self.RING_CHUNKS if self.ring else 0)   # event: the kernels that read the chunk in this ring region are queued
         self.stream = torch.cuda.Stream(device=device)
         # `dev` comes from the caching allocator of the compute stream and may be a block that kernels of an earlier call
-        # (still queued on that stream: the raw_only / aligner paths return without synchronising) are yet to read: the
+        # (still queued on that stream: the raw_only path returns without synchronising) are yet to read: the
         # copy stream starts after everything issued so far, and the block is not recycled before the copies are done
         self.stream.wait_stream(torch.cuda.current_stream(device))
         self.dev.record_stream(self.stream)
