@@ -177,6 +177,17 @@ int vda_attention_temporal_step_batched(const void* qkv, void* pool, const float
 int vda_preprocess_frames(const uint8_t* frames, const int32_t* idx, float* out, int n, int H0, int W0, int nh, int nw,
                           void* stream);
 
+/* Frame preprocessing of a ragged batch (util/transform.py:109-158): batch row i < n is its own frame, described by
+ * rows[i] (device memory, read by the kernel); every row is resized to the same (nh, nw) -> out fp32 [n, 3, nh, nw].
+ * Per row bit-identical to vda_preprocess_frames of that frame alone (same per-pixel code).  Pixels are 3 contiguous
+ * bytes (RGB), row y of a frame starts at src + y * pitch, pitch >= 3 * W0. */
+typedef struct vda_frame_desc {
+  const uint8_t* src;
+  int64_t pitch;
+  int32_t H0, W0;
+} vda_frame_desc;
+int vda_preprocess_frames_ragged(const vda_frame_desc* rows, int n, int nh, int nw, float* out, void* stream);
+
 /* Encoder-feature reuse across overlapping windows (video_depth.py:197-201: 10 of a window's 32 slots repeat frames
  * of earlier windows, and the DINOv2 encoder is per-frame): copies n per-frame slabs of frame_bytes bytes, slab
  * src_idx[i] of src -> slab dst_idx[i] of dst (device int32 lists; NULL = identity).  frame_bytes % 16 == 0. */
@@ -238,6 +249,15 @@ int vda_tail_fused(const void* in, const void* w, const float* bias, const float
 
 /* bilinear, align_corners=True, single-channel fp32 [n,ih,iw] -> [n,oh,ow] (video_depth.py:162,208) */
 int vda_bilinear_f32(const float* in, float* out, int n, int ih, int iw, int oh, int ow, void* stream);
+
+/* The same per row of a ragged batch (video_depth.py:208): row i of in fp32 [n, ih, iw] -> rows[i].dst fp32
+ * [rows[i].H0, rows[i].W0] (descriptors in device memory, read by the kernel), bit-identical to vda_bilinear_f32 of that
+ * row alone; a row of size (ih, iw) is copied, a row with H0 == 0 writes nothing. */
+typedef struct vda_out_desc {
+  float* dst;
+  int32_t H0, W0;
+} vda_out_desc;
+int vda_bilinear_f32_ragged(const float* in, const vda_out_desc* rows, int n, int ih, int iw, void* stream);
 
 /* h16 elementwise: out = a + b (either may alias out) */
 int vda_add_h16(const void* a, const void* b, void* out, int64_t n, int dtype, void* stream);

@@ -14,6 +14,15 @@ shapes also the batched kernel at B = 8 (8 streams' frames in one launch).
 Then stream groups (VideoDepthAnything.stream_group) of each --streams count for ViT-S and ViT-L at 518x518: every push
 names every stream, push latency p50 / p99 over --group-pushes pushes after 40 warm-up pushes, and aggregate frames/s
 (streams / p50 push).
+With --mixed (ViT-L, bf16, each count of --mixed-streams): cameras of two frame sizes that share one network size
+(1280x720 and 1920x1080 -> 518x924), push p50 / p99 (host clock, every push names every stream, --group-pushes pushes
+after 40 warm-up pushes) and aggregate frames/s for
+  (a) one group, every camera 1280x720 (host frames, host depths: the only form before per-stream sizes);
+  (b) one group, half the cameras 1280x720 and half 1920x1080;
+  (c) (b) with the frames as CUDA tensors and to_host=False (depths stay on the device);
+  (d) the cameras of (b) as two groups, one per frame size, pushed one after the other (a push = both pushes);
+then, in a run of its own under torch.profiler (graphs off, so every kernel is listed), the device time of the ragged
+ingest and egress kernels within a push of (b) and (c).
 The card's name and power limit are read in the same run."""
 import argparse
 import json
@@ -153,6 +162,100 @@ def bench_group(enc, h0, w0, S, warmup, pushes, dtype):
             "aggregate_fps": round(S * 1e3 / p50, 1)}
 
 
+MIXED_SIZES = [(720, 1280), (1080, 1920)]
+
+
+def bench_mixed(S, warmup, pushes, dtype):
+    """Arms (a)-(d) of the module docstring at S cameras."""
+    m = model("vitl", dtype)
+    rng = np.random.default_rng(0)
+    host = {hw: rng.integers(0, 256, (4, *hw, 3), dtype=np.uint8) for hw in MIXED_SIZES}
+    dev = {hw: torch.from_numpy(f).cuda() for hw, f in host.items()}
+    half = [MIXED_SIZES[0]] * (S // 2) + [MIXED_SIZES[1]] * (S - S // 2)
+
+    def timed(push):
+        ts = []
+        for t in range(warmup + pushes):
+            t0 = time.perf_counter()
+            push(t)
+            if t >= warmup:
+                ts.append((time.perf_counter() - t0) * 1e3)
+        return ts
+
+    def one_group(sizes, frames, to_host):
+        g = m.stream_group(max_streams=S)
+        hs = [(g.open(), hw) for hw in sizes]
+        ts = timed(lambda t: g.push({h: frames[hw][(t + i) % 4] for i, (h, hw) in enumerate(hs)}, to_host=to_host))
+        g.close()
+        return ts
+
+    def two_groups():
+        gs = []
+        for hw in MIXED_SIZES:
+            g = m.stream_group(max_streams=S // 2)
+            gs.append((g, [g.open() for _ in range(S // 2)], hw))
+        ts = timed(lambda t: [g.push({h: host[hw][(t + i) % 4] for i, h in enumerate(hs)}) for g, hs, hw in gs])
+        for g, _, _ in gs:
+            g.close()
+        return ts
+
+    arms = {"a_uniform_720p_host": lambda: one_group([MIXED_SIZES[0]] * S, host, True),
+            "b_mixed_host": lambda: one_group(half, host, True),
+            "c_mixed_cuda_frames_cuda_depth": lambda: one_group(half, dev, False),
+            "d_two_groups_host": two_groups}
+    out = {"streams": S, "frames": [list(hw) for hw in MIXED_SIZES], "network": list(get_resize_hw(*MIXED_SIZES[0]))}
+    for name, run in arms.items():
+        ts = run()
+        torch.cuda.empty_cache()
+        p50 = pct(ts, 50)
+        out[name] = {"push_ms_p50": round(p50, 3), "push_ms_p99": round(pct(ts, 99), 3),
+                     "aggregate_fps": round(S * 1e3 / p50, 1)}
+    del m
+    torch.cuda.empty_cache()
+    return out
+
+
+def profile_ragged(S, dtype, pushes=5):
+    """Device time per push of the two ragged kernels and of all kernels, arms (b) and (c), from torch.profiler."""
+    from torch.profiler import ProfilerActivity, profile
+    m = model("vitl", dtype)
+    eng = m._ensure_engine()
+    rng = np.random.default_rng(0)
+    half = [MIXED_SIZES[0]] * (S // 2) + [MIXED_SIZES[1]] * (S - S // 2)
+    host = [rng.integers(0, 256, (*hw, 3), dtype=np.uint8) for hw in half]
+    res = {}
+    for arm, frames, to_host in (("b_mixed_host", host, True),
+                                 ("c_mixed_cuda_frames_cuda_depth", [torch.from_numpy(f).cuda() for f in host], False)):
+        g = m.stream_group(max_streams=S)
+        hs = [g.open() for _ in half]
+        eng.use_graphs = False                        # eager: the same launches as the graph, each one traced
+        for _ in range(2):
+            g.push(dict(zip(hs, frames)), to_host=to_host)
+        torch.cuda.synchronize()
+        with profile(activities=[ProfilerActivity.CUDA]) as prof:
+            for _ in range(pushes):
+                g.push(dict(zip(hs, frames)), to_host=to_host)
+            torch.cuda.synchronize()
+        eng.use_graphs = True
+        g.close()
+        kern = {"preprocess_ragged_kernel": 0.0, "bilinear_f32_ragged_kernel": 0.0}
+        total = 0.0
+        for e in prof.key_averages():
+            us = e.device_time_total
+            if e.device_type.name != "CUDA" or us <= 0:
+                continue
+            if "Memcpy" not in e.key and "Memset" not in e.key:
+                total += us
+            for k in kern:
+                if k in e.key:
+                    kern[k] += us
+        res[arm] = {**{k + "_us_per_push": round(v / pushes, 1) for k, v in kern.items()},
+                    "all_kernels_ms_per_push": round(total / pushes / 1e3, 3)}
+    del m
+    torch.cuda.empty_cache()
+    return res
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--warmup", type=int, default=40)
@@ -160,11 +263,18 @@ def main():
     ap.add_argument("--streams", default="", help="comma-separated stream counts for the group sweep, e.g. 1,2,4,8,16")
     ap.add_argument("--group-pushes", type=int, default=100)
     ap.add_argument("--skip-single", action="store_true", help="only the group sweep and the batched kernel")
+    ap.add_argument("--mixed", action="store_true", help="only the mixed frame size / CUDA frame arms (a)-(d)")
+    ap.add_argument("--mixed-streams", default="8,16")
     ap.add_argument("--out", default=os.path.join(ROOT, "profiles", "stream_b200.json"))
     a = ap.parse_args()
     counts = [int(x) for x in a.streams.split(",") if x]
     if not torch.cuda.is_available():
         sys.exit("bench_stream.py needs a GPU")
+    if a.mixed:
+        res = {"what": "stream groups of mixed frame sizes, host vs CUDA frames (ViT-L bf16)", **card(),
+               "mixed": [bench_mixed(int(S), a.warmup, a.group_pushes, torch.bfloat16) for S in a.mixed_streams.split(",")],
+               "ragged_kernels_profiled": {S: profile_ragged(int(S), torch.bfloat16) for S in a.mixed_streams.split(",")}}
+        return write(res, a.out)
     res = {"what": "streaming push latency / step device time / step kernel", **card(), "configs": [], "step_kernel": []}
     seen = set()
     for enc, h0, w0 in CONFIGS:
@@ -185,10 +295,14 @@ def main():
                                  for mm, (hw, C) in enumerate(vitl)]
         res["groups"] = [bench_group(enc, 518, 518, S, a.warmup, a.group_pushes, torch.bfloat16)
                          for enc in ("vits", "vitl") for S in counts]
+    write(res, a.out)
+
+
+def write(res, path):
     line = json.dumps(res)
     print(line)
-    os.makedirs(os.path.dirname(os.path.abspath(a.out)), exist_ok=True)
-    with open(a.out, "w") as f:
+    os.makedirs(os.path.dirname(os.path.abspath(path)), exist_ok=True)
+    with open(path, "w") as f:
         f.write(line + "\n")
 
 

@@ -56,6 +56,7 @@ _SIGS = {
     "vda_attention_temporal_step_batched": (C.c_int, [C.c_void_p] * 6 + [C.c_int] * 8 + [C.c_void_p]),
     "vda_preprocess_frames": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int,
                                         C.c_void_p]),
+    "vda_preprocess_frames_ragged": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p]),
     "vda_copy_frames": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int64, C.c_void_p]),
     "vda_eval_sequence": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int64, C.c_double, C.c_void_p, C.c_void_p,
                                     C.c_void_p, C.c_void_p]),
@@ -71,6 +72,7 @@ _SIGS = {
     "vda_tail_fused": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_float, C.c_void_p, C.c_int, C.c_int,
                                  C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p]),
     "vda_bilinear_f32": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p]),
+    "vda_bilinear_f32_ragged": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p]),
     "vda_add_h16": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_int, C.c_void_p]),
     "vda_lsq_scale_shift": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p]),
     "vda_align_chain": (C.c_int, [C.c_void_p, C.c_int, C.c_int64, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]),

@@ -1,6 +1,6 @@
 // Bandwidth-bound data-movement kernels: patch im2col, cls/pos-embed, bicubic pos-embed resampling,
-// stride-2 im2col, bilinear (align_corners=True) resampling, elementwise add.  All 128-bit vectorised along
-// the contiguous (channel) dimension, grid-stride loops sized in multiples of the SM count.
+// stride-2 im2col, bilinear (align_corners=True) resampling (also of a ragged batch), elementwise add.  All 128-bit
+// vectorised along the contiguous (channel) dimension, grid-stride loops sized in multiples of the SM count.
 #include "../../include/vda.h"
 #include "common.cuh"
 
@@ -175,6 +175,38 @@ __global__ void bilinear_f32_kernel(const float* __restrict__ in, float* __restr
   }
 }
 
+// Ragged batch: row f of in [n, ih, iw] goes to rows[f].dst at its own (H0, W0), grid (x, n) with a grid-stride loop
+// over the row's pixels, so the launch does not depend on the sizes.  Same arithmetic as bilinear_f32_kernel; the
+// scales are the host's IEEE divisions (__fdiv_rn: the library is built with --use_fast_math).  A row of the input's
+// size is copied (the caller skipped the resize there before); H0 == 0 writes nothing (pad rows).
+__global__ void __launch_bounds__(256)
+bilinear_f32_ragged_kernel(const float* __restrict__ in, const vda_out_desc* __restrict__ rows, int ih, int iw) {
+  const int img = blockIdx.y;
+  const vda_out_desc r = rows[img];
+  const int oh = r.H0, ow = r.W0;
+  const long long total = static_cast<long long>(oh) * ow;
+  const float* b = in + static_cast<long long>(img) * ih * iw;
+  const bool same = oh == ih && ow == iw;
+  const float sy = oh > 1 ? __fdiv_rn(static_cast<float>(ih - 1), static_cast<float>(oh - 1)) : 0.f;
+  const float sx = ow > 1 ? __fdiv_rn(static_cast<float>(iw - 1), static_cast<float>(ow - 1)) : 0.f;
+  for (long long idx = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x; idx < total;
+       idx += static_cast<long long>(gridDim.x) * blockDim.x) {
+    if (same) {
+      r.dst[idx] = b[idx];
+      continue;
+    }
+    const int ox = static_cast<int>(idx % ow);
+    const int oy = static_cast<int>(idx / ow);
+    const float fy = sy * oy, fx = sx * ox;
+    const int y0 = min(static_cast<int>(fy), ih - 1), x0 = min(static_cast<int>(fx), iw - 1);
+    const int y1 = min(y0 + 1, ih - 1), x1 = min(x0 + 1, iw - 1);
+    const float ly = fy - y0, lx = fx - x0;
+    const float top = b[y0 * iw + x0] * (1.f - lx) + b[y0 * iw + x1] * lx;
+    const float bot = b[y1 * iw + x0] * (1.f - lx) + b[y1 * iw + x1] * lx;
+    r.dst[idx] = top * (1.f - ly) + bot * ly;
+  }
+}
+
 template <typename T>
 __global__ void add_h16_kernel(const T* __restrict__ a, const T* __restrict__ b, T* __restrict__ out, long long nvec) {
   for (long long idx = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x; idx < nvec;
@@ -265,6 +297,16 @@ extern "C" int vda_bilinear_f32(const float* in, float* out, int n, int ih, int 
   const float sx = ow > 1 ? static_cast<float>(iw - 1) / (ow - 1) : 0.f;
   const long long total = static_cast<long long>(n) * oh * ow;
   bilinear_f32_kernel<<<grid_for(total, 256), 256, 0, static_cast<cudaStream_t>(stream)>>>(in, out, n, ih, iw, oh, ow, sy, sx);
+  VDA_CUDA(cudaGetLastError());
+  return 0;
+}
+
+extern "C" int vda_bilinear_f32_ragged(const float* in, const vda_out_desc* rows, int n, int ih, int iw, void* stream) {
+  VDA_CHECK(n > 0 && ih > 0 && iw > 0, "bilinear_f32_ragged: bad shape");
+  // fixed grid (sizes live in device memory): about 8 CTAs per SM over the whole batch, at least one per row
+  const unsigned gx = static_cast<unsigned>(n >= 148 * 8 ? 1 : (148 * 8) / n);
+  bilinear_f32_ragged_kernel<<<dim3(gx, static_cast<unsigned>(n)), 256, 0, static_cast<cudaStream_t>(stream)>>>(in, rows, ih,
+                                                                                                             iw);
   VDA_CUDA(cudaGetLastError());
   return 0;
 }

@@ -554,16 +554,15 @@ class Engine:
         hws = [hp * wp, ((hp - 1) // 2 + 1) * ((wp - 1) // 2 + 1), hp * wp, 4 * hp * wp]
         return [self._hnew(S, slots, hws[m], 2 * self.mm_c[m]) for m in range(4) for _ in (0, 1)]
 
-    def stream_group_step(self, frames: torch.Tensor, idx: torch.Tensor, rows: torch.Tensor, ctx: torch.Tensor,
-                          pool: List[torch.Tensor], nh: int, nw: int) -> torch.Tensor:
-        """One streamed frame of each of B streams: frames uint8 [*,H0,W0,3] (device), batch row b takes frame idx[b]
-        (int32 [B]), pool entry rows[b] (int32 [B], -1: pad row) and context row ctx[b] (int32 [B, stride], see
-        vda_attention_temporal_step_batched) -> fp32 depth [B,H0,W0] (>= 0).  Preprocessing as in infer_video_depth,
-        encoder and head on the B frames at T = 1 with every temporal attention against the rows' pool entries,
-        bilinear resize to the frame size.  The launches do not depend on B.  No host decisions: graph-capturable."""
-        h0, w0 = frames.shape[1:3]
-        x = ops.preprocess_frames(frames, idx, nh, nw)
-        d = self.head(self.encode(x), idx.numel(), 1, nh // 14, nw // 14, stream=(pool, rows, ctx))
-        if (nh, nw) != (h0, w0):
-            d = ops.bilinear_f32(d, h0, w0)
-        return d
+    def stream_group_step(self, frame_desc: torch.Tensor, out_desc: torch.Tensor, rows: torch.Tensor, ctx: torch.Tensor,
+                          pool: List[torch.Tensor], nh: int, nw: int) -> None:
+        """One streamed frame of each of B streams, every frame of its own size: batch row b reads the frame frame_desc[b]
+        and writes its depth fp32 [H0,W0] (>= 0) to out_desc[b] (vda_frame_desc / vda_out_desc arrays, device bytes,
+        windows.group_descriptors), takes pool entry rows[b] (int32 [B], -1: pad row) and context row ctx[b] (int32
+        [B, stride], see vda_attention_temporal_step_batched).  Preprocessing to (nh, nw) as in infer_video_depth,
+        encoder and head on the B frames at T = 1 with every temporal attention against the rows' pool entries, bilinear
+        resize to each row's frame size.  The launches depend on neither B nor the sizes.  No host decisions:
+        graph-capturable, and every frame-dependent address is read from the descriptors at run time."""
+        x = ops.preprocess_frames_ragged(frame_desc, nh, nw)
+        d = self.head(self.encode(x), rows.numel(), 1, nh // 14, nw // 14, stream=(pool, rows, ctx))
+        ops.bilinear_f32_ragged(d, out_desc)

@@ -13,6 +13,7 @@ from ._lib import (A_CONV3, A_PLAIN, ACT_GELU, ACT_NONE, ACT_RELU, EPI_CONVT, EP
                    GemmParams, VDA_BF16, VDA_FP16, check)
 
 LSQ_MAX_PARTIALS = 592   # include/vda.h VDA_LSQ_MAX_PARTIALS
+FRAME_DESC_BYTES, OUT_DESC_BYTES = 24, 16   # sizeof(vda_frame_desc), sizeof(vda_out_desc)
 LAUNCHES = 0   # number of libvda kernel launches issued (bench.py reports it as gpu_launches)
 PROFILE = None  # when a list: every op appends (name, info dict, start_event, end_event)   [bench.py / tools]
 _INFO = {}
@@ -247,6 +248,20 @@ def preprocess_frames(frames_u8: torch.Tensor, idx: torch.Tensor, nh: int, nw: i
     return out
 
 
+def preprocess_frames_ragged(rows: torch.Tensor, nh: int, nw: int, out: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """One frame per batch row, each of its own size: rows = the vda_frame_desc array (device bytes [n * 24],
+    windows.FRAME_DESC) -> fp32 [n,3,nh,nw], per row what preprocess_frames gives for that frame alone."""
+    lib = _lib.load()
+    assert rows.dtype == torch.uint8 and rows.is_contiguous() and rows.numel() % FRAME_DESC_BYTES == 0
+    n = rows.numel() // FRAME_DESC_BYTES
+    if out is None:
+        out = torch.empty(n, 3, nh, nw, dtype=torch.float32, device=rows.device)
+    assert out.is_contiguous() and out.dtype == torch.float32 and tuple(out.shape) == (n, 3, nh, nw)
+    check(lib.vda_preprocess_frames_ragged(_p(rows), n, nh, nw, _p(out), _stream()))
+    _count()
+    return out
+
+
 def copy_frames(src: torch.Tensor, src_idx: Optional[torch.Tensor], dst: torch.Tensor, dst_idx: Optional[torch.Tensor],
                 n: int) -> torch.Tensor:
     """dst[dst_idx[i]] = src[src_idx[i]] for i < n over the leading (frame) axis; idx: device int32 or None (identity)."""
@@ -330,6 +345,17 @@ def bilinear_f32(x: torch.Tensor, oh: int, ow: int, out: Optional[torch.Tensor] 
     return out
 
 
+def bilinear_f32_ragged(x: torch.Tensor, rows: torch.Tensor) -> None:
+    """x fp32 [n,ih,iw] -> row i resized (align_corners=True) into its vda_out_desc rows[i] (device bytes [n * 16],
+    windows.OUT_DESC): dst [H0,W0], bit-identical to bilinear_f32 of that row alone; H0 = 0 writes nothing."""
+    lib = _lib.load()
+    n, ih, iw = x.shape
+    assert x.is_contiguous() and x.dtype == torch.float32
+    assert rows.dtype == torch.uint8 and rows.is_contiguous() and rows.numel() == n * OUT_DESC_BYTES
+    check(lib.vda_bilinear_f32_ragged(_p(x), _p(rows), n, ih, iw, _stream()))
+    _count()
+
+
 def add_h16(a: torch.Tensor, b: torch.Tensor, out: torch.Tensor):
     lib = _lib.load()
     check(lib.vda_add_h16(_p(a), _p(b), _p(out), a.numel(), dt_code(a.dtype), _stream()))
@@ -385,8 +411,8 @@ def _profiled(fn, name):
     return wrapper
 
 
-for _n in ("preprocess_frames", "copy_frames", "gemm", "layernorm", "rowstats_cast", "groupnorm", "attention_spatial", "attention_temporal",
+for _n in ("preprocess_frames", "preprocess_frames_ragged", "copy_frames", "gemm", "layernorm", "rowstats_cast", "groupnorm", "attention_spatial", "attention_temporal",
            "attention_temporal_step", "patch_im2col", "write_cls",
-           "pos_embed_bicubic", "im2col3x3_s2", "bilinear_nhwc", "tail_fused", "bilinear_f32", "add_h16", "lsq_scale_shift", "align_chain",
+           "pos_embed_bicubic", "im2col3x3_s2", "bilinear_nhwc", "tail_fused", "bilinear_f32", "bilinear_f32_ragged", "add_h16", "lsq_scale_shift", "align_chain",
            "affine_clamp_blend"):
     globals()[_n] = _profiled(globals()[_n], _n)

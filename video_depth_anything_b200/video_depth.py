@@ -26,8 +26,8 @@ from . import ops
 from .engine import Engine
 from .synth import ENCODER_DIMS, synth_state_dict
 from .windows import (INFER_LEN, INTERP_LEN, KEYFRAMES, OVERLAP, aligner_ring_len, aligner_ring_pos, get_resize_hw,
-                      StreamGroupPlan, plan_feature_cache, split_group_table, upload_ring_plan,
-                      window_source_indices)
+                      StreamGroupPlan, group_block_layout, group_descriptors, plan_feature_cache, split_group_table,
+                      upload_ring_plan, window_source_indices)
 
 
 VALIDATION_DTYPE = torch.float16     # operand type of the `fp32=True` path (see _ensure_engine)
@@ -201,9 +201,10 @@ class VideoDepthAnything(nn.Module):
         return DepthStreamGroup(self, self._ensure_engine(validation=bool(fp32)), max_streams, input_size)
 
     @torch.no_grad()
-    def infer_video_depth_one(self, frame: np.ndarray, input_size: int = 518, device="cuda", fp32: bool = False) -> np.ndarray:
+    def infer_video_depth_one(self, frame, input_size: int = 518, device="cuda", fp32: bool = False, to_host: bool = True):
         """Depth of the next frame of the model's own stream (the name of the upstream project's streaming entry
-        point): frame uint8 [H0,W0,3] -> float32 [H0,W0].  The stream is opened on the first call and reopened (its
+        point): frame uint8 [H0,W0,3] (numpy array or CUDA tensor) -> float32 [H0,W0] (numpy array, or with
+        `to_host=False` a CUDA tensor; DepthStream.push).  The stream is opened on the first call and reopened (its
         temporal context starts over) when `input_size`, `fp32` or the device change or new weights were loaded."""
         if torch.device(device).type != "cuda":
             raise RuntimeError("infer_video_depth_one: the B200 engine has no CPU path (device must be 'cuda')")
@@ -214,7 +215,7 @@ class VideoDepthAnything(nn.Module):
             if st is not None:
                 st.close()
             st = self._stream_one = self.stream(input_size, fp32)
-        return st.push(frame)
+        return st.push(frame, to_host)
 
 
 class DepthStreamGroup:
@@ -224,14 +225,24 @@ class DepthStreamGroup:
     Each stream follows DepthStream's semantics exactly, with its own step counter t and its own temporal context
     (windows.stream_context over its own row of a pooled k'|v' cache).  A push names any subset of the open streams,
     each at most once; a stream left out does not advance.  The batch is padded up to a bucket (the powers of two below
-    `max_streams`, then `max_streams`; windows.stream_buckets): pad rows take the first frame and pool row -1, which
-    reads and writes no pool byte.  One CUDA graph per bucket, captured on first use and owned by the group (the
-    engine's forward / video graphs neither evict nor are evicted by them).  A push is one H2D of the frames, one H2D of
-    the int32 rows | ctx | idx table, a replay and one D2H of [bucket, H0, W0].
+    `max_streams`, then `max_streams`; windows.stream_buckets): pad rows read the first row's frame, take pool row -1,
+    which reads and writes no pool byte, and write no output.  One CUDA graph per bucket, captured on first use and
+    owned by the group (the engine's forward / video graphs neither evict nor are evicted by them).
+
+    Sizes: one network size per group, fixed by the first push (windows.get_resize_hw of its frames); every stream has
+    its own frame size, fixed by its first frame (a closed stream's pool row starts over with a new size).  So 1280x720
+    and 1920x1080 cameras (both 518x924) share a group; a 640x480 camera (518x686) needs a group of its own.
+
+    Frames are uint8 RGB [H0, W0, 3], as numpy arrays or as CUDA tensors on the group's device (rows may be pitched:
+    stride (pitch, 3, 1)), mixed freely.  Every frame-dependent address and size of a push is in a per-row descriptor
+    block in device memory (windows.group_descriptors), so the graphs replay whatever mix of sizes and buffers later
+    pushes bring.  A push is one H2D of the host frames (packed in a pinned arena, read from a device arena), one H2D
+    of the descriptors and the int32 rows | ctx | idx table, a replay, and with to_host one D2H of the depths (packed in
+    a device arena).  CUDA frames are read in place.  The arenas grow to the largest push seen; growing captures nothing.
 
     Device memory: the pool holds max_streams x (L + 1) = 32 frame slots per temporal-attention block, allocated at the
-    first push: 903 MB per stream for ViT-L at 518x518 (214 MB for ViT-S), plus one graph's activations per bucket used.
-    Frame size (and so the network size) is fixed by the first push, for every stream of the group."""
+    first push: 903 MB per stream for ViT-L at 518x518 (214 MB for ViT-S), plus one graph's activations per bucket used
+    and the arenas."""
 
     def __init__(self, model: VideoDepthAnything, engine: Engine, max_streams: int = 8, input_size: int = 518):
         self.engine, self.input_size = engine, int(input_size)
@@ -240,11 +251,11 @@ class DepthStreamGroup:
         L = model.num_frames - 1
         if not 1 <= L <= INFER_LEN - 1:
             raise ValueError(f"streaming needs num_frames in 2..{INFER_LEN}, got {model.num_frames}")
-        self.plan = StreamGroupPlan(int(max_streams), L)
+        self.plan = StreamGroupPlan(int(max_streams), L, self.input_size)
         self.max_streams = self.plan.max_streams
-        self.size = None                             # (h0, w0), fixed by the first push
         self.pool = None
         self.graphs = {}                             # bucket -> captured step (Engine.run_graphed)
+        self.arenas = {}                             # name -> buffer, grown on demand (_arena)
         self.closed = False
 
     def open(self) -> int:
@@ -257,67 +268,111 @@ class DepthStreamGroup:
         """Close one stream; its pool row is free for a later open (which starts over at t = 0)."""
         self.plan.close(handle)
 
-    def _alloc(self, h0: int, w0: int) -> None:
+    def _alloc(self) -> None:
         eng, S, L = self.engine, self.max_streams, self.plan.L
-        self.nh, self.nw = get_resize_hw(h0, w0, self.input_size)
+        self.nh, self.nw = self.plan.net
+        nbytes = group_block_layout(S, L)[2].stop
         with torch.cuda.device(self.device):
             self.pool = eng.stream_pool(S, self.nh // 14, self.nw // 14, L + 1)
-            self.frames_dev = torch.empty(S, h0, w0, 3, dtype=torch.uint8, device=self.device)
-            self.table_dev = torch.zeros(S * (L + 4), dtype=torch.int32, device=self.device)
-            self.frames_host = torch.empty(S, h0, w0, 3, dtype=torch.uint8).pin_memory()
-            self.table_host = torch.zeros(S * (L + 4), dtype=torch.int32).pin_memory()
-            self.out_host = torch.empty(S, h0, w0, dtype=torch.float32).pin_memory()
-        self.size = (h0, w0)
+            self.meta_dev = torch.zeros(nbytes, dtype=torch.uint8, device=self.device)
+            self.meta_host = torch.zeros(nbytes, dtype=torch.uint8).pin_memory()
 
-    def _step(self, bk: int) -> torch.Tensor:
+    def _arena(self, name: str, n: int, dtype, pinned: bool) -> torch.Tensor:
+        """Buffer `name` with at least n elements; regrown (in 2 MiB steps) only when a push needs more."""
+        t = self.arenas.get(name)
+        if t is None or t.numel() < n:
+            n = -(-max(n, 1) * dtype.itemsize // (2 << 20)) * (2 << 20) // dtype.itemsize
+            t = torch.empty(n, dtype=dtype).pin_memory() if pinned else torch.empty(n, dtype=dtype, device=self.device)
+            self.arenas[name] = t
+        return t
+
+    def _step(self, bk: int) -> None:
         eng = self.engine
-        rows, ctx, idx = split_group_table(self.table_dev, bk, self.plan.L)
-        inputs = [self.frames_dev, idx, rows, ctx]
+        fs, os_, ts = group_block_layout(bk, self.plan.L)
+        rows, ctx, _ = split_group_table(self.meta_dev[ts].view(torch.int32), bk, self.plan.L)
+        inputs = [self.meta_dev[fs], self.meta_dev[os_], rows, ctx]
 
-        def fn(frames, idx, rows, ctx):
-            return eng.stream_group_step(frames, idx, rows, ctx, self.pool, self.nh, self.nw)
+        def fn(frame_desc, out_desc, rows, ctx):
+            return eng.stream_group_step(frame_desc, out_desc, rows, ctx, self.pool, self.nh, self.nw)
         if eng.use_graphs and ops.PROFILE is None:
             return eng.run_graphed(self.graphs, bk, fn, inputs, adopt=True)
         return fn(*inputs)
 
+    def _check_frame(self, f):
+        if isinstance(f, torch.Tensor):
+            if not f.is_cuda or f.device != self.device:
+                raise ValueError(f"a tensor frame must be a CUDA tensor on the group's device {self.device}, got {f.device}")
+            if f.dtype != torch.uint8 or f.dim() != 3 or f.shape[2] != 3:
+                raise ValueError(f"a CUDA frame must be a uint8 tensor [H0,W0,3], got {f.dtype} {tuple(f.shape)}")
+            if f.stride(2) != 1 or f.stride(1) != 3 or f.stride(0) < 3 * f.shape[1]:
+                raise ValueError(f"a CUDA frame's pixels must be contiguous, stride (pitch >= 3 * W0, 3, 1), "
+                                 f"got {f.stride()}")
+        elif not isinstance(f, np.ndarray) or f.ndim != 3 or f.shape[2] != 3 or f.dtype != np.uint8:
+            raise ValueError("a frame must be a uint8 numpy array [H0,W0,3] or a uint8 CUDA tensor [H0,W0,3]")
+        return int(f.shape[0]), int(f.shape[1])
+
     @torch.no_grad()
-    def push(self, frames) -> dict:
-        """frames: {handle: uint8 RGB [H0,W0,3]} (or (handle, frame) pairs) -> {handle: depth float32 [H0,W0] (>= 0)},
-        fresh arrays."""
+    def push(self, frames, to_host: bool = True) -> dict:
+        """frames: {handle: uint8 RGB [H0,W0,3] numpy array or CUDA tensor} (or (handle, frame) pairs) ->
+        {handle: depth [H0,W0] (>= 0)}: fresh float32 numpy arrays, or with `to_host=False` fresh float32 CUDA tensors
+        on the group's device (no device-to-host copy).  Returns after the step has finished, so the caller may reuse
+        its frame buffers at once."""
         if self.closed:
             raise RuntimeError("push on a closed DepthStreamGroup")
         if self.engine.generation != self.generation or not self.engine.loaded:
             raise RuntimeError("the model's weights changed since this stream group was opened; open a new one")
         items = list(frames.items()) if isinstance(frames, dict) else list(frames)
-        size = self.size
-        for _, f in items:
-            if not isinstance(f, np.ndarray) or f.ndim != 3 or f.shape[2] != 3 or f.dtype != np.uint8:
-                raise ValueError("a frame must be a uint8 numpy array [H0,W0,3]")
-            size = size or tuple(f.shape[:2])
-            if tuple(f.shape[:2]) != size:
-                raise ValueError(f"frame size {tuple(f.shape[:2])} differs from the group's {size}")
+        sizes = [self._check_frame(f) for _, f in items]
         handles = [h for h, _ in items]
-        bk, table = self.plan.step(handles)          # ValueError: empty push, unknown / closed / repeated handle
-        if self.size is None:
-            self._alloc(*size)
-        n = len(items)
-        np.copyto(self.table_host.numpy()[:table.size], table)
-        fh = self.frames_host.numpy()
-        for i, (_, f) in enumerate(items):
-            np.copyto(fh[i], f)
+        # ValueError: empty push, unknown / closed / repeated handle, a frame size the group cannot take
+        bk, table = self.plan.step(handles, sizes)
+        if self.pool is None:
+            self._alloc()
+        host = [i for i, (_, f) in enumerate(items) if isinstance(f, np.ndarray)]
+        packed = np.cumsum([0] + [3 * sizes[i][0] * sizes[i][1] for i in host]).tolist()   # host frames, packed
+        in_off, in_bytes = dict(zip(host, packed)), packed[-1]
+        out_off = np.cumsum([0] + [h0 * w0 for h0, w0 in sizes]).tolist()                  # depths, packed
+        out_elems = out_off[-1]
         with torch.cuda.device(self.device):
-            self.frames_dev[:n].copy_(self.frames_host[:n], non_blocking=True)
-            self.table_dev[:table.size].copy_(self.table_host[:table.size], non_blocking=True)
-            d = self._step(bk)
-            self.out_host[:bk].copy_(d, non_blocking=True)
-            torch.cuda.current_stream().synchronize()   # (also: the pinned inputs are free for the next push)
-        out = self.out_host.numpy()
-        return {h: out[i].copy() for i, h in enumerate(handles)}
+            if host:
+                in_host = self._arena("in_host", in_bytes, torch.uint8, True)
+                in_dev = self._arena("in_dev", in_bytes, torch.uint8, False)
+                ih = in_host.numpy()
+                for i in host:
+                    h0, w0 = sizes[i]
+                    np.copyto(ih[in_off[i]:in_off[i] + 3 * h0 * w0].reshape(h0, w0, 3), items[i][1])
+            srcs = [(f.data_ptr(), f.stride(0), h0, w0) if isinstance(f, torch.Tensor) else
+                    (in_dev.data_ptr() + in_off[i], 3 * w0, h0, w0) for i, ((_, f), (h0, w0)) in enumerate(zip(items, sizes))]
+            if to_host:
+                out_dev = self._arena("out_dev", out_elems, torch.float32, False)
+                dsts = [out_dev.data_ptr() + 4 * o for o in out_off[:-1]]
+            else:
+                # the kernel writes straight into the returned tensors (one allocation each from the caching allocator):
+                # no device-to-device pass over the depths, and no arena a caller's tensor could alias
+                outs = [torch.empty(h0, w0, dtype=torch.float32, device=self.device) for h0, w0 in sizes]
+                dsts = [o.data_ptr() for o in outs]
+            fd, od = group_descriptors(bk, srcs, dsts)
+            fs, os_, ts = group_block_layout(bk, self.plan.L)
+            mh = self.meta_host.numpy()
+            mh[fs], mh[os_], mh[ts] = fd.view(np.uint8), od.view(np.uint8), table.view(np.uint8)
+            if host:
+                in_dev[:in_bytes].copy_(in_host[:in_bytes], non_blocking=True)
+            self.meta_dev[:ts.stop].copy_(self.meta_host[:ts.stop], non_blocking=True)
+            self._step(bk)
+            if to_host:
+                out_host = self._arena("out_host", out_elems, torch.float32, True)
+                out_host[:out_elems].copy_(out_dev[:out_elems], non_blocking=True)
+            torch.cuda.current_stream().synchronize()   # (also: the pinned arenas are free for the next push)
+        if not to_host:
+            return dict(zip(handles, outs))
+        oh = out_host.numpy()
+        return {h: oh[out_off[i]:out_off[i + 1]].reshape(sizes[i]).copy() for i, h in enumerate(handles)}
 
     def close(self) -> None:
-        """Release the group's graphs and pool (also done when the object is collected)."""
+        """Release the group's graphs, pool and arenas (also done when the object is collected)."""
         self.graphs = {}
         self.pool = None
+        self.arenas = {}
         self.closed = True
 
     def __del__(self):
@@ -341,17 +396,19 @@ class DepthStream:
     A cached frame is kept as its k'|v' = LayerNorm output @ [W_k | W_v]^T rows, without the positional encoding, whose
     share is added by the step kernel at the frame's current position: a step never re-projects old frames.  Device
     memory is bounded: L + 1 cache slots per block.  A DepthStream is a DepthStreamGroup of one stream: the whole step
-    (preprocess, encoder, head, resize) is one CUDA graph; a push is one H2D of the frame and of the context, a replay
-    and one D2H of the depth.  Frame size (and so the network size) is fixed by the first frame."""
+    (preprocess, encoder, head, resize) is one CUDA graph; a push is one H2D of the frame (none for a CUDA frame) and of
+    the context, a replay and one D2H of the depth (none with to_host=False).  Frame size (and so the network size) is
+    fixed by the first frame."""
 
     def __init__(self, model: VideoDepthAnything, engine: Engine, input_size: int = 518):
         self.group = DepthStreamGroup(model, engine, 1, input_size)
         self.engine, self.input_size, self.generation = engine, self.group.input_size, self.group.generation
         self.handle = self.group.open()
 
-    def push(self, frame: np.ndarray) -> np.ndarray:
-        """frame uint8 RGB [H0,W0,3] -> its depth float32 [H0,W0] (>= 0); a fresh array on every call."""
-        return self.group.push([(self.handle, frame)])[self.handle]
+    def push(self, frame, to_host: bool = True):
+        """frame uint8 RGB [H0,W0,3] (numpy array, or CUDA tensor on the stream's device, rows may be pitched) -> its
+        depth float32 [H0,W0] (>= 0): a fresh numpy array on every call, or with `to_host=False` a fresh CUDA tensor."""
+        return self.group.push([(self.handle, frame)], to_host)[self.handle]
 
     def close(self) -> None:
         """Release the stream's graph and cache (also done when the object is collected)."""

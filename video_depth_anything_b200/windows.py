@@ -169,13 +169,21 @@ class StreamGroupPlan:
     reused after close) and its own step counter t, which only a push that names it advances.  `step(handles)` returns
     the push's bucket and its int32 table rows [bucket] | ctx [bucket, 2 + L] | idx [bucket]: batch row i < len(handles)
     is stream handles[i] with pool row, stream_context(t, L) as {n_ctx, write slot, context slots...} and frame i;
-    the pad rows behind it take pool row -1, n_ctx = 0 and frame 0."""
+    the pad rows behind it take pool row -1, n_ctx = 0 and frame 0.
 
-    def __init__(self, max_streams: int, L: int = STREAM_CONTEXT):
+    Frame sizes: `step(handles, sizes)` also checks the push's frame sizes [(H0, W0)] (batch-row order).  A stream's
+    size is fixed by its first frame (a reopened pool row starts over with a new size); the group's network size
+    get_resize_hw(H0, W0, input_size) is fixed by its first push, and every frame must map to it.  Nothing changes
+    when a push is rejected."""
+
+    def __init__(self, max_streams: int, L: int = STREAM_CONTEXT, input_size: int = 518):
         self.buckets = stream_buckets(max_streams)
         self.max_streams, self.L = max_streams, L
         self.stride = 2 + L
+        self.input_size = input_size
         self.row, self.t = {}, {}                      # handle -> pool row, handle -> frames pushed so far
+        self.size = {}                                 # handle -> (H0, W0) of its first frame
+        self.net = None                                # (nh, nw) of the group, fixed by the first push
         self._next = 0
 
     def open(self) -> int:
@@ -195,18 +203,44 @@ class StreamGroupPlan:
     def close(self, h) -> None:
         self.check(h)
         del self.row[h], self.t[h]
+        self.size.pop(h, None)
 
     def bucket(self, n: int) -> int:
         return next(b for b in self.buckets if b >= n)
 
-    def step(self, handles):
-        """Table of one push of `handles` (distinct open streams, in batch-row order); advances their t."""
+    def _check_sizes(self, handles, sizes):
+        """The group's network size after this push; ValueError if a frame breaks the size rules."""
+        if len(sizes) != len(handles):
+            raise ValueError("one frame size per stream of the push")
+        net = self.net
+        for h, (h0, w0) in zip(handles, sizes):
+            if h0 < 1 or w0 < 1:
+                raise ValueError(f"empty frame of size {(h0, w0)}")
+            if h in self.size and self.size[h] != (h0, w0):
+                raise ValueError(f"frame size {(h0, w0)} of stream {h!r} differs from its first frame's {self.size[h]}")
+            nhw = get_resize_hw(h0, w0, self.input_size)
+            if net is None:
+                net = nhw
+            elif nhw != net:
+                what = "the group's" if self.net is not None else "that of another frame of this push,"
+                raise ValueError(f"frame size {(h0, w0)} maps to network size {nhw}, {what} {net}; "
+                                 f"streams of other network sizes need a group of their own")
+        return net
+
+    def step(self, handles, sizes=None):
+        """Table of one push of `handles` (distinct open streams, in batch-row order); advances their t.  With `sizes`,
+        the frame sizes of the push are checked and recorded too (see the class docstring)."""
         for h in handles:
             self.check(h)
         if len(set(handles)) != len(handles):
             raise ValueError("a stream is named more than once in one push")
         if not handles:
             raise ValueError("a push names at least one stream")
+        if sizes is not None:
+            sizes = [(int(a), int(b)) for a, b in sizes]
+            self.net = self._check_sizes(handles, sizes)
+            for h, hw in zip(handles, sizes):
+                self.size[h] = hw
         bk = self.bucket(len(handles))
         rows = np.full(bk, -1, np.int32)
         ctx = np.zeros((bk, self.stride), np.int32)
@@ -225,3 +259,32 @@ def split_group_table(table, bk: int, L: int = STREAM_CONTEXT):
     """Views (rows [bk], ctx [bk, 2 + L], idx [bk]) of a StreamGroupPlan table (numpy array or tensor)."""
     s = 2 + L
     return table[:bk], table[bk:bk + bk * s].reshape(bk, s), table[bk + bk * s:bk * (s + 2)]
+
+
+# include/vda.h vda_frame_desc / vda_out_desc: what the ragged ingest and egress kernels read per batch row
+FRAME_DESC = np.dtype([("src", "<u8"), ("pitch", "<i8"), ("H0", "<i4"), ("W0", "<i4")])
+OUT_DESC = np.dtype([("dst", "<u8"), ("H0", "<i4"), ("W0", "<i4")])
+
+
+def group_descriptors(bk: int, frames, dsts):
+    """Descriptor arrays of one push: frames = [(device address, row pitch in bytes, H0, W0)] and dsts = [device address
+    of the fp32 [H0, W0] output] of the real rows in batch-row order -> (FRAME_DESC [bk], OUT_DESC [bk]).  Pad rows read
+    the first row's frame (any valid frame would do) and write nothing (H0 = W0 = 0)."""
+    if not 1 <= len(frames) <= bk or len(dsts) != len(frames):
+        raise ValueError(f"{len(frames)} frames / {len(dsts)} outputs for a bucket of {bk}")
+    fd, od = np.zeros(bk, FRAME_DESC), np.zeros(bk, OUT_DESC)
+    for i, ((src, pitch, h0, w0), dst) in enumerate(zip(frames, dsts)):
+        if pitch < 3 * w0:
+            raise ValueError(f"row pitch {pitch} < 3 * W0 = {3 * w0}")
+        fd[i] = (src, pitch, h0, w0)
+        od[i] = (dst, h0, w0)
+    fd[len(frames):] = fd[0]
+    return fd, od
+
+
+def group_block_layout(bk: int, L: int = STREAM_CONTEXT):
+    """Byte ranges (frame descriptors, output descriptors, int32 table) of a push's metadata block: everything a push
+    uploads besides frame pixels, in one copy.  The descriptors come first, so every part is aligned to its type."""
+    a = bk * FRAME_DESC.itemsize
+    b = a + bk * OUT_DESC.itemsize
+    return slice(0, a), slice(a, b), slice(b, b + 4 * bk * (L + 4))
