@@ -171,6 +171,27 @@ int vda_attention_temporal_step_batched(const void* qkv, void* pool, const float
                                         const int32_t* ctx, void* out, int B, int S, int ctx_stride, int hw, int C,
                                         int heads, int slots, int dtype, void* stream);
 
+/* The streaming step of several consecutive frames of one stream (and of other streams) in one launch.  Arguments as
+ * for vda_attention_temporal_step_batched, with two differences:
+ *   ctx:  a context entry e >= 0 is a slot of the row's pool entry, as there; an entry e < 0 names batch row -1 - e of
+ *         this launch (clamped to 0..B-1): that key's k'|v' are read from the row's block of `qkv` (columns C..3C) at
+ *         the same position, with the positional share of its place in this row's sequence.  So frame t + j of a push
+ *         reads its context frames >= t from the push's own rows and the older ones from the pool.
+ *   pool: only read.  The kernel writes no cache slot: with k >= 2 frames of one stream in a launch, the slot frame
+ *         t + j overwrites (that of frame t + j - L) is still a context slot of the push's earlier rows, so the writes
+ *         are deferred to vda_stream_cache_store, launched after this kernel on the same stream.
+ * Per row, the key order, key-split assignment and arithmetic are those of vda_attention_temporal_step_batched, so a
+ * row is bit-identical to that kernel run with the same keys in the pool.  Pad rows as there. */
+int vda_attention_temporal_step_causal(const void* qkv, const void* pool, const float* pe, const int32_t* rows,
+                                       const int32_t* ctx, void* out, int B, int S, int ctx_stride, int hw, int C,
+                                       int heads, int slots, int dtype, void* stream);
+
+/* The deferred cache write of a causal step: for every real batch row b (0 <= rows[b] < S), its k'|v' (columns C..3C of
+ * its rows of qkv h16 [B*hw, 3*C]) are copied unchanged to pool[rows[b]], slot ctx[b][1] (clamped to 0..slots-1); no
+ * other pool byte is touched.  Bandwidth-bound, 16-byte accesses. */
+int vda_stream_cache_store(const void* qkv, void* pool, const int32_t* rows, const int32_t* ctx, int B, int S,
+                           int ctx_stride, int hw, int C, int slots, int dtype, void* stream);
+
 /* Frame preprocessing of infer_video_depth (video_depth.py:173-185,197-198; util/transform.py:109-158): for every
  * i < n, frame idx[i] of the device-resident uint8 RGB video frames [*, H0, W0, 3] -> /255 -> cv2-style INTER_CUBIC
  * resize to (nh, nw) -> (x - mean) / std (float64) -> out fp32 [n, 3, nh, nw].  idx: device int32 [n]. */

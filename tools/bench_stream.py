@@ -23,6 +23,12 @@ after 40 warm-up pushes) and aggregate frames/s for
   (d) the cameras of (b) as two groups, one per frame size, pushed one after the other (a push = both pushes);
 then, in a run of its own under torch.profiler (graphs off, so every kernel is listed), the device time of the ragged
 ingest and egress kernels within a push of (b) and (c).
+With --chunks (e.g. 1,2,4,8,16): a lone stream pushing k consecutive frames per push (DepthStream.push of a stack) for
+ViT-S 518x518, ViT-L 518x518 and ViT-L 1280x720 (host frames, and CUDA stacks with to_host=False): push p50 / p99 on the
+host clock (push synchronises), frames/s = k / p50, over --chunk-pushes pushes after 6 warm-up pushes of the same k
+(the first captures the bucket's graph); then the causal step kernel alone at the ViT-L 518x518 block shapes (one stream,
+k = 8 rows, 31 context frames each, L2 overwritten between launches) next to the batched kernel at B = 8, and the cache
+store kernel.
 The card's name and power limit are read in the same run."""
 import argparse
 import json
@@ -138,6 +144,83 @@ def bench_kernel(hw, C, dtype, B=1, iters=30):
     gbs = nbytes / (ms * 1e-3) / 1e9
     return {"B": B, "hw": hw, "C": C, "head_dim": C // 8, "us": round(ms * 1e3, 2), "MB": round(nbytes / 1e6, 2),
             "GB_s": round(gbs, 1), "hbm_share": round(gbs * 1e9 / HBM_BYTES_PER_S, 3)}
+
+
+def bench_chunks(enc, h0, w0, chunks, pushes, dtype, cuda=False):
+    """A lone stream pushing k frames per push, for each k of `chunks` (module docstring)."""
+    m = model(enc, dtype)
+    pool = np.random.default_rng(0).integers(0, 256, (32, h0, w0, 3), dtype=np.uint8)
+    src = torch.from_numpy(pool).cuda() if cuda else pool
+    out = {"encoder": enc, "frame": [h0, w0], "network": list(get_resize_hw(h0, w0)), "dtype": str(dtype).split(".")[-1],
+           "frames": "CUDA stacks, to_host=False" if cuda else "host stacks, host depths", "chunks": []}
+    for k in chunks:
+        st = m.stream()
+        for t in range(2):                               # past frame 0: the context slides from push 6 on for k >= 8
+            st.push(src[t], to_host=not cuda)
+        ts = []
+        for p in range(6 + pushes):
+            a = (p * k) % (32 - k + 1)
+            t0 = time.perf_counter()
+            st.push(src[a:a + k] if k > 1 else src[a], to_host=not cuda)
+            if p >= 6:
+                ts.append((time.perf_counter() - t0) * 1e3)
+        gr = st.group.causal_graphs if k > 1 else st.group.graphs
+        (bk, entry), = gr.items()
+        st.close()
+        p50 = pct(ts, 50)
+        out["chunks"].append({"k": k, "bucket": bk, "launches_per_push": entry[3], "push_ms_p50": round(p50, 3),
+                              "push_ms_p99": round(pct(ts, 99), 3), "fps": round(k * 1e3 / p50, 1)})
+    r1 = next((c for c in out["chunks"] if c["k"] == 1), None)
+    if r1:
+        for c in out["chunks"]:
+            c["vs_k1"] = round(c["fps"] / r1["fps"], 3)
+    del m
+    torch.cuda.empty_cache()
+    return out
+
+
+def bench_causal_kernel(hw, C, dtype, k=8, iters=30):
+    """The causal step kernel at one stream, k rows at t = 100.. (31 context frames each: row j reads j of them from
+    the push's own rows), and the store kernel of the same rows; L2 overwritten before every launch."""
+    from video_depth_anything_b200.windows import StreamGroupPlan, split_group_table
+    L, slots = 31, 32
+    plan = StreamGroupPlan(1, L)
+    h = plan.open()
+    plan.t[h] = 100
+    bk, table = plan.step([h], counts=[k])
+    rows, ctx, _ = split_group_table(torch.from_numpy(table).cuda(), bk, L)
+    g = torch.Generator(device="cuda").manual_seed(0)
+    qkv = torch.randn(bk * hw, 3 * C, device="cuda", generator=g).to(dtype)
+    pool = torch.randn(1, slots, hw, 2 * C, device="cuda", generator=g).to(dtype)
+    pe = torch.randn(32, 3 * C, device="cuda", generator=g)
+    out = torch.empty(bk * hw, C, dtype=dtype, device="cuda")
+    flush = torch.empty(512 << 20, dtype=torch.uint8, device="cuda")
+
+    def timed(launch):
+        launch()
+        ts = []
+        for _ in range(iters):
+            flush.zero_()
+            s, e = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+            s.record()
+            launch()
+            e.record()
+            e.synchronize()
+            ts.append(s.elapsed_time(e))
+        return pct(ts, 50)
+    ms_a = timed(lambda: ops.attention_temporal_step_causal(qkv, pool, pe, ctx, out, rows))
+    ms_s = timed(lambda: ops.stream_cache_store(qkv, pool, rows, ctx))
+    # bytes the causal kernel must move: pool rows of the context frames older than the push, q'|k'|v' of the k rows
+    # (the in-push keys are these same rows), the output
+    pool_rows = sum(L - j for j in range(k))
+    nb_a = 2 * hw * (pool_rows * 2 * C + k * (3 * C + C))
+    nb_s = 2 * hw * k * (2 * C + 2 * C)
+    res = {}
+    for name, ms, nb in (("causal", ms_a, nb_a), ("store", ms_s, nb_s)):
+        gbs = nb / (ms * 1e-3) / 1e9
+        res[name] = {"us": round(ms * 1e3, 2), "MB": round(nb / 1e6, 2), "GB_s": round(gbs, 1),
+                     "hbm_share": round(gbs * 1e9 / HBM_BYTES_PER_S, 3)}
+    return {"k": k, "hw": hw, "C": C, "head_dim": C // 8, **res}
 
 
 def bench_group(enc, h0, w0, S, warmup, pushes, dtype):
@@ -265,11 +348,28 @@ def main():
     ap.add_argument("--skip-single", action="store_true", help="only the group sweep and the batched kernel")
     ap.add_argument("--mixed", action="store_true", help="only the mixed frame size / CUDA frame arms (a)-(d)")
     ap.add_argument("--mixed-streams", default="8,16")
+    ap.add_argument("--chunks", default="", help="only the multi-frame push sweep, k frames per push, e.g. 1,2,4,8,16")
+    ap.add_argument("--chunk-pushes", type=int, default=40)
     ap.add_argument("--out", default=os.path.join(ROOT, "profiles", "stream_b200.json"))
     a = ap.parse_args()
     counts = [int(x) for x in a.streams.split(",") if x]
     if not torch.cuda.is_available():
         sys.exit("bench_stream.py needs a GPU")
+    if a.chunks:
+        ks = [int(x) for x in a.chunks.split(",")]
+        bf = torch.bfloat16
+        res = {"what": "lone stream, k consecutive frames per push (DepthStream.push of a stack), bf16", **card(),
+               "chunks": [bench_chunks("vits", 518, 518, ks, a.chunk_pushes, bf),
+                          bench_chunks("vitl", 518, 518, ks, a.chunk_pushes, bf),
+                          bench_chunks("vitl", 720, 1280, ks, a.chunk_pushes, bf),
+                          bench_chunks("vitl", 720, 1280, ks, a.chunk_pushes, bf, cuda=True)]}
+        hp = 518 // 14
+        vitl = [(hp * hp, 1024), ((hp + 1) // 2 * ((hp + 1) // 2), 1024), (hp * hp, 256), (4 * hp * hp, 256)]
+        res["causal_kernel_k8"] = [{"config": f"vitl 518x518 mm{mm}", **bench_causal_kernel(hw, C, bf)}
+                                   for mm, (hw, C) in enumerate(vitl)]
+        res["step_kernel_b8"] = [{"config": f"vitl 518x518 mm{mm}", **bench_kernel(hw, C, bf, B=8)}
+                                 for mm, (hw, C) in enumerate(vitl)]
+        return write(res, a.out)
     if a.mixed:
         res = {"what": "stream groups of mixed frame sizes, host vs CUDA frames (ViT-L bf16)", **card(),
                "mixed": [bench_mixed(int(S), a.warmup, a.group_pushes, torch.bfloat16) for S in a.mixed_streams.split(",")],

@@ -54,6 +54,8 @@ _SIGS = {
     "vda_attention_temporal_step": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int,
                                               C.c_int, C.c_int, C.c_int, C.c_void_p]),
     "vda_attention_temporal_step_batched": (C.c_int, [C.c_void_p] * 6 + [C.c_int] * 8 + [C.c_void_p]),
+    "vda_attention_temporal_step_causal": (C.c_int, [C.c_void_p] * 6 + [C.c_int] * 8 + [C.c_void_p]),
+    "vda_stream_cache_store": (C.c_int, [C.c_void_p] * 4 + [C.c_int] * 7 + [C.c_void_p]),
     "vda_preprocess_frames": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int,
                                         C.c_void_p]),
     "vda_preprocess_frames_ragged": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p]),

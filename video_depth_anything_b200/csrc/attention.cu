@@ -250,6 +250,11 @@ static int dispatch_temporal(const void* qkv, void* out, int T_, int hw, int C, 
 // kernel is HBM-bound: the cached K'|V' rows are the traffic).  Scores are reduced over the G lanes of a split with
 // xor shuffles; every split keeps an online softmax (fp32) and the splits are merged at the end (max, rescale, sum).
 // A row whose pool index is outside 0..S-1 (-1: a pad row) attends to itself only and touches no pool byte.
+//
+// CAUSAL (vda_attention_temporal_step_causal: several consecutive frames of one stream in one launch): a context entry
+// e < 0 names batch row -1 - e of the same launch, whose k'|v' are read from its q'|k'|v' block of `qkv` instead of a
+// pool slot, and the kernel writes no pool byte (vda_stream_cache_store does, after it).  Everything else is the same
+// code, so a row gives the bits the one-frame kernel gives against a pool that holds those frames.
 // ---------------------------------------------------------------------------------------------
 template <typename T>
 __device__ __forceinline__ void unpack8(const uint4& u, float (&f)[8]) {
@@ -277,7 +282,7 @@ __device__ __forceinline__ void lds_pe8(const float* p, float (&f)[8]) {
 constexpr int STEP_WARPS = 8;
 
 // (min. 2 CTAs per SM: without it ptxas caps one instantiation at 64 registers and spills)
-template <typename T, int G, int PPT>
+template <typename T, int G, int PPT, bool CAUSAL>
 __global__ void __launch_bounds__(STEP_WARPS * 32, 2)
 temporal_step_kernel(const T* __restrict__ qkv, T* __restrict__ pool, const float* __restrict__ pe,
                      const int32_t* __restrict__ rows, const int32_t* __restrict__ ctx, T* __restrict__ out, int hw,
@@ -323,7 +328,7 @@ temporal_step_kernel(const T* __restrict__ qkv, T* __restrict__ pool, const floa
       if (act && pos < hw) {
         const T* rq = cq + pos * 3 * C + col;
         uq = __ldg(reinterpret_cast<const uint4*>(rq));
-        if (ks == 0 && real) {                       // the current frame's k'|v' go to the write slot unchanged
+        if (!CAUSAL && ks == 0 && real) {            // the current frame's k'|v' go to the write slot unchanged
           T* w = cache + (static_cast<long long>(ws) * hw + pos) * row2 + col;
           *reinterpret_cast<uint4*>(w) = __ldg(reinterpret_cast<const uint4*>(rq + C));
           *reinterpret_cast<uint4*>(w + C) = __ldg(reinterpret_cast<const uint4*>(rq + 2 * C));
@@ -351,14 +356,39 @@ temporal_step_kernel(const T* __restrict__ qkv, T* __restrict__ pool, const floa
     lds_pe8(spe + j * 2 * dh + sco, pk);
     lds_pe8(spe + j * 2 * dh + dh + sco, pv);
     uint4 uk[PPT], uv[PPT];
+    if constexpr (CAUSAL) {
+      // key row base and row pitch: the current frame, an earlier row of this launch (e < 0) or a pool slot
+      const int e = cur ? 0 : __ldg(cx + 2 + j);
+      const T* kb;
+      long long kp;
+      if (cur) {
+        kb = cq + C + col, kp = 3LL * C;
+      } else if (e < 0) {
+        const int rb = min(-1 - e, static_cast<int>(gridDim.y) - 1);
+        kb = qkv + static_cast<long long>(rb) * hwl * 3 * C + C + col, kp = 3LL * C;
+      } else {
+        kb = cache + static_cast<long long>(slot) * hw * row2 + col, kp = row2;
+      }
 #pragma unroll
-    for (int i = 0; i < PPT; ++i) {
-      const long long pos = p0 + i;
-      uk[i] = uv[i] = make_uint4(0, 0, 0, 0);
-      if (act && pos < hw) {
-        const T* rk = cur ? cq + pos * 3 * C + C + col : cache + (static_cast<long long>(slot) * hw + pos) * row2 + col;
-        uk[i] = __ldg(reinterpret_cast<const uint4*>(rk));
-        uv[i] = __ldg(reinterpret_cast<const uint4*>(rk + C));
+      for (int i = 0; i < PPT; ++i) {
+        const long long pos = p0 + i;
+        uk[i] = uv[i] = make_uint4(0, 0, 0, 0);
+        if (act && pos < hw) {
+          const T* rk = kb + pos * kp;
+          uk[i] = __ldg(reinterpret_cast<const uint4*>(rk));
+          uv[i] = __ldg(reinterpret_cast<const uint4*>(rk + C));
+        }
+      }
+    } else {
+#pragma unroll
+      for (int i = 0; i < PPT; ++i) {
+        const long long pos = p0 + i;
+        uk[i] = uv[i] = make_uint4(0, 0, 0, 0);
+        if (act && pos < hw) {
+          const T* rk = cur ? cq + pos * 3 * C + C + col : cache + (static_cast<long long>(slot) * hw + pos) * row2 + col;
+          uk[i] = __ldg(reinterpret_cast<const uint4*>(rk));
+          uv[i] = __ldg(reinterpret_cast<const uint4*>(rk + C));
+        }
       }
     }
 #pragma unroll
@@ -419,29 +449,30 @@ struct StepArgs {
   const int32_t* ctx;
   void* out;
   int B, S, ctx_stride, hw, C, heads, slots;
+  bool causal;                                       // vda_attention_temporal_step_causal
 };
 
-template <typename T, int G>
+template <typename T, int G, bool CAUSAL>
 static int launch_step(const StepArgs& a, cudaStream_t st) {
   constexpr int PPT = 2;
   const int tiles = (a.hw + STEP_WARPS * PPT - 1) / (STEP_WARPS * PPT);
   const dim3 grid(static_cast<unsigned>(tiles * a.heads), static_cast<unsigned>(a.B));
   const size_t smem = static_cast<size_t>(32) * 2 * (a.C / a.heads) * sizeof(float);   // <= 32 KB (dh <= 128)
-  temporal_step_kernel<T, G, PPT><<<grid, STEP_WARPS * 32, smem, st>>>(
+  temporal_step_kernel<T, G, PPT, CAUSAL><<<grid, STEP_WARPS * 32, smem, st>>>(
       static_cast<const T*>(a.qkv), static_cast<T*>(a.pool), a.pe, a.rows, a.ctx, static_cast<T*>(a.out), a.hw, a.C,
       a.heads, a.S, a.slots, a.ctx_stride);
   VDA_CUDA(cudaGetLastError());
   return 0;
 }
 
-template <typename T>
+template <typename T, bool CAUSAL>
 static int dispatch_step(const StepArgs& a, cudaStream_t st) {
   const int chunks = a.C / a.heads / 8;
-  if (chunks <= 1) return launch_step<T, 1>(a, st);
-  if (chunks <= 2) return launch_step<T, 2>(a, st);
-  if (chunks <= 4) return launch_step<T, 4>(a, st);
-  if (chunks <= 8) return launch_step<T, 8>(a, st);
-  return launch_step<T, 16>(a, st);
+  if (chunks <= 1) return launch_step<T, 1, CAUSAL>(a, st);
+  if (chunks <= 2) return launch_step<T, 2, CAUSAL>(a, st);
+  if (chunks <= 4) return launch_step<T, 4, CAUSAL>(a, st);
+  if (chunks <= 8) return launch_step<T, 8, CAUSAL>(a, st);
+  return launch_step<T, 16, CAUSAL>(a, st);
 }
 
 static int temporal_step(const StepArgs& a, int dtype, void* stream) {
@@ -459,8 +490,36 @@ static int temporal_step(const StepArgs& a, int dtype, void* stream) {
               reinterpret_cast<uintptr_t>(a.pe) | reinterpret_cast<uintptr_t>(a.out)) & 15) == 0,
             "qkv/cache/pe/out must be 16-byte aligned");
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  if (dtype == VDA_BF16) return dispatch_step<__nv_bfloat16>(a, st);
-  return dispatch_step<__half>(a, st);
+  if (a.causal) {
+    if (dtype == VDA_BF16) return dispatch_step<__nv_bfloat16, true>(a, st);
+    return dispatch_step<__half, true>(a, st);
+  }
+  if (dtype == VDA_BF16) return dispatch_step<__nv_bfloat16, false>(a, st);
+  return dispatch_step<__half, false>(a, st);
+}
+
+// ---------------------------------------------------------------------------------------------
+// Deferred cache write of a causal step (vda_stream_cache_store): batch row b's k'|v' (columns C..3C of its q'|k'|v'
+// rows) -> pool[rows[b]], slot ctx[b][1].  A pool slot is a contiguous [hw, 2C] block, so thread i of row b moves
+// 16-byte chunk i of it; the source chunk sits at position i / (C/4), column C + 8 (i % (C/4)) of the row's block.
+// ---------------------------------------------------------------------------------------------
+__global__ void __launch_bounds__(256)
+stream_cache_store_kernel(const uint16_t* __restrict__ qkv, uint16_t* __restrict__ pool, const int32_t* __restrict__ rows,
+                          const int32_t* __restrict__ ctx, int S, int ctx_stride, int hw, int C, int slots) {
+  const int b = blockIdx.y;
+  const int r = __ldg(rows + b);
+  if (r < 0 || r >= S) return;                        // pad row
+  const int ws = min(max(__ldg(ctx + static_cast<long long>(b) * ctx_stride + 1), 0), slots - 1);
+  const int cpr = C / 4;                              // 16-byte chunks per k'|v' row
+  const long long n = static_cast<long long>(hw) * cpr;
+  const uint16_t* src = qkv + static_cast<long long>(b) * hw * 3 * C + C;
+  uint4* dst = reinterpret_cast<uint4*>(pool + (static_cast<long long>(r) * slots + ws) * hw * 2 * C);
+  for (long long i = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x; i < n;
+       i += static_cast<long long>(gridDim.x) * blockDim.x) {
+    const long long pos = i / cpr;
+    const int c = static_cast<int>(i - pos * cpr);
+    dst[i] = __ldg(reinterpret_cast<const uint4*>(src + pos * 3 * C + c * 8));
+  }
 }
 
 }  // namespace vda
@@ -472,6 +531,33 @@ extern "C" int vda_attention_temporal_step_batched(const void* qkv, void* pool, 
                                                    int C, int heads, int slots, int dtype, void* stream) {
   VDA_CHECK(rows, "temporal step: null row table");
   return temporal_step({qkv, pool, pe, rows, ctx, out, B, S, ctx_stride, hw, C, heads, slots}, dtype, stream);
+}
+
+extern "C" int vda_attention_temporal_step_causal(const void* qkv, const void* pool, const float* pe, const int32_t* rows,
+                                                  const int32_t* ctx, void* out, int B, int S, int ctx_stride, int hw,
+                                                  int C, int heads, int slots, int dtype, void* stream) {
+  VDA_CHECK(rows, "temporal step: null row table");
+  return temporal_step({qkv, const_cast<void*>(pool), pe, rows, ctx, out, B, S, ctx_stride, hw, C, heads, slots, true},
+                       dtype, stream);
+}
+
+extern "C" int vda_stream_cache_store(const void* qkv, void* pool, const int32_t* rows, const int32_t* ctx, int B, int S,
+                                      int ctx_stride, int hw, int C, int slots, int dtype, void* stream) {
+  VDA_CHECK(dtype == VDA_BF16 || dtype == VDA_FP16, "bad dtype %d", dtype);
+  VDA_CHECK(hw > 0 && C > 0 && C % 8 == 0, "cache store: need hw > 0 and C a positive multiple of 8, got hw=%d C=%d", hw, C);
+  VDA_CHECK(slots >= 2 && slots <= 32, "cache store: the cache holds 2..32 frame slots, got %d", slots);
+  VDA_CHECK(B >= 1 && B <= 65535, "cache store: 1..65535 batch rows, got %d", B);
+  VDA_CHECK(S >= 1, "cache store: the pool needs at least one entry, got %d", S);
+  VDA_CHECK(ctx_stride >= 2, "cache store: a context row holds at least {n_ctx, write slot}, got stride %d", ctx_stride);
+  VDA_CHECK(qkv && pool && rows && ctx, "cache store: null pointer");
+  VDA_CHECK(((reinterpret_cast<uintptr_t>(qkv) | reinterpret_cast<uintptr_t>(pool)) & 15) == 0,
+            "qkv/pool must be 16-byte aligned");
+  const long long chunks = static_cast<long long>(hw) * (C / 4);
+  const dim3 grid(static_cast<unsigned>((chunks + 255) / 256 < 4096 ? (chunks + 255) / 256 : 4096), static_cast<unsigned>(B));
+  stream_cache_store_kernel<<<grid, 256, 0, static_cast<cudaStream_t>(stream)>>>(
+      static_cast<const uint16_t*>(qkv), static_cast<uint16_t*>(pool), rows, ctx, S, ctx_stride, hw, C, slots);
+  VDA_CUDA(cudaGetLastError());
+  return 0;
 }
 
 extern "C" int vda_attention_temporal_step(const void* qkv, void* cache, const float* pe, const int32_t* ctx, void* out,

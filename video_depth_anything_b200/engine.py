@@ -351,8 +351,9 @@ class Engine:
 
     def _motion(self, m, x, B, T, hw, stream=None):
         """TemporalModule (motion_module.py:60-65, 102-126, 164-177).  x h16 [B*T*hw, C] rows (b, f, pos).
-        `stream` = (pool, rows, ctx): one streamed frame per batch row (T = 1) whose temporal attention reads its
-        stream's cached frames (stream_group_step)."""
+        `stream` = (pool, rows, ctx[, causal]): one streamed frame per batch row (T = 1) whose temporal attention reads its
+        stream's cached frames (stream_group_step); `causal`: context entries may name earlier rows of the batch, and the
+        rows' k'|v' go to the pool after the attention."""
         w, C = self.w, self.mm_c[m]
         M = B * T * hw
         p = f"mm{m}."
@@ -374,7 +375,11 @@ class Engine:
             else:                                          # positional encoding enters through the `pet` table
                 ops.layernorm(h, w[f"{p}a{a}.ln.w"], w[f"{p}a{a}.ln.b"], 1e-5, n)
                 ops.gemm(n, w[f"{p}a{a}.qkv.w"], qkv, bias=self._const(0.0, 3 * C))
-                ops.attention_temporal_step(qkv, stream[0][2 * m + a], w[f"{p}a{a}.pet"], stream[2], o, rows=stream[1])
+                if len(stream) > 3 and stream[3]:
+                    ops.attention_temporal_step_causal(qkv, stream[0][2 * m + a], w[f"{p}a{a}.pet"], stream[2], o, stream[1])
+                    ops.stream_cache_store(qkv, stream[0][2 * m + a], stream[1], stream[2])
+                else:
+                    ops.attention_temporal_step(qkv, stream[0][2 * m + a], w[f"{p}a{a}.pet"], stream[2], o, rows=stream[1])
             ops.gemm(o, w[f"{p}a{a}.o.w"], h, bias=w[f"{p}a{a}.o.b"], gamma=self._const(1.0, C), res1=h)   # unit LayerScale: ditto
         ops.layernorm(h, w[p + "ffn.w"], w[p + "ffn.b"], 1e-5, n)                        # :174
         g = self._hnew(M, 4 * C)
@@ -555,14 +560,17 @@ class Engine:
         return [self._hnew(S, slots, hws[m], 2 * self.mm_c[m]) for m in range(4) for _ in (0, 1)]
 
     def stream_group_step(self, frame_desc: torch.Tensor, out_desc: torch.Tensor, rows: torch.Tensor, ctx: torch.Tensor,
-                          pool: List[torch.Tensor], nh: int, nw: int) -> None:
+                          pool: List[torch.Tensor], nh: int, nw: int, causal: bool = False) -> None:
         """One streamed frame of each of B streams, every frame of its own size: batch row b reads the frame frame_desc[b]
         and writes its depth fp32 [H0,W0] (>= 0) to out_desc[b] (vda_frame_desc / vda_out_desc arrays, device bytes,
         windows.group_descriptors), takes pool entry rows[b] (int32 [B], -1: pad row) and context row ctx[b] (int32
         [B, stride], see vda_attention_temporal_step_batched).  Preprocessing to (nh, nw) as in infer_video_depth,
         encoder and head on the B frames at T = 1 with every temporal attention against the rows' pool entries, bilinear
         resize to each row's frame size.  The launches depend on neither B nor the sizes.  No host decisions:
-        graph-capturable, and every frame-dependent address is read from the descriptors at run time."""
+        graph-capturable, and every frame-dependent address is read from the descriptors at run time.
+        `causal`: rows may be consecutive frames of one stream (ctx entries < 0 name earlier rows of the batch,
+        vda_attention_temporal_step_causal); each temporal attention is then followed by the pool write of the rows'
+        k'|v' (vda_stream_cache_store): 8 more launches, nothing else differs."""
         x = ops.preprocess_frames_ragged(frame_desc, nh, nw)
-        d = self.head(self.encode(x), rows.numel(), 1, nh // 14, nw // 14, stream=(pool, rows, ctx))
+        d = self.head(self.encode(x), rows.numel(), 1, nh // 14, nw // 14, stream=(pool, rows, ctx, causal))
         ops.bilinear_f32_ragged(d, out_desc)

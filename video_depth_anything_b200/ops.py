@@ -234,6 +234,52 @@ def attention_temporal_step(qkv: torch.Tensor, cache: torch.Tensor, pe: torch.Te
     return out
 
 
+def attention_temporal_step_causal(qkv: torch.Tensor, pool: torch.Tensor, pe: torch.Tensor, ctx: torch.Tensor,
+                                   out: torch.Tensor, rows: torch.Tensor, heads: int = 8):
+    """Streaming temporal attention of several consecutive frames per stream in one launch (vda.h
+    vda_attention_temporal_step_causal): as attention_temporal_step with `rows`, but a context entry e < 0 reads batch row
+    -1 - e's k'|v' from `qkv`, and the pool is only read (stream_cache_store writes the new frames afterwards)."""
+    lib = _lib.load()
+    Cc = qkv.shape[1] // 3
+    B = rows.numel()
+    hw = qkv.shape[0] // B
+    assert qkv.is_contiguous() and pool.is_contiguous() and pe.is_contiguous() and out.is_contiguous()
+    assert pool.dim() == 4 and pool.shape[-2:] == (hw, 2 * Cc) and pool.dtype == qkv.dtype and out.dtype == qkv.dtype
+    assert qkv.shape[0] == B * hw and out.shape == (B * hw, Cc)
+    assert pe.dtype == torch.float32 and pe.shape[-1] == 3 * Cc and pe.shape[0] >= 32
+    assert rows.dtype == torch.int32 and rows.is_contiguous()
+    assert ctx.dtype == torch.int32 and ctx.is_contiguous() and ctx.dim() == 2 and ctx.shape[0] == B
+    if PROFILE is not None:
+        # no `bytes`: which context frames come from the pool and which from the push's own rows (already read as q'|k'|v')
+        # is in the device table, so the HBM traffic is not known here (tools/bench_stream.py counts it per stack size);
+        # key_row_bytes counts every k'|v' row read, wherever it comes from
+        _INFO.update(kind="attention_temporal_step_causal",
+                     key_row_bytes=float(qkv.element_size() * B * hw * 31 * 2 * Cc))
+    check(lib.vda_attention_temporal_step_causal(_p(qkv), _p(pool), _p(pe), _p(rows), _p(ctx), _p(out), B, pool.shape[0],
+                                                 ctx.shape[1], hw, Cc, heads, pool.shape[1], dt_code(qkv.dtype), _stream()))
+    _count()
+    return out
+
+
+def stream_cache_store(qkv: torch.Tensor, pool: torch.Tensor, rows: torch.Tensor, ctx: torch.Tensor):
+    """The cache write of a causal step (vda.h vda_stream_cache_store): every real row's k'|v' (qkv [B*hw, 3C], columns
+    C..3C) -> pool[rows[b]] h16 [S, slots, hw, 2C], slot ctx[b, 1]."""
+    lib = _lib.load()
+    Cc = qkv.shape[1] // 3
+    B = rows.numel()
+    hw = qkv.shape[0] // B
+    assert qkv.is_contiguous() and pool.is_contiguous() and pool.dim() == 4 and pool.dtype == qkv.dtype
+    assert qkv.shape[0] == B * hw and pool.shape[-2:] == (hw, 2 * Cc)
+    assert rows.dtype == torch.int32 and rows.is_contiguous()
+    assert ctx.dtype == torch.int32 and ctx.is_contiguous() and ctx.dim() == 2 and ctx.shape[0] == B
+    if PROFILE is not None:      # k'|v' rows read and written
+        _INFO.update(kind="stream_cache_store", bytes=float(qkv.element_size() * B * hw * 4 * Cc))
+    check(lib.vda_stream_cache_store(_p(qkv), _p(pool), _p(rows), _p(ctx), B, pool.shape[0], ctx.shape[1], hw, Cc,
+                                     pool.shape[1], dt_code(qkv.dtype), _stream()))
+    _count()
+    return pool
+
+
 def preprocess_frames(frames_u8: torch.Tensor, idx: torch.Tensor, nh: int, nw: int) -> torch.Tensor:
     """uint8 RGB [N,H0,W0,3] (device) + int32 frame indices [n] (device) -> normalised fp32 [n,3,nh,nw]
     (util/transform.py Resize(INTER_CUBIC) / NormalizeImage / PrepareForNet)."""
@@ -412,7 +458,7 @@ def _profiled(fn, name):
 
 
 for _n in ("preprocess_frames", "preprocess_frames_ragged", "copy_frames", "gemm", "layernorm", "rowstats_cast", "groupnorm", "attention_spatial", "attention_temporal",
-           "attention_temporal_step", "patch_im2col", "write_cls",
+           "attention_temporal_step", "attention_temporal_step_causal", "stream_cache_store", "patch_im2col", "write_cls",
            "pos_embed_bicubic", "im2col3x3_s2", "bilinear_nhwc", "tail_fused", "bilinear_f32", "bilinear_f32_ragged", "add_h16", "lsq_scale_shift", "align_chain",
            "affine_clamp_blend"):
     globals()[_n] = _profiled(globals()[_n], _n)

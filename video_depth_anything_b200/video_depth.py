@@ -188,17 +188,20 @@ class VideoDepthAnything(nn.Module):
             return aligner.result(), target_fps
 
     # ---- streaming -----------------------------------------------------------------------------
-    def stream(self, input_size: int = 518, fp32: bool = False) -> "DepthStream":
-        """Open a depth stream on this model's device: `push` one uint8 frame, get its depth back at once.  Each frame
-        attends to frame 0 and the 30 frames before it (DepthStream).  Streams are independent of each other and of
-        `forward` / `infer_video_depth`; `fp32=True` selects the validation-precision engine as in infer_video_depth."""
-        return DepthStream(self, self._ensure_engine(validation=bool(fp32)), input_size)
+    def stream(self, input_size: int = 518, fp32: bool = False, max_frames: int = 16) -> "DepthStream":
+        """Open a depth stream on this model's device: `push` one uint8 frame, get its depth back at once, or push a stack
+        of up to `max_frames` consecutive frames and get their depths as one step.  Each frame attends to frame 0 and the
+        30 frames before it (DepthStream).  Streams are independent of each other and of `forward` /
+        `infer_video_depth`; `fp32=True` selects the validation-precision engine as in infer_video_depth."""
+        return DepthStream(self, self._ensure_engine(validation=bool(fp32)), input_size, max_frames)
 
-    def stream_group(self, max_streams: int = 8, input_size: int = 518, fp32: bool = False) -> "DepthStreamGroup":
+    def stream_group(self, max_streams: int = 8, input_size: int = 518, fp32: bool = False,
+                     max_frames: Optional[int] = None) -> "DepthStreamGroup":
         """Open a group of up to `max_streams` depth streams (several cameras) on this model's device: each `push` takes
-        one frame of any subset of the group's open streams and runs them as one batched step (DepthStreamGroup).  Every
-        stream behaves as a DepthStream of its own; `fp32=True` selects the validation-precision engine."""
-        return DepthStreamGroup(self, self._ensure_engine(validation=bool(fp32)), max_streams, input_size)
+        one frame, or a stack of consecutive frames, of any subset of the group's open streams and runs them as one
+        batched step of at most `max_frames` frames (default max(max_streams, 16); DepthStreamGroup).  Every stream
+        behaves as a DepthStream of its own; `fp32=True` selects the validation-precision engine."""
+        return DepthStreamGroup(self, self._ensure_engine(validation=bool(fp32)), max_streams, input_size, max_frames)
 
     @torch.no_grad()
     def infer_video_depth_one(self, frame, input_size: int = 518, device="cuda", fp32: bool = False, to_host: bool = True):
@@ -208,6 +211,8 @@ class VideoDepthAnything(nn.Module):
         temporal context starts over) when `input_size`, `fp32` or the device change or new weights were loaded."""
         if torch.device(device).type != "cuda":
             raise RuntimeError("infer_video_depth_one: the B200 engine has no CPU path (device must be 'cuda')")
+        if getattr(frame, "ndim", None) != 3:
+            raise ValueError("infer_video_depth_one takes one frame uint8 [H0,W0,3]; push stacks through model.stream()")
         self.to(device)
         eng = self._ensure_engine(validation=bool(fp32))
         st = self._stream_one
@@ -242,19 +247,31 @@ class DepthStreamGroup:
 
     Device memory: the pool holds max_streams x (L + 1) = 32 frame slots per temporal-attention block, allocated at the
     first push: 903 MB per stream for ViT-L at 518x518 (214 MB for ViT-S), plus one graph's activations per bucket used
-    and the arenas."""
+    and the arenas.
 
-    def __init__(self, model: VideoDepthAnything, engine: Engine, max_streams: int = 8, input_size: int = 518):
+    Several frames per stream: a push may give a stream a stack of k consecutive frames uint8 [k, H0, W0, 3] (1 <= k <=
+    L = num_frames - 1; a CUDA stack may have any frame stride, and its rows may be pitched), for at most `max_frames`
+    frames in the push.  The stream advances by k and gets [k, H0, W0] back: the depths the k one-frame pushes would have
+    returned, in order (bit-identical with fp32=True; in the default mode the encoder's LayerNorm fold depends on the
+    bucket, as for groups).  Each frame takes a batch row of its own, and the buckets continue above max_streams up to
+    max_frames (windows.stream_buckets).  A push that gives any stream k > 1 frames replays the bucket's causal graph
+    (captured once per bucket, kept in `causal_graphs`): its temporal attention reads a frame's newer context from the
+    push's own rows and writes the cache afterwards (Engine.stream_group_step(causal=True)); any other push replays
+    today's graph."""
+
+    def __init__(self, model: VideoDepthAnything, engine: Engine, max_streams: int = 8, input_size: int = 518,
+                 max_frames: Optional[int] = None):
         self.engine, self.input_size = engine, int(input_size)
         self.device = engine.device
         self.generation = engine.generation
         L = model.num_frames - 1
         if not 1 <= L <= INFER_LEN - 1:
             raise ValueError(f"streaming needs num_frames in 2..{INFER_LEN}, got {model.num_frames}")
-        self.plan = StreamGroupPlan(int(max_streams), L, self.input_size)
-        self.max_streams = self.plan.max_streams
+        self.plan = StreamGroupPlan(int(max_streams), L, self.input_size, max_frames)
+        self.max_streams, self.max_frames = self.plan.max_streams, self.plan.max_frames
         self.pool = None
         self.graphs = {}                             # bucket -> captured step (Engine.run_graphed)
+        self.causal_graphs = {}                      # bucket -> captured causal step (pushes with stacks)
         self.arenas = {}                             # name -> buffer, grown on demand (_arena)
         self.closed = False
 
@@ -271,7 +288,7 @@ class DepthStreamGroup:
     def _alloc(self) -> None:
         eng, S, L = self.engine, self.max_streams, self.plan.L
         self.nh, self.nw = self.plan.net
-        nbytes = group_block_layout(S, L)[2].stop
+        nbytes = group_block_layout(self.plan.buckets[-1], L)[2].stop
         with torch.cuda.device(self.device):
             self.pool = eng.stream_pool(S, self.nh // 14, self.nw // 14, L + 1)
             self.meta_dev = torch.zeros(nbytes, dtype=torch.uint8, device=self.device)
@@ -286,71 +303,89 @@ class DepthStreamGroup:
             self.arenas[name] = t
         return t
 
-    def _step(self, bk: int) -> None:
+    def _step(self, bk: int, causal: bool = False) -> None:
         eng = self.engine
         fs, os_, ts = group_block_layout(bk, self.plan.L)
         rows, ctx, _ = split_group_table(self.meta_dev[ts].view(torch.int32), bk, self.plan.L)
         inputs = [self.meta_dev[fs], self.meta_dev[os_], rows, ctx]
 
         def fn(frame_desc, out_desc, rows, ctx):
-            return eng.stream_group_step(frame_desc, out_desc, rows, ctx, self.pool, self.nh, self.nw)
+            return eng.stream_group_step(frame_desc, out_desc, rows, ctx, self.pool, self.nh, self.nw, causal)
         if eng.use_graphs and ops.PROFILE is None:
-            return eng.run_graphed(self.graphs, bk, fn, inputs, adopt=True)
+            return eng.run_graphed(self.causal_graphs if causal else self.graphs, bk, fn, inputs, adopt=True)
         return fn(*inputs)
 
     def _check_frame(self, f):
+        """(k, H0, W0) of a frame (k = None) or of a stack of k frames; ValueError if it is neither."""
         if isinstance(f, torch.Tensor):
             if not f.is_cuda or f.device != self.device:
                 raise ValueError(f"a tensor frame must be a CUDA tensor on the group's device {self.device}, got {f.device}")
-            if f.dtype != torch.uint8 or f.dim() != 3 or f.shape[2] != 3:
-                raise ValueError(f"a CUDA frame must be a uint8 tensor [H0,W0,3], got {f.dtype} {tuple(f.shape)}")
-            if f.stride(2) != 1 or f.stride(1) != 3 or f.stride(0) < 3 * f.shape[1]:
+            if f.dtype != torch.uint8 or f.dim() not in (3, 4) or f.shape[-1] != 3:
+                raise ValueError(f"a CUDA frame must be a uint8 tensor [H0,W0,3] (or a stack [k,H0,W0,3]), "
+                                 f"got {f.dtype} {tuple(f.shape)}")
+            if f.stride(-1) != 1 or f.stride(-2) != 3 or f.stride(-3) < 3 * f.shape[-2]:
                 raise ValueError(f"a CUDA frame's pixels must be contiguous, stride (pitch >= 3 * W0, 3, 1), "
                                  f"got {f.stride()}")
-        elif not isinstance(f, np.ndarray) or f.ndim != 3 or f.shape[2] != 3 or f.dtype != np.uint8:
-            raise ValueError("a frame must be a uint8 numpy array [H0,W0,3] or a uint8 CUDA tensor [H0,W0,3]")
-        return int(f.shape[0]), int(f.shape[1])
+        elif not isinstance(f, np.ndarray) or f.ndim not in (3, 4) or f.shape[-1] != 3 or f.dtype != np.uint8:
+            raise ValueError("a frame must be a uint8 numpy array [H0,W0,3] or a uint8 CUDA tensor [H0,W0,3] "
+                             "(or a stack [k,H0,W0,3] of either)")
+        k = int(f.shape[0]) if f.ndim == 4 else None
+        if k is not None and not 1 <= k <= self.plan.L:
+            raise ValueError(f"a stack holds 1..{self.plan.L} frames, got {k}")
+        return k, int(f.shape[-3]), int(f.shape[-2])
 
     @torch.no_grad()
     def push(self, frames, to_host: bool = True) -> dict:
-        """frames: {handle: uint8 RGB [H0,W0,3] numpy array or CUDA tensor} (or (handle, frame) pairs) ->
-        {handle: depth [H0,W0] (>= 0)}: fresh float32 numpy arrays, or with `to_host=False` fresh float32 CUDA tensors
-        on the group's device (no device-to-host copy).  Returns after the step has finished, so the caller may reuse
-        its frame buffers at once."""
+        """frames: {handle: uint8 RGB [H0,W0,3] numpy array or CUDA tensor, or a stack [k,H0,W0,3] of k consecutive
+        frames} (or (handle, frame) pairs) -> {handle: depth [H0,W0] (>= 0), or [k,H0,W0] for a stack}: fresh float32
+        numpy arrays, or with `to_host=False` fresh float32 CUDA tensors on the group's device (no device-to-host copy).
+        Returns after the step has finished, so the caller may reuse its frame buffers at once."""
         if self.closed:
             raise RuntimeError("push on a closed DepthStreamGroup")
         if self.engine.generation != self.generation or not self.engine.loaded:
             raise RuntimeError("the model's weights changed since this stream group was opened; open a new one")
         items = list(frames.items()) if isinstance(frames, dict) else list(frames)
-        sizes = [self._check_frame(f) for _, f in items]
+        shapes = [self._check_frame(f) for _, f in items]
+        sizes = [(h0, w0) for _, h0, w0 in shapes]
+        counts = [k or 1 for k, _, _ in shapes]
         handles = [h for h, _ in items]
-        # ValueError: empty push, unknown / closed / repeated handle, a frame size the group cannot take
-        bk, table = self.plan.step(handles, sizes)
+        # ValueError: empty push, unknown / closed / repeated handle, a frame size the group cannot take, too many frames
+        bk, table = self.plan.step(handles, sizes, counts)
         if self.pool is None:
             self._alloc()
-        host = [i for i, (_, f) in enumerate(items) if isinstance(f, np.ndarray)]
-        packed = np.cumsum([0] + [3 * sizes[i][0] * sizes[i][1] for i in host]).tolist()   # host frames, packed
+        # batch rows: (item, frame of the item, H0, W0), the frames of a stack on consecutive rows
+        rows = [(i, j, h0, w0) for i, (h0, w0) in enumerate(sizes) for j in range(counts[i])]
+        host = [r for r, (i, _, _, _) in enumerate(rows) if isinstance(items[i][1], np.ndarray)]
+        packed = np.cumsum([0] + [3 * rows[r][2] * rows[r][3] for r in host]).tolist()      # host frames, packed
         in_off, in_bytes = dict(zip(host, packed)), packed[-1]
-        out_off = np.cumsum([0] + [h0 * w0 for h0, w0 in sizes]).tolist()                  # depths, packed
+        out_off = np.cumsum([0] + [h0 * w0 for _, _, h0, w0 in rows]).tolist()             # depths, packed
         out_elems = out_off[-1]
+        first = np.cumsum([0] + counts).tolist()                                           # first batch row of item i
         with torch.cuda.device(self.device):
             if host:
                 in_host = self._arena("in_host", in_bytes, torch.uint8, True)
                 in_dev = self._arena("in_dev", in_bytes, torch.uint8, False)
                 ih = in_host.numpy()
-                for i in host:
-                    h0, w0 = sizes[i]
-                    np.copyto(ih[in_off[i]:in_off[i] + 3 * h0 * w0].reshape(h0, w0, 3), items[i][1])
-            srcs = [(f.data_ptr(), f.stride(0), h0, w0) if isinstance(f, torch.Tensor) else
-                    (in_dev.data_ptr() + in_off[i], 3 * w0, h0, w0) for i, ((_, f), (h0, w0)) in enumerate(zip(items, sizes))]
+                for r in host:
+                    i, j, h0, w0 = rows[r]
+                    f = items[i][1]
+                    np.copyto(ih[in_off[r]:in_off[r] + 3 * h0 * w0].reshape(h0, w0, 3), f[j] if f.ndim == 4 else f)
+            srcs = []
+            for r, (i, j, h0, w0) in enumerate(rows):
+                f = items[i][1]
+                if isinstance(f, torch.Tensor):
+                    srcs.append((f[j].data_ptr(), f.stride(1), h0, w0) if f.dim() == 4 else (f.data_ptr(), f.stride(0), h0, w0))
+                else:
+                    srcs.append((in_dev.data_ptr() + in_off[r], 3 * w0, h0, w0))
             if to_host:
                 out_dev = self._arena("out_dev", out_elems, torch.float32, False)
                 dsts = [out_dev.data_ptr() + 4 * o for o in out_off[:-1]]
             else:
                 # the kernel writes straight into the returned tensors (one allocation each from the caching allocator):
                 # no device-to-device pass over the depths, and no arena a caller's tensor could alias
-                outs = [torch.empty(h0, w0, dtype=torch.float32, device=self.device) for h0, w0 in sizes]
-                dsts = [o.data_ptr() for o in outs]
+                outs = [torch.empty(*((k,) if k else ()), h0, w0, dtype=torch.float32, device=self.device)
+                        for k, h0, w0 in shapes]
+                dsts = [outs[i].data_ptr() + 4 * j * h0 * w0 for i, j, h0, w0 in rows]
             fd, od = group_descriptors(bk, srcs, dsts)
             fs, os_, ts = group_block_layout(bk, self.plan.L)
             mh = self.meta_host.numpy()
@@ -358,7 +393,15 @@ class DepthStreamGroup:
             if host:
                 in_dev[:in_bytes].copy_(in_host[:in_bytes], non_blocking=True)
             self.meta_dev[:ts.stop].copy_(self.meta_host[:ts.stop], non_blocking=True)
-            self._step(bk)
+            causal = max(counts) > 1
+            if causal and bk not in self.causal_graphs and self.engine.use_graphs and ops.PROFILE is None:
+                # capturing runs the step twice (warm-up, then the replay), and a causal step is not idempotent: its
+                # cache store overwrites slots its earlier rows read.  So the capture runs with every row a pad row
+                # (pool row -1: no pool byte read or written), then the push's own table replays the new graph.
+                self.meta_dev[ts.start:ts.start + 4 * bk].fill_(255)
+                self._step(bk, causal)
+                self.meta_dev[:ts.stop].copy_(self.meta_host[:ts.stop], non_blocking=True)
+            self._step(bk, causal)
             if to_host:
                 out_host = self._arena("out_host", out_elems, torch.float32, True)
                 out_host[:out_elems].copy_(out_dev[:out_elems], non_blocking=True)
@@ -366,11 +409,13 @@ class DepthStreamGroup:
         if not to_host:
             return dict(zip(handles, outs))
         oh = out_host.numpy()
-        return {h: oh[out_off[i]:out_off[i + 1]].reshape(sizes[i]).copy() for i, h in enumerate(handles)}
+        return {h: oh[out_off[first[i]]:out_off[first[i + 1]]].reshape(((k,) if k else ()) + sizes[i]).copy()
+                for i, (h, (k, _, _)) in enumerate(zip(handles, shapes))}
 
     def close(self) -> None:
         """Release the group's graphs, pool and arenas (also done when the object is collected)."""
         self.graphs = {}
+        self.causal_graphs = {}
         self.pool = None
         self.arenas = {}
         self.closed = True
@@ -398,16 +443,21 @@ class DepthStream:
     memory is bounded: L + 1 cache slots per block.  A DepthStream is a DepthStreamGroup of one stream: the whole step
     (preprocess, encoder, head, resize) is one CUDA graph; a push is one H2D of the frame (none for a CUDA frame) and of
     the context, a replay and one D2H of the depth (none with to_host=False).  Frame size (and so the network size) is
-    fixed by the first frame."""
+    fixed by the first frame.
 
-    def __init__(self, model: VideoDepthAnything, engine: Engine, input_size: int = 518):
-        self.group = DepthStreamGroup(model, engine, 1, input_size)
+    A push may also be a stack of k <= max_frames consecutive frames [k, H0, W0, 3] (k <= 31), e.g. when replaying a
+    recording or draining a backlog: one batched step of k rows, returning the [k, H0, W0] depths the k one-frame pushes
+    would have returned (DepthStreamGroup)."""
+
+    def __init__(self, model: VideoDepthAnything, engine: Engine, input_size: int = 518, max_frames: int = 16):
+        self.group = DepthStreamGroup(model, engine, 1, input_size, max_frames)
         self.engine, self.input_size, self.generation = engine, self.group.input_size, self.group.generation
         self.handle = self.group.open()
 
     def push(self, frame, to_host: bool = True):
         """frame uint8 RGB [H0,W0,3] (numpy array, or CUDA tensor on the stream's device, rows may be pitched) -> its
-        depth float32 [H0,W0] (>= 0): a fresh numpy array on every call, or with `to_host=False` a fresh CUDA tensor."""
+        depth float32 [H0,W0] (>= 0): a fresh numpy array on every call, or with `to_host=False` a fresh CUDA tensor.
+        A stack [k,H0,W0,3] of the next k frames gives their depths [k,H0,W0]."""
         return self.group.push([(self.handle, frame)], to_host)[self.handle]
 
     def close(self) -> None:

@@ -157,11 +157,18 @@ def stream_context(t: int, L: int = STREAM_CONTEXT):
 # ------------------------------------------------------------------------------------------------
 # stream groups (video_depth.DepthStreamGroup): handles, pool rows, per-stream steps, buckets and the per-push table
 # ------------------------------------------------------------------------------------------------
-def stream_buckets(max_streams: int):
-    """Batch sizes a group of at most `max_streams` streams runs at: the powers of two below it, then itself."""
+def stream_buckets(max_streams: int, max_frames=None):
+    """Batch sizes a group of at most `max_streams` streams runs at: the powers of two below it, then itself.  With
+    `max_frames` (frames per push, >= max_streams; pushes that give a stream several frames), followed by the powers of two
+    above max_streams and below max_frames, then max_frames: a push of <= max_streams single frames keeps its bucket."""
     if max_streams < 1:
         raise ValueError(f"a stream group needs max_streams >= 1, got {max_streams}")
-    return [1 << i for i in range(max_streams.bit_length()) if 1 << i < max_streams] + [max_streams]
+    out = [1 << i for i in range(max_streams.bit_length()) if 1 << i < max_streams] + [max_streams]
+    if max_frames is None or max_frames == max_streams:
+        return out
+    if max_frames < max_streams:
+        raise ValueError(f"max_frames={max_frames} is below max_streams={max_streams}")
+    return out + [1 << i for i in range(max_frames.bit_length()) if max_streams < 1 << i < max_frames] + [max_frames]
 
 
 class StreamGroupPlan:
@@ -174,11 +181,20 @@ class StreamGroupPlan:
     Frame sizes: `step(handles, sizes)` also checks the push's frame sizes [(H0, W0)] (batch-row order).  A stream's
     size is fixed by its first frame (a reopened pool row starts over with a new size); the group's network size
     get_resize_hw(H0, W0, input_size) is fixed by its first push, and every frame must map to it.  Nothing changes
-    when a push is rejected."""
+    when a push is rejected.
 
-    def __init__(self, max_streams: int, L: int = STREAM_CONTEXT, input_size: int = 518):
-        self.buckets = stream_buckets(max_streams)
-        self.max_streams, self.L = max_streams, L
+    Several frames per stream: `step(handles, sizes, counts)` gives stream handles[i] counts[i] (1..L) consecutive
+    frames t, t + 1, ... on consecutive batch rows, at most `max_frames` rows in all (default max(max_streams, 16)).  Row
+    j of a stream at step t gets stream_context(t + j): a context frame >= t, produced by this push, is entered as
+    -1 - (its batch row), an older one as its slot, and the write slot is slot(t + j).  The kernel reads the negative
+    entries from the push's own rows and the pool writes follow the attention (vda_attention_temporal_step_causal,
+    vda_stream_cache_store), so a slot the push overwrites is still read with its old frame.  Single-frame tables are
+    unchanged."""
+
+    def __init__(self, max_streams: int, L: int = STREAM_CONTEXT, input_size: int = 518, max_frames=None):
+        max_frames = max(max_streams, 16) if max_frames is None else int(max_frames)
+        self.buckets = stream_buckets(max_streams, max_frames)
+        self.max_streams, self.max_frames, self.L = max_streams, max_frames, L
         self.stride = 2 + L
         self.input_size = input_size
         self.row, self.t = {}, {}                      # handle -> pool row, handle -> frames pushed so far
@@ -227,31 +243,45 @@ class StreamGroupPlan:
                                  f"streams of other network sizes need a group of their own")
         return net
 
-    def step(self, handles, sizes=None):
-        """Table of one push of `handles` (distinct open streams, in batch-row order); advances their t.  With `sizes`,
-        the frame sizes of the push are checked and recorded too (see the class docstring)."""
+    def step(self, handles, sizes=None, counts=None):
+        """Table of one push of `handles` (distinct open streams, in batch-row order); advances their t by their frame
+        counts (`counts`, default one each).  With `sizes`, the frame sizes of the push are checked and recorded too (see
+        the class docstring)."""
         for h in handles:
             self.check(h)
         if len(set(handles)) != len(handles):
             raise ValueError("a stream is named more than once in one push")
         if not handles:
             raise ValueError("a push names at least one stream")
+        counts = [1] * len(handles) if counts is None else [int(c) for c in counts]
+        if len(counts) != len(handles):
+            raise ValueError("one frame count per stream of the push")
+        for h, c in zip(handles, counts):
+            if not 1 <= c <= self.L:
+                raise ValueError(f"stream {h!r}: {c} frames in one push; a push gives a stream 1..{self.L} frames")
+        if sum(counts) > self.max_frames:
+            raise ValueError(f"{sum(counts)} frames in one push, more than the group's max_frames={self.max_frames}")
         if sizes is not None:
             sizes = [(int(a), int(b)) for a, b in sizes]
             self.net = self._check_sizes(handles, sizes)
             for h, hw in zip(handles, sizes):
                 self.size[h] = hw
-        bk = self.bucket(len(handles))
+        bk = self.bucket(sum(counts))
         rows = np.full(bk, -1, np.int32)
         ctx = np.zeros((bk, self.stride), np.int32)
         idx = np.zeros(bk, np.int32)
-        for i, h in enumerate(handles):
-            _, slots, write = stream_context(self.t[h], self.L)
-            rows[i], idx[i] = self.row[h], i
-            ctx[i, 0], ctx[i, 1] = len(slots), write
-            ctx[i, 2:2 + len(slots)] = slots
-        for h in handles:
-            self.t[h] += 1
+        i = 0
+        for h, c in zip(handles, counts):
+            t0 = self.t[h]
+            for j in range(c):
+                ids, slots, write = stream_context(t0 + j, self.L)
+                rows[i], idx[i] = self.row[h], i
+                ctx[i, 0], ctx[i, 1] = len(slots), write
+                # frames of this push (ids >= t0) sit j' = f - t0 rows behind the stream's first row i - j
+                ctx[i, 2:2 + len(slots)] = [-1 - (i - j + f - t0) if f >= t0 else s for f, s in zip(ids, slots)]
+                i += 1
+        for h, c in zip(handles, counts):
+            self.t[h] += c
         return bk, np.concatenate([rows, ctx.ravel(), idx])
 
 
