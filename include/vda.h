@@ -333,6 +333,66 @@ int vda_forward(vda_model* m, const float* x, int B, int T, int H, int W, float*
                 int64_t workspace_bytes, void* stream);
 int vda_destroy(vda_model* m);
 
+/* ---------------------------------------------------------------------------------------------------------------
+ * Streaming for C hosts: a stream group (several live streams, e.g. cameras, each frame attending to its stream's frame 0
+ * and the frames before it) behind a host planner and one device call per push.  The same schedule and the same table
+ * encoding as the Python DepthStreamGroup (video_depth_anything_b200/video_depth.py, windows.StreamGroupPlan,
+ * engine.py Engine.stream_group_step), bit-identical output.  L = num_frames - 1 (31) context frames per stream.
+ *
+ * Planner (host only, touches no GPU):
+ *   vda_stream_plan_create   max_streams >= 1 streams open at once; max_frames frames per push (<= 0: max(max_streams, 16),
+ *                            else >= max_streams); num_frames as given to vda_create (2..32); input_size as for
+ *                            infer_video_depth (518).
+ *   vda_stream_plan_buckets  the batch sizes the group runs at: powers of two below max_streams, max_streams, then powers
+ *                            of two below max_frames, max_frames.  *n = their count; up to `capacity` are written to out.
+ *   vda_stream_plan_open     a new stream at t = 0.  Handles are never reused; its pool row is the lowest free one.
+ *   vda_stream_plan_close    frees the stream's pool row (a later open starts over on it, with a new frame size).
+ *   vda_stream_plan_step     one push of n distinct open streams in batch-row order: handles[i] gives counts[i] (1..L;
+ *                            counts NULL: 1 each) consecutive frames of size sizes[2i] x sizes[2i+1] (H0, W0; NULL: not
+ *                            checked), at most max_frames frames in all.  A stream's frame size is fixed by its first
+ *                            frame, the group's network size (vda_resize_hw) by its first push.  Writes the table of
+ *                            the push (bucket bk = the smallest bucket >= the frame count; table_capacity >= bk * (L + 4)
+ *                            int32):  rows [bk] | ctx [bk, L + 2] | idx [bk]: batch row i is a frame of stream handles[s]
+ *                            at step t with its pool row, ctx = {n_ctx, write slot, context entries...} (a context frame
+ *                            of this push is entered as -1 - its batch row, an older one as its cache slot), idx = i; pad
+ *                            rows take pool row -1, n_ctx 0.  *nh, *nw = the group's network size (0 if no push gave
+ *                            sizes yet).  Advances the streams.  A rejected push changes nothing.
+ *   vda_resize_hw            network input size of an (h0, w0) frame (video_depth.py:167-171, util/transform.py:62-107).
+ *
+ * Device step:
+ *   vda_stream_pool_bytes       bytes of the temporal cache of S streams at network size (nh, nw): 8 blocks, block
+ *                               2 * m + a (attention block a of motion module m) h16 (fp16) [S, num_frames, hw_m, 2 C_m]
+ *                               with hw = (nh / 14) (nw / 14), hw_m = {hw, ceil(nh / 28) ceil(nw / 28), hw, 4 hw}, C_m =
+ *                               {out_channels[2], out_channels[3], features, features}, one after the other (each a multiple
+ *                               of 256 bytes).  The pool is the caller's, 256-byte aligned; its content needs no
+ *                               initialisation (a stream reads only slots it wrote).  -1 on error.
+ *   vda_stream_workspace_bytes  scratch of one step of B batch rows (-1 on error).
+ *   vda_stream_step             one push: batch row b < B (= the bucket) reads frames[b] (uint8 RGB, any size) and writes
+ *                               its depth fp32 [H0, W0] >= 0 to outs[b] (pad rows: any valid frame, H0 = W0 = 0 writes
+ *                               nothing); table = the planner's table of the push.  frames, outs, table, pool and
+ *                               workspace (1024-byte aligned, >= vda_stream_workspace_bytes) are device memory.  causal != 0
+ *                               when the push gives some stream more than one frame (8 more launches: each temporal
+ *                               attention then reads the push's own rows and writes the pool afterwards); 0 otherwise.
+ *                               Enqueues on `stream`; no allocation and no synchronisation, and every per-push value is in
+ *                               the descriptors and the table, so one CUDA graph per (bucket, causal) replays every later
+ *                               push.  The first step at a new network size resamples the position embedding into
+ *                               model-owned memory: run it outside a capture.  Everything is checked before anything is
+ *                               launched; pool rows inside the table are the kernels' business (outside 0..S-1: a pad row).
+ */
+typedef struct vda_stream_plan vda_stream_plan;
+int vda_stream_plan_create(int max_streams, int max_frames, int num_frames, int input_size, vda_stream_plan** out);
+int vda_stream_plan_buckets(const vda_stream_plan* p, int32_t* out, int capacity, int* n);
+int vda_stream_plan_open(vda_stream_plan* p, int64_t* handle);
+int vda_stream_plan_close(vda_stream_plan* p, int64_t handle);
+int vda_stream_plan_step(vda_stream_plan* p, const int64_t* handles, const int32_t* sizes, const int32_t* counts, int n,
+                         int32_t* table, int64_t table_capacity, int* bucket, int* nh, int* nw);
+int vda_stream_plan_destroy(vda_stream_plan* p);
+int vda_resize_hw(int h0, int w0, int input_size, int* nh, int* nw);
+int64_t vda_stream_pool_bytes(vda_model* m, int S, int nh, int nw);
+int64_t vda_stream_workspace_bytes(vda_model* m, int B, int nh, int nw);
+int vda_stream_step(vda_model* m, const vda_frame_desc* frames, const vda_out_desc* outs, const int32_t* table, int B,
+                    int causal, void* pool, int S, int nh, int nw, void* workspace, int64_t workspace_bytes, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

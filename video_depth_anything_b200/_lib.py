@@ -85,6 +85,18 @@ _SIGS = {
     "vda_forward": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_int64,
                               C.c_void_p]),
     "vda_destroy": (C.c_int, [C.c_void_p]),
+    "vda_stream_plan_create": (C.c_int, [C.c_int, C.c_int, C.c_int, C.c_int, C.POINTER(C.c_void_p)]),
+    "vda_stream_plan_buckets": (C.c_int, [C.c_void_p, C.POINTER(C.c_int32), C.c_int, C.POINTER(C.c_int)]),
+    "vda_stream_plan_open": (C.c_int, [C.c_void_p, C.POINTER(C.c_int64)]),
+    "vda_stream_plan_close": (C.c_int, [C.c_void_p, C.c_int64]),
+    "vda_stream_plan_step": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_int64,
+                                       C.POINTER(C.c_int), C.POINTER(C.c_int), C.POINTER(C.c_int)]),
+    "vda_stream_plan_destroy": (C.c_int, [C.c_void_p]),
+    "vda_resize_hw": (C.c_int, [C.c_int, C.c_int, C.c_int, C.POINTER(C.c_int), C.POINTER(C.c_int)]),
+    "vda_stream_pool_bytes": (C.c_int64, [C.c_void_p, C.c_int, C.c_int, C.c_int]),
+    "vda_stream_workspace_bytes": (C.c_int64, [C.c_void_p, C.c_int, C.c_int, C.c_int]),
+    "vda_stream_step": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_int,
+                                  C.c_int, C.c_int, C.c_void_p, C.c_int64, C.c_void_p]),
     "vda_affine_clamp_blend": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int64,
                                          C.c_void_p]),
 }

@@ -1,6 +1,7 @@
 // Handle-level C ABI (SURVEY.md §8(b)): the whole forward of VideoDepthAnything (video_depth_anything/video_depth.py:89-164)
 // behind   vda_create -> vda_set_weight* -> vda_finalize_weights -> vda_workspace_bytes -> vda_forward   so that a host that
-// is not Python does not have to re-implement the engine's launch schedule.  This file is that schedule (the same sequence
+// is not Python does not have to re-implement the engine's launch schedule; vda_stream_step is the streaming step of a
+// stream group (engine.py Engine.stream_group_step) on the same schedule.  This file is that schedule (the same sequence
 // of libvda operator calls as video_depth_anything_b200/engine.py: encode / head / motion module / fusion blocks) plus the
 // weight packing (reference state-dict tensors -> kernel layouts), written against the operator-level entry points of
 // include/vda.h.  tests/test_cmodel_gpu.py requires its output to be BIT-identical to the Python engine's.
@@ -317,8 +318,21 @@ static void* fusion(Ctx& c, int r, const void* x0, const Map& skip, int n, int H
   return up;
 }
 
-// TemporalModule (motion_module.py:60-65, 102-126, 164-177).  x h16 [B*T*hw, C], rows (b, f, pos)
-static void* motion(Ctx& c, vda_model* mm, int mi, const void* x, int B, int T, int hw) {
+// One streamed frame per batch row (T = 1) whose temporal attentions read the rows' pool entries (engine.py
+// Engine.stream_group_step): the pool block of attention block a of motion module m starts at off[2 * m + a].
+struct StreamStep {
+  char* pool;
+  size_t off[8];
+  const int32_t* rows;   // [B]
+  const int32_t* ctx;    // [B, stride]
+  int S, slots, stride;
+  bool causal;
+};
+
+// TemporalModule (motion_module.py:60-65, 102-126, 164-177).  x h16 [B*T*hw, C], rows (b, f, pos).
+// `s`: the streaming branch of engine.py Engine._motion (LayerNorm without the positional encoding, whose share enters
+// through the `pet` tables inside the step kernels)
+static void* motion(Ctx& c, vda_model* mm, int mi, const void* x, int B, int T, int hw, const StreamStep* s) {
   const vda_model* m = c.m;
   const int C = m->mm_c[mi], M = B * T * hw, hdt = m->hdtype;
   const std::string p = "mm" + std::to_string(mi) + ".";
@@ -334,12 +348,25 @@ static void* motion(Ctx& c, vda_model* mm, int mi, const void* x, int B, int T, 
   const float* onec = const_vec(mm, 1.f, C);
   for (int a = 0; a < 2; ++a) {
     const std::string ab = p + "a" + std::to_string(a) + ".";
-    RUN(c, vda_layernorm(h, 1, nrm, c.Wf(ab + "ln.w"), c.Wf(ab + "ln.b"), 1e-5f, M, C, hdt, 0, c.Wf(ab + "pe"), hw, T, c.st));
+    RUN(c, vda_layernorm(h, 1, nrm, c.Wf(ab + "ln.w"), c.Wf(ab + "ln.b"), 1e-5f, M, C, hdt, 0, s ? nullptr : c.Wf(ab + "pe"),
+                         s ? 0 : hw, s ? 0 : T, c.st));
     { G g; g.dtype = hdt; g.bias = zero3c; gemm(c, nrm, M, C, c.W(ab + "qkv.w"), 3 * C, qkv, 3 * C, g); }
-    for (int b = 0; b < B; ++b) {
-      const size_t off = static_cast<size_t>(b) * T * hw;
-      RUN(c, vda_attention_temporal(static_cast<const char*>(qkv) + off * 3 * C * 2, static_cast<char*>(o) + off * C * 2, T, hw, C, 8,
-                                    hdt, c.st));
+    if (!s) {
+      for (int b = 0; b < B; ++b) {
+        const size_t off = static_cast<size_t>(b) * T * hw;
+        RUN(c, vda_attention_temporal(static_cast<const char*>(qkv) + off * 3 * C * 2, static_cast<char*>(o) + off * C * 2, T, hw, C,
+                                      8, hdt, c.st));
+      }
+    } else {
+      void* blk = s->pool + s->off[2 * mi + a];
+      if (s->causal) {
+        RUN(c, vda_attention_temporal_step_causal(qkv, blk, c.Wf(ab + "pet"), s->rows, s->ctx, o, B, s->S, s->stride, hw, C, 8,
+                                                  s->slots, hdt, c.st));
+        RUN(c, vda_stream_cache_store(qkv, blk, s->rows, s->ctx, B, s->S, s->stride, hw, C, s->slots, hdt, c.st));
+      } else {
+        RUN(c, vda_attention_temporal_step_batched(qkv, blk, c.Wf(ab + "pet"), s->rows, s->ctx, o, B, s->S, s->stride, hw, C, 8,
+                                                   s->slots, hdt, c.st));
+      }
     }
     { G g; g.dtype = hdt; g.bias = c.Wf(ab + "o.b"); g.gamma = onec; g.res1 = h; g.ldr1 = C; g.res1_f32 = 1; g.out_f32 = 1;
       gemm(c, o, M, C, c.W(ab + "o.w"), C, h, C, g); }
@@ -355,8 +382,8 @@ static void* motion(Ctx& c, vda_model* mm, int mi, const void* x, int B, int T, 
   return out;
 }
 
-// DPTHeadTemporal.forward (dpt_temporal.py:53-114) -> fp32 [B*T, 14hp, 14wp]
-static void head(Ctx& c, vda_model* mm, void* taps[4], int B, int T, int hp, int wp, float* depth) {
+// DPTHeadTemporal.forward (dpt_temporal.py:53-114) -> fp32 [B*T, 14hp, 14wp]; `s`: see motion
+static void head(Ctx& c, vda_model* mm, void* taps[4], int B, int T, int hp, int wp, float* depth, const StreamStep* s) {
   const vda_model* m = c.m;
   const int F = m->F, D = m->D, BT = B * T, P = hp * wp, hdt = m->hdtype;
   const int* oc = m->oc;
@@ -379,8 +406,8 @@ static void head(Ctx& c, vda_model* mm, void* taps[4], int B, int T, int hp, int
   RUN(c, vda_im2col3x3_s2(pr[3], col, BT, hp, wp, oc[3], hdt, c.st));
   void* l4 = c.a.get(static_cast<size_t>(BT) * h4 * w4 * oc[3] * 2);
   { G g; g.dtype = hdt; g.bias = c.Wf("rs3.b"); gemm(c, col, BT * h4 * w4, 9 * oc[3], c.W("rs3.w"), oc[3], l4, oc[3], g); }
-  l3 = motion(c, mm, 0, l3, B, T, P);
-  l4 = motion(c, mm, 1, l4, B, T, h4 * w4);
+  l3 = motion(c, mm, 0, l3, B, T, P, s);
+  l4 = motion(c, mm, 1, l4, B, T, h4 * w4, s);
   auto rn = [&](int i, const void* x, int H, int W, int ci) {   // layer{i}_rn (+ relu'd copy)
     Map o;
     o.p = c.a.get(static_cast<size_t>(BT) * H * W * F * 2);
@@ -392,9 +419,9 @@ static void head(Ctx& c, vda_model* mm, void* taps[4], int B, int T, int hp, int
   const Map l1r = rn(1, l1, h1, w1, m->c_l1), l2r = rn(2, l2, h2, w2, m->c_l2), l3r = rn(3, l3, hp, wp, oc[2]),
             l4r = rn(4, l4, h4, w4, oc[3]);
   void* p4 = fusion(c, 4, nullptr, l4r, BT, h4, w4, hp, wp);
-  p4 = motion(c, mm, 2, p4, B, T, P);
+  p4 = motion(c, mm, 2, p4, B, T, P, s);
   void* p3 = fusion(c, 3, p4, l3r, BT, hp, wp, h2, w2);
-  p3 = motion(c, mm, 3, p3, B, T, h2 * w2);
+  p3 = motion(c, mm, 3, p3, B, T, h2 * w2, s);
   void* p2 = fusion(c, 2, p3, l2r, BT, h2, w2, h1, w1);
   void* p1 = fusion(c, 1, p2, l1r, BT, h1, w1, 2 * h1, 2 * w1);
   const int H8 = 2 * h1, W8 = 2 * w1;
@@ -435,7 +462,58 @@ static int run_forward(vda_model* m, const float* x, int B, int T, int H, int W,
   }
   void* taps[4] = {nullptr, nullptr, nullptr, nullptr};
   encode(c, x, B * T, H, W, pos, taps);
-  head(c, m, taps, B, T, H / 14, W / 14, depth);
+  head(c, m, taps, B, T, H / 14, W / 14, depth, nullptr);
+  if (need) *need = c.a.off + 1024;
+  return c.rc;
+}
+
+// Byte offsets of the 8 blocks of a stream pool (engine.py Engine.stream_pool order: block 2 * m + a is attention block a
+// of motion module m, h16 [S, slots, hw_m, 2 C_m]); returns the total.  Every block is a multiple of 256 bytes (C_m is a
+// multiple of 64), so each starts 256-byte aligned without padding.
+static size_t pool_layout(const vda_model* m, int S, int hp, int wp, size_t off[8]) {
+  const int hws[4] = {hp * wp, ((hp - 1) / 2 + 1) * ((wp - 1) / 2 + 1), hp * wp, 4 * hp * wp};
+  size_t total = 0;
+  for (int b = 0; b < 8; ++b) {
+    off[b] = total;
+    total += static_cast<size_t>(S) * m->num_frames * hws[b / 2] * 2 * m->mm_c[b / 2] * 2;
+  }
+  return total;
+}
+
+// engine.py Engine.stream_group_step: ragged preprocessing to (nh, nw), encoder and head on the B frames at T = 1 with
+// every temporal attention against the rows' pool entries, ragged bilinear resize to each row's frame size
+static int run_step(vda_model* m, const vda_frame_desc* frames, const vda_out_desc* outs, const int32_t* table, int B, bool causal,
+                    void* pool, int S, int nh, int nw, void* ws, size_t ws_bytes, void* st, bool dry, size_t* need) {
+  Ctx c;
+  c.m = m;
+  c.a.base = static_cast<char*>(ws);
+  c.a.off = 0;
+  c.a.cap = ws_bytes;
+  c.st = st;
+  c.dry = dry;
+  c.rc = 0;
+  const int hp = nh / 14, wp = nw / 14;
+  const float* pos = nullptr;
+  if (!dry && pos_for(m, hp, wp, st, &pos)) return 1;
+  for (int mi = 0; mi < 4; ++mi) {
+    if (!const_vec(m, 0.f, 3 * m->mm_c[mi]) || !const_vec(m, 1.f, m->mm_c[mi])) return 1;
+  }
+  StreamStep s;
+  s.pool = static_cast<char*>(pool);
+  pool_layout(m, S, hp, wp, s.off);
+  s.rows = table;
+  s.ctx = table ? table + B : nullptr;
+  s.S = S;
+  s.slots = m->num_frames;
+  s.stride = m->num_frames + 1;
+  s.causal = causal;
+  float* x = static_cast<float*>(c.a.get(static_cast<size_t>(B) * 3 * nh * nw * 4));
+  RUN(c, vda_preprocess_frames_ragged(frames, B, nh, nw, x, st));
+  void* taps[4] = {nullptr, nullptr, nullptr, nullptr};
+  encode(c, x, B, nh, nw, pos, taps);
+  float* depth = static_cast<float*>(c.a.get(static_cast<size_t>(B) * nh * nw * 4));
+  head(c, m, taps, B, 1, hp, wp, depth, &s);
+  RUN(c, vda_bilinear_f32_ragged(depth, outs, B, nh, nw, st));
   if (need) *need = c.a.off + 1024;
   return c.rc;
 }
@@ -602,6 +680,20 @@ extern "C" int vda_finalize_weights(vda_model* m) {
             f32(dst + "pe", ab + "pos_encoder.pe") || f32(dst + "ln.w", blk + "norms." + std::to_string(a) + ".weight") ||
             f32(dst + "ln.b", blk + "norms." + std::to_string(a) + ".bias"))
           return 1;
+        // streaming: pet = pe[:32] [W_q | W_k | W_v]^T fp32 [32, 3C], summed in double and rounded once (engine.py load
+        // does the same, so both tables hold the same bits); the step kernels add it at a frame's current position
+        const int C = m->mm_c[mi];
+        const std::vector<float>& pe = T(ab + "pos_encoder.pe").v;
+        const int npe = static_cast<int>(pe.size() / static_cast<size_t>(C)) < 32 ? static_cast<int>(pe.size() / C) : 32;
+        std::vector<float> pet(static_cast<size_t>(32) * 3 * C, 0.f);
+        for (int r = 0; r < npe; ++r)
+          for (int n = 0; n < 3 * C; ++n) {
+            double acc = 0.0;
+            for (int k = 0; k < C; ++k)
+              acc += static_cast<double>(pe[static_cast<size_t>(r) * C + k]) * static_cast<double>(cat[static_cast<size_t>(n) * C + k]);
+            pet[static_cast<size_t>(r) * 3 * C + n] = static_cast<float>(acc);
+          }
+        if (up_f32(m, dst + "pet", pet.data(), pet.size())) return 1;
       }
       if (f32(p + "ffn.w", blk + "ff_norm.weight") || f32(p + "ffn.b", blk + "ff_norm.bias")) return 1;
       std::vector<float> wp, bp;
@@ -642,6 +734,42 @@ extern "C" int vda_forward(vda_model* m, const float* x, int B, int T, int H, in
               static_cast<long long>(workspace_bytes));
   }
   return run_forward(m, x, B, T, H, W, depth, workspace, static_cast<size_t>(workspace_bytes), stream, false, nullptr);
+}
+
+extern "C" int64_t vda_stream_pool_bytes(vda_model* m, int S, int nh, int nw) {
+  if (!m || S < 1 || nh <= 0 || nw <= 0 || nh % 14 || nw % 14) return -1;
+  size_t off[8];
+  return static_cast<int64_t>(pool_layout(m, S, nh / 14, nw / 14, off));
+}
+
+extern "C" int64_t vda_stream_workspace_bytes(vda_model* m, int B, int nh, int nw) {
+  if (!m || !m->finalized || B < 1 || nh <= 0 || nw <= 0 || nh % 14 || nw % 14) return -1;
+  size_t need = 0;
+  if (run_step(m, nullptr, nullptr, nullptr, B, false, nullptr, 1, nh, nw, nullptr, 0, nullptr, true, &need)) return -1;
+  return static_cast<int64_t>(need);
+}
+
+extern "C" int vda_stream_step(vda_model* m, const vda_frame_desc* frames, const vda_out_desc* outs, const int32_t* table, int B,
+                               int causal, void* pool, int S, int nh, int nw, void* workspace, int64_t workspace_bytes,
+                               void* stream) {
+  VDA_CHECK(m && m->finalized, "vda_stream_step: weights not finalized");
+  VDA_CHECK(frames && outs && table && pool && workspace, "vda_stream_step: null pointer");
+  VDA_CHECK(B >= 1, "vda_stream_step: bad batch B=%d", B);
+  VDA_CHECK(S >= 1, "vda_stream_step: bad pool size S=%d", S);
+  VDA_CHECK(m->num_frames >= 2 && m->num_frames <= 32, "vda_stream_step: streaming needs num_frames in 2..32, got %d",
+            m->num_frames);
+  VDA_CHECK(nh > 0 && nw > 0 && nh % 14 == 0 && nw % 14 == 0,
+            "vda_stream_step: nh (%d) and nw (%d) must be multiples of the patch size 14", nh, nw);
+  VDA_CHECK((reinterpret_cast<uintptr_t>(workspace) & 1023) == 0, "vda_stream_step: workspace must be 1024-byte aligned");
+  VDA_CHECK((reinterpret_cast<uintptr_t>(pool) & 255) == 0, "vda_stream_step: pool must be 256-byte aligned");
+  {
+    size_t need = 0;
+    if (run_step(m, nullptr, nullptr, nullptr, B, false, nullptr, S, nh, nw, nullptr, 0, nullptr, true, &need)) return 1;
+    VDA_CHECK(workspace_bytes >= 0 && static_cast<size_t>(workspace_bytes) >= need, "vda_stream_step: workspace too small: %zu bytes needed, %lld given",
+              need, static_cast<long long>(workspace_bytes));
+  }
+  return run_step(m, frames, outs, table, B, causal != 0, pool, S, nh, nw, workspace, static_cast<size_t>(workspace_bytes), stream,
+                  false, nullptr);
 }
 
 extern "C" int vda_destroy(vda_model* m) {
