@@ -209,6 +209,38 @@ typedef struct vda_frame_desc {
 } vda_frame_desc;
 int vda_preprocess_frames_ragged(const vda_frame_desc* rows, int n, int nh, int nw, float* out, void* stream);
 
+/* YUV 4:2:0 frames, as video decoders hand them over: NVDEC / GStreamer / DeepStream give NV12 (a Y plane, then one
+ * interleaved U,V plane), FFmpeg's software decoders I420 = yuv420p (a Y plane, then a U and a V plane).  Chroma planes
+ * are [H0/2, W0/2] samples; H0 and W0 must be even.  Each pixel is converted to RGB as it is fetched, then goes through
+ * the RGB path above unchanged.  The conversion is BT.601 limited range with nearest chroma -- pixel (y, x) takes chroma
+ * sample (y/2, x/2) -- in the integer form of OpenCV's cv2.cvtColor(COLOR_YUV2RGB_NV12 / COLOR_YUV2RGB_I420), which it
+ * equals on every (Y, U, V) triple:
+ *   u' = U - 128, v' = V - 128, y' = max(0, Y - 16) * 1220542, h = 1 << 19
+ *   R = clamp((y' + h + 1673527 v') >> 20, 0, 255)
+ *   G = clamp((y' + h - 852492 v' - 409993 u') >> 20, 0, 255)
+ *   B = clamp((y' + h + 2116026 u') >> 20, 0, 255)
+ * So a YUV frame gives bit-identical results to its cv2-converted RGB frame through the RGB entry points. */
+enum { VDA_PIX_NV12 = 1, VDA_PIX_I420 = 2 };
+
+/* vda_preprocess_frames for packed YUV 4:2:0 frames in OpenCV's layout: frame i is 3 * H0 * W0 / 2 bytes, the Y plane
+ * [H0, W0], then the UV plane [H0/2, W0] (NV12) or the U and V planes [H0/2, W0/2] each (I420), no padding. */
+int vda_preprocess_frames_yuv(const uint8_t* frames, const int32_t* idx, int format, float* out, int n, int H0, int W0,
+                              int nh, int nw, void* stream);
+
+/* vda_preprocess_frames_ragged for YUV 4:2:0 frames: batch row i reads rows[i] (device memory, read by the kernel).
+ * Every plane has its own address and row pitch in bytes, so decoder surfaces are read in place (an NVDEC surface puts
+ * its UV plane at Y + pitch * aligned height, not right after row H0 - 1).  NV12: plane = {Y, UV}, pitch[0] >= W0,
+ * pitch[1] >= W0, plane[2] / pitch[2] unused; I420: plane = {Y, U, V}, pitch[0] >= W0, pitch[1], pitch[2] >= W0/2.
+ * H0 and W0 even, format VDA_PIX_NV12 | VDA_PIX_I420, reserved 0.  The descriptors live in device memory and are not
+ * checked by the launcher; the host that writes them checks them (the Python mirror does: windows.group_descriptors).
+ * The per-row format leaves room for other pixel formats without an ABI change. */
+typedef struct vda_frame_planes {
+  const uint8_t* plane[3];
+  int64_t pitch[3];
+  int32_t H0, W0, format, reserved;
+} vda_frame_planes; /* 64 bytes */
+int vda_preprocess_frames_planes(const vda_frame_planes* rows, int n, int nh, int nw, float* out, void* stream);
+
 /* Encoder-feature reuse across overlapping windows (video_depth.py:197-201: 10 of a window's 32 slots repeat frames
  * of earlier windows, and the DINOv2 encoder is per-frame): copies n per-frame slabs of frame_bytes bytes, slab
  * src_idx[i] of src -> slab dst_idx[i] of dst (device int32 lists; NULL = identity).  frame_bytes % 16 == 0. */
@@ -392,6 +424,13 @@ int64_t vda_stream_pool_bytes(vda_model* m, int S, int nh, int nw);
 int64_t vda_stream_workspace_bytes(vda_model* m, int B, int nh, int nw);
 int vda_stream_step(vda_model* m, const vda_frame_desc* frames, const vda_out_desc* outs, const int32_t* table, int B,
                     int causal, void* pool, int S, int nh, int nw, void* workspace, int64_t workspace_bytes, void* stream);
+/* vda_stream_step for YUV 4:2:0 frames (NV12 / I420 decoder output, see vda_frame_planes): batch row b reads frames[b]
+ * through vda_preprocess_frames_planes instead of vda_preprocess_frames_ragged; everything else -- workspace size, pool,
+ * table, capture rule, launch count -- is vda_stream_step's, and the depths are bit-identical to vda_stream_step on the
+ * cv2-converted RGB frames.  Pad rows: any valid frame (e.g. row 0's descriptor). */
+int vda_stream_step_planes(vda_model* m, const vda_frame_planes* frames, const vda_out_desc* outs, const int32_t* table,
+                           int B, int causal, void* pool, int S, int nh, int nw, void* workspace, int64_t workspace_bytes,
+                           void* stream);
 
 #ifdef __cplusplus
 }

@@ -13,6 +13,7 @@ VDA_BF16, VDA_FP16 = 0, 1
 ACT_NONE, ACT_GELU, ACT_RELU = 0, 1, 2
 EPI_LINEAR, EPI_GEGLU, EPI_CONVT, EPI_TAIL = 0, 1, 2, 3
 A_PLAIN, A_CONV3 = 0, 1
+PIX_NV12, PIX_I420 = 1, 2                  # vda_frame_planes.format (VDA_PIX_*)
 
 
 class VdaError(RuntimeError):
@@ -59,6 +60,9 @@ _SIGS = {
     "vda_preprocess_frames": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int,
                                         C.c_void_p]),
     "vda_preprocess_frames_ragged": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p]),
+    "vda_preprocess_frames_yuv": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int,
+                                            C.c_int, C.c_void_p]),
+    "vda_preprocess_frames_planes": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p]),
     "vda_copy_frames": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int64, C.c_void_p]),
     "vda_eval_sequence": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int64, C.c_double, C.c_void_p, C.c_void_p,
                                     C.c_void_p, C.c_void_p]),
@@ -97,6 +101,8 @@ _SIGS = {
     "vda_stream_workspace_bytes": (C.c_int64, [C.c_void_p, C.c_int, C.c_int, C.c_int]),
     "vda_stream_step": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_int,
                                   C.c_int, C.c_int, C.c_void_p, C.c_int64, C.c_void_p]),
+    "vda_stream_step_planes": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_int,
+                                         C.c_int, C.c_int, C.c_void_p, C.c_int64, C.c_void_p]),
     "vda_affine_clamp_blend": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int64,
                                          C.c_void_p]),
 }

@@ -14,7 +14,8 @@ import torch
 from . import _lib
 from ._lib import check
 from .ops import dt_code
-from .windows import group_block_layout, group_descriptors
+from .video_depth import check_yuv_frame, yuv_source
+from .windows import group_block_layout, group_descriptors, pixel_format_code
 
 
 class CModel:
@@ -140,10 +141,14 @@ class CStreamGroup:
     """A stream group run through the C library alone: the C planner (CStreamPlan) and vda_stream_step, with one CUDA
     graph per (bucket, causal) captured on first use.  The push contract of DepthStreamGroup.push(..., to_host=False) for
     uint8 CUDA frames: {handle: frame [H0,W0,3] or stack [k,H0,W0,3]} (or pairs) -> {handle: fresh fp32 CUDA depth [H0,W0]
-    or [k,H0,W0]}.  Frames are read in place (rows may be pitched).  `graphs=False` runs every step eagerly."""
+    or [k,H0,W0]}.  Frames are read in place (rows may be pitched).  `graphs=False` runs every step eagerly.
+    `pixel_format` "nv12" | "i420": YUV 4:2:0 CUDA frames (packed [3*H0/2, W0] or plane tuples, the CUDA forms of
+    DepthStreamGroup.push) through vda_frame_planes descriptors and vda_stream_step_planes."""
 
     def __init__(self, model: CModel, max_streams: int = 8, input_size: int = 518, max_frames: Optional[int] = None,
-                 graphs: bool = True):
+                 graphs: bool = True, pixel_format: str = "rgb"):
+        pixel_format_code(pixel_format)
+        self.pixel_format = pixel_format
         self.model, self.lib, self.device = model, model.lib, model.device
         self.plan = CStreamPlan(max_streams, model.num_frames, input_size, max_frames)
         self.max_streams, self.L = int(max_streams), self.plan.L
@@ -163,7 +168,7 @@ class CStreamGroup:
         self.ws_bytes = self.lib.vda_stream_workspace_bytes(h, self.plan.buckets[-1], self.nh, self.nw)
         if pool_bytes < 0 or self.ws_bytes < 0:
             raise _lib.VdaError(self.lib.vda_last_error().decode(errors="replace"))
-        nbytes = group_block_layout(self.plan.buckets[-1], self.L)[2].stop
+        nbytes = group_block_layout(self.plan.buckets[-1], self.L, self.pixel_format)[2].stop
         with torch.cuda.device(self.device):
             self.pool = torch.empty(pool_bytes, dtype=torch.uint8, device=self.device)
             self._ws = torch.empty(self.ws_bytes + 1024, dtype=torch.uint8, device=self.device)
@@ -172,9 +177,10 @@ class CStreamGroup:
         self.ws = -(-self._ws.data_ptr() // 1024) * 1024          # vda_stream_step wants a 1024-byte aligned workspace
 
     def _launch(self, bk: int, causal: bool) -> None:
-        fs, os_, ts = group_block_layout(bk, self.L)
+        fs, os_, ts = group_block_layout(bk, self.L, self.pixel_format)
         m = self.meta_dev.data_ptr()
-        check(self.lib.vda_stream_step(self.model.handle, m + fs.start, m + os_.start, m + ts.start, bk, int(causal),
+        step = self.lib.vda_stream_step if self.pixel_format == "rgb" else self.lib.vda_stream_step_planes
+        check(step(self.model.handle, m + fs.start, m + os_.start, m + ts.start, bk, int(causal),
                                        self.pool.data_ptr(), self.max_streams, self.nh, self.nw, self.ws, self.ws_bytes,
                                        torch.cuda.current_stream().cuda_stream))
 
@@ -185,7 +191,7 @@ class CStreamGroup:
         if g is None:
             # a step is not idempotent (it writes the pool), so the warm-up and the capture run on pad rows (pool row -1:
             # no pool byte read or written); the push's own table is restored for the replay
-            ts = group_block_layout(bk, self.L)[2]
+            ts = group_block_layout(bk, self.L, self.pixel_format)[2]
             self.meta_dev[ts.start:ts.start + 4 * bk].fill_(255)
             self._launch(bk, causal)                  # warm-up, outside the capture: a new network size's position table
             torch.cuda.current_stream().synchronize()
@@ -197,6 +203,8 @@ class CStreamGroup:
         g.replay()
 
     def _check_frame(self, f):
+        if self.pixel_format != "rgb":
+            return check_yuv_frame(f, self.pixel_format, self.device, self.L, host=False)
         if not isinstance(f, torch.Tensor) or not f.is_cuda or f.device != self.device:
             raise ValueError(f"a frame must be a CUDA tensor on the group's device {self.device}")
         if f.dtype != torch.uint8 or f.dim() not in (3, 4) or f.shape[-1] != 3:
@@ -218,10 +226,13 @@ class CStreamGroup:
             srcs, dsts = [], []
             for (_, f), o, (k, h0, w0) in zip(items, outs, shapes):
                 for j in range(k or 1):
-                    srcs.append((f[j].data_ptr(), f.stride(1), h0, w0) if k else (f.data_ptr(), f.stride(0), h0, w0))
+                    if self.pixel_format != "rgb":
+                        srcs.append(yuv_source(f, j if k else None, h0, w0, self.pixel_format) + (h0, w0))
+                    else:
+                        srcs.append((f[j].data_ptr(), f.stride(1), h0, w0) if k else (f.data_ptr(), f.stride(0), h0, w0))
                     dsts.append(o.data_ptr() + 4 * j * h0 * w0)
-            fd, od = group_descriptors(bk, srcs, dsts)
-            fs, os_, ts = group_block_layout(bk, self.L)
+            fd, od = group_descriptors(bk, srcs, dsts, self.pixel_format)
+            fs, os_, ts = group_block_layout(bk, self.L, self.pixel_format)
             mh = self.meta_host.numpy()
             mh[fs], mh[os_], mh[ts] = fd.view(np.uint8), od.view(np.uint8), table.view(np.uint8)
             self.meta_dev[:ts.stop].copy_(self.meta_host[:ts.stop], non_blocking=True)

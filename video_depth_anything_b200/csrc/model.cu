@@ -481,9 +481,13 @@ static size_t pool_layout(const vda_model* m, int S, int hp, int wp, size_t off[
 }
 
 // engine.py Engine.stream_group_step: ragged preprocessing to (nh, nw), encoder and head on the B frames at T = 1 with
-// every temporal attention against the rows' pool entries, ragged bilinear resize to each row's frame size
-static int run_step(vda_model* m, const vda_frame_desc* frames, const vda_out_desc* outs, const int32_t* table, int B, bool causal,
-                    void* pool, int S, int nh, int nw, void* ws, size_t ws_bytes, void* st, bool dry, size_t* need) {
+// every temporal attention against the rows' pool entries, ragged bilinear resize to each row's frame size.  `ingest` is
+// the ragged preprocessing entry point of the frames' descriptor type: vda_preprocess_frames_ragged (RGB) or
+// vda_preprocess_frames_planes (YUV 4:2:0); nothing else depends on the pixel format.
+template <class Desc>
+static int run_step(vda_model* m, int (*ingest)(const Desc*, int, int, int, float*, void*), const Desc* frames,
+                    const vda_out_desc* outs, const int32_t* table, int B, bool causal, void* pool, int S, int nh, int nw,
+                    void* ws, size_t ws_bytes, void* st, bool dry, size_t* need) {
   Ctx c;
   c.m = m;
   c.a.base = static_cast<char*>(ws);
@@ -508,7 +512,7 @@ static int run_step(vda_model* m, const vda_frame_desc* frames, const vda_out_de
   s.stride = m->num_frames + 1;
   s.causal = causal;
   float* x = static_cast<float*>(c.a.get(static_cast<size_t>(B) * 3 * nh * nw * 4));
-  RUN(c, vda_preprocess_frames_ragged(frames, B, nh, nw, x, st));
+  RUN(c, ingest(frames, B, nh, nw, x, st));
   void* taps[4] = {nullptr, nullptr, nullptr, nullptr};
   encode(c, x, B, nh, nw, pos, taps);
   float* depth = static_cast<float*>(c.a.get(static_cast<size_t>(B) * nh * nw * 4));
@@ -745,31 +749,51 @@ extern "C" int64_t vda_stream_pool_bytes(vda_model* m, int S, int nh, int nw) {
 extern "C" int64_t vda_stream_workspace_bytes(vda_model* m, int B, int nh, int nw) {
   if (!m || !m->finalized || B < 1 || nh <= 0 || nw <= 0 || nh % 14 || nw % 14) return -1;
   size_t need = 0;
-  if (run_step(m, nullptr, nullptr, nullptr, B, false, nullptr, 1, nh, nw, nullptr, 0, nullptr, true, &need)) return -1;
+  if (run_step<vda_frame_desc>(m, vda_preprocess_frames_ragged, nullptr, nullptr, nullptr, B, false, nullptr, 1, nh, nw, nullptr,
+                               0, nullptr, true, &need))
+    return -1;
   return static_cast<int64_t>(need);
+}
+
+// vda_stream_step and vda_stream_step_planes: the checks, then the step with the frames' ingest
+template <class Desc>
+static int stream_step(const char* fn, vda_model* m, int (*ingest)(const Desc*, int, int, int, float*, void*),
+                       const Desc* frames, const vda_out_desc* outs, const int32_t* table, int B, int causal, void* pool, int S,
+                       int nh, int nw, void* workspace, int64_t workspace_bytes, void* stream) {
+  VDA_CHECK(m && m->finalized, "%s: weights not finalized", fn);
+  VDA_CHECK(frames && outs && table && pool && workspace, "%s: null pointer", fn);
+  VDA_CHECK(B >= 1, "%s: bad batch B=%d", fn, B);
+  VDA_CHECK(S >= 1, "%s: bad pool size S=%d", fn, S);
+  VDA_CHECK(m->num_frames >= 2 && m->num_frames <= 32, "%s: streaming needs num_frames in 2..32, got %d", fn,
+            m->num_frames);
+  VDA_CHECK(nh > 0 && nw > 0 && nh % 14 == 0 && nw % 14 == 0,
+            "%s: nh (%d) and nw (%d) must be multiples of the patch size 14", fn, nh, nw);
+  VDA_CHECK((reinterpret_cast<uintptr_t>(workspace) & 1023) == 0, "%s: workspace must be 1024-byte aligned", fn);
+  VDA_CHECK((reinterpret_cast<uintptr_t>(pool) & 255) == 0, "%s: pool must be 256-byte aligned", fn);
+  {
+    size_t need = 0;
+    if (run_step(m, ingest, static_cast<const Desc*>(nullptr), nullptr, nullptr, B, false, nullptr, S, nh, nw, nullptr, 0,
+                 nullptr, true, &need))
+      return 1;
+    VDA_CHECK(workspace_bytes >= 0 && static_cast<size_t>(workspace_bytes) >= need, "%s: workspace too small: %zu bytes needed, %lld given",
+              fn, need, static_cast<long long>(workspace_bytes));
+  }
+  return run_step(m, ingest, frames, outs, table, B, causal != 0, pool, S, nh, nw, workspace, static_cast<size_t>(workspace_bytes),
+                  stream, false, nullptr);
 }
 
 extern "C" int vda_stream_step(vda_model* m, const vda_frame_desc* frames, const vda_out_desc* outs, const int32_t* table, int B,
                                int causal, void* pool, int S, int nh, int nw, void* workspace, int64_t workspace_bytes,
                                void* stream) {
-  VDA_CHECK(m && m->finalized, "vda_stream_step: weights not finalized");
-  VDA_CHECK(frames && outs && table && pool && workspace, "vda_stream_step: null pointer");
-  VDA_CHECK(B >= 1, "vda_stream_step: bad batch B=%d", B);
-  VDA_CHECK(S >= 1, "vda_stream_step: bad pool size S=%d", S);
-  VDA_CHECK(m->num_frames >= 2 && m->num_frames <= 32, "vda_stream_step: streaming needs num_frames in 2..32, got %d",
-            m->num_frames);
-  VDA_CHECK(nh > 0 && nw > 0 && nh % 14 == 0 && nw % 14 == 0,
-            "vda_stream_step: nh (%d) and nw (%d) must be multiples of the patch size 14", nh, nw);
-  VDA_CHECK((reinterpret_cast<uintptr_t>(workspace) & 1023) == 0, "vda_stream_step: workspace must be 1024-byte aligned");
-  VDA_CHECK((reinterpret_cast<uintptr_t>(pool) & 255) == 0, "vda_stream_step: pool must be 256-byte aligned");
-  {
-    size_t need = 0;
-    if (run_step(m, nullptr, nullptr, nullptr, B, false, nullptr, S, nh, nw, nullptr, 0, nullptr, true, &need)) return 1;
-    VDA_CHECK(workspace_bytes >= 0 && static_cast<size_t>(workspace_bytes) >= need, "vda_stream_step: workspace too small: %zu bytes needed, %lld given",
-              need, static_cast<long long>(workspace_bytes));
-  }
-  return run_step(m, frames, outs, table, B, causal != 0, pool, S, nh, nw, workspace, static_cast<size_t>(workspace_bytes), stream,
-                  false, nullptr);
+  return stream_step("vda_stream_step", m, vda_preprocess_frames_ragged, frames, outs, table, B, causal, pool, S, nh, nw,
+                     workspace, workspace_bytes, stream);
+}
+
+extern "C" int vda_stream_step_planes(vda_model* m, const vda_frame_planes* frames, const vda_out_desc* outs,
+                                      const int32_t* table, int B, int causal, void* pool, int S, int nh, int nw,
+                                      void* workspace, int64_t workspace_bytes, void* stream) {
+  return stream_step("vda_stream_step_planes", m, vda_preprocess_frames_planes, frames, outs, table, B, causal, pool, S, nh,
+                     nw, workspace, workspace_bytes, stream);
 }
 
 extern "C" int vda_destroy(vda_model* m) {

@@ -560,7 +560,7 @@ class Engine:
         return [self._hnew(S, slots, hws[m], 2 * self.mm_c[m]) for m in range(4) for _ in (0, 1)]
 
     def stream_group_step(self, frame_desc: torch.Tensor, out_desc: torch.Tensor, rows: torch.Tensor, ctx: torch.Tensor,
-                          pool: List[torch.Tensor], nh: int, nw: int, causal: bool = False) -> None:
+                          pool: List[torch.Tensor], nh: int, nw: int, causal: bool = False, planes: bool = False) -> None:
         """One streamed frame of each of B streams, every frame of its own size: batch row b reads the frame frame_desc[b]
         and writes its depth fp32 [H0,W0] (>= 0) to out_desc[b] (vda_frame_desc / vda_out_desc arrays, device bytes,
         windows.group_descriptors), takes pool entry rows[b] (int32 [B], -1: pad row) and context row ctx[b] (int32
@@ -570,7 +570,9 @@ class Engine:
         graph-capturable, and every frame-dependent address is read from the descriptors at run time.
         `causal`: rows may be consecutive frames of one stream (ctx entries < 0 name earlier rows of the batch,
         vda_attention_temporal_step_causal); each temporal attention is then followed by the pool write of the rows'
-        k'|v' (vda_stream_cache_store): 8 more launches, nothing else differs."""
-        x = ops.preprocess_frames_ragged(frame_desc, nh, nw)
+        k'|v' (vda_stream_cache_store): 8 more launches, nothing else differs.
+        `planes`: frame_desc is a vda_frame_planes array (YUV 4:2:0 frames, windows.FRAME_PLANES), read by
+        vda_preprocess_frames_planes; nothing else differs."""
+        x = (ops.preprocess_frames_planes if planes else ops.preprocess_frames_ragged)(frame_desc, nh, nw)
         d = self.head(self.encode(x), rows.numel(), 1, nh // 14, nw // 14, stream=(pool, rows, ctx, causal))
         ops.bilinear_f32_ragged(d, out_desc)

@@ -14,6 +14,7 @@ from ._lib import (A_CONV3, A_PLAIN, ACT_GELU, ACT_NONE, ACT_RELU, EPI_CONVT, EP
 
 LSQ_MAX_PARTIALS = 592   # include/vda.h VDA_LSQ_MAX_PARTIALS
 FRAME_DESC_BYTES, OUT_DESC_BYTES = 24, 16   # sizeof(vda_frame_desc), sizeof(vda_out_desc)
+FRAME_PLANES_BYTES = 64                     # sizeof(vda_frame_planes)
 LAUNCHES = 0   # number of libvda kernel launches issued (bench.py reports it as gpu_launches)
 PROFILE = None  # when a list: every op appends (name, info dict, start_event, end_event)   [bench.py / tools]
 _INFO = {}
@@ -308,6 +309,34 @@ def preprocess_frames_ragged(rows: torch.Tensor, nh: int, nw: int, out: Optional
     return out
 
 
+def preprocess_frames_yuv(frames_u8: torch.Tensor, idx: torch.Tensor, fmt: int, nh: int, nw: int) -> torch.Tensor:
+    """preprocess_frames for YUV 4:2:0 frames packed in OpenCV's layout, uint8 [N, 3*H0/2, W0] (device), fmt = VDA_PIX_NV12
+    | VDA_PIX_I420: per frame what preprocess_frames gives for cv2.cvtColor(frame, COLOR_YUV2RGB_NV12 / _I420)."""
+    lib = _lib.load()
+    assert frames_u8.is_contiguous() and frames_u8.dtype == torch.uint8 and frames_u8.dim() == 3
+    assert idx.dtype == torch.int32 and idx.is_contiguous()
+    n = idx.numel()
+    h0, w0 = frames_u8.shape[1] * 2 // 3, frames_u8.shape[2]
+    out = torch.empty(n, 3, nh, nw, dtype=torch.float32, device=frames_u8.device)
+    check(lib.vda_preprocess_frames_yuv(_p(frames_u8), _p(idx), fmt, _p(out), n, h0, w0, nh, nw, _stream()))
+    _count()
+    return out
+
+
+def preprocess_frames_planes(rows: torch.Tensor, nh: int, nw: int, out: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """preprocess_frames_ragged for YUV 4:2:0 frames: rows = the vda_frame_planes array (device bytes [n * 64],
+    windows.FRAME_PLANES) -> fp32 [n,3,nh,nw], per row what preprocess_frames_ragged gives for its frame's cv2 RGB."""
+    lib = _lib.load()
+    assert rows.dtype == torch.uint8 and rows.is_contiguous() and rows.numel() % FRAME_PLANES_BYTES == 0
+    n = rows.numel() // FRAME_PLANES_BYTES
+    if out is None:
+        out = torch.empty(n, 3, nh, nw, dtype=torch.float32, device=rows.device)
+    assert out.is_contiguous() and out.dtype == torch.float32 and tuple(out.shape) == (n, 3, nh, nw)
+    check(lib.vda_preprocess_frames_planes(_p(rows), n, nh, nw, _p(out), _stream()))
+    _count()
+    return out
+
+
 def copy_frames(src: torch.Tensor, src_idx: Optional[torch.Tensor], dst: torch.Tensor, dst_idx: Optional[torch.Tensor],
                 n: int) -> torch.Tensor:
     """dst[dst_idx[i]] = src[src_idx[i]] for i < n over the leading (frame) axis; idx: device int32 or None (identity)."""
@@ -457,7 +486,7 @@ def _profiled(fn, name):
     return wrapper
 
 
-for _n in ("preprocess_frames", "preprocess_frames_ragged", "copy_frames", "gemm", "layernorm", "rowstats_cast", "groupnorm", "attention_spatial", "attention_temporal",
+for _n in ("preprocess_frames", "preprocess_frames_ragged", "preprocess_frames_yuv", "preprocess_frames_planes", "copy_frames", "gemm", "layernorm", "rowstats_cast", "groupnorm", "attention_spatial", "attention_temporal",
            "attention_temporal_step", "attention_temporal_step_causal", "stream_cache_store", "patch_im2col", "write_cls",
            "pos_embed_bicubic", "im2col3x3_s2", "bilinear_nhwc", "tail_fused", "bilinear_f32", "bilinear_f32_ragged", "add_h16", "lsq_scale_shift", "align_chain",
            "affine_clamp_blend"):

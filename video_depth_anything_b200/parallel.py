@@ -23,7 +23,7 @@ import numpy as np
 import torch
 import torch.distributed as dist
 
-from .windows import INFER_LEN, INTERP_LEN, KEYFRAMES, OVERLAP, STEP, num_windows
+from .windows import INFER_LEN, INTERP_LEN, KEYFRAMES, OVERLAP, STEP, num_windows, video_frame_shape
 
 KEYFRAME_REF = KEYFRAMES[1]           # slot 12: the frame whose aligned depth becomes the next window's reference
 
@@ -220,7 +220,7 @@ def two_phase_finalise(raws: torch.Tensor, counts: Sequence[int], K: int, n: int
 
 
 @torch.no_grad()
-def _infer_two_phase(model, frames, target_fps, input_size, device, dst, group):
+def _infer_two_phase(model, frames, target_fps, input_size, device, dst, group, pixel_format="rgb"):
     """Scalable form for ranks on one host (SURVEY.md §8e option 2).  Every rank computes its block of windows
     with no data-path collective; then
       1. the last 8 raw slots of every block travel to the next rank (cross-fade halo; NCCL batch_isend_irecv),
@@ -235,7 +235,7 @@ def _infer_two_phase(model, frames, target_fps, input_size, device, dst, group):
     from .video_depth import HostDrain
     rank, world = _world(group)
     dev = torch.device(device)
-    n, h0, w0 = frames.shape[:3]
+    n, h0, w0 = video_frame_shape(frames, pixel_format)
     K = num_windows(n)
     parts = partition_windows(K, world)
     counts = [len(p) for p in parts]
@@ -276,7 +276,7 @@ def _infer_two_phase(model, frames, target_fps, input_size, device, dst, group):
         drain = HostDrain(host, dev, touch=slice(lo, hi), copy_threads=max(2, min(6, share - 1)), touch_threads=1,
                           direct=hi > lo)
         raws = model.infer_video_depth(frames, target_fps, input_size=input_size, device=dev,
-                                       window_ids=list(parts[rank]), raw_only=True)          # [k_r,32,h0,w0]
+                                       window_ids=list(parts[rank]), raw_only=True, pixel_format=pixel_format)   # [k_r,32,h0,w0]
         stamp("windows computed")
         two_phase_finalise(raws, counts, K, n, not model.metric, _DeviceKernels(dev), drain.send, group, stamp)
         drain.finish()
@@ -305,25 +305,26 @@ _LIVE_SEGMENTS: list = []             # shared-memory segments backing arrays ha
 
 @torch.no_grad()
 def infer_video_depth_sharded(model, frames: np.ndarray, target_fps, input_size: int = 518, device=None,
-                              dst: int = 0, group=None):
+                              dst: int = 0, group=None, pixel_format: str = "rgb"):
     """Drop-in for `model.infer_video_depth(frames, target_fps, input_size, device)` under torchrun: every rank
     passes the same `frames`; rank `dst` returns `(depths float32 [N,H0,W0], target_fps)`, the others `(None,
     target_fps)`.  With one process (no process group) it is exactly `model.infer_video_depth`.  Ranks on one host
     use the two-phase form (_infer_two_phase); ranks on several hosts, which cannot share one result array, send their
-    raw window stacks to `dst` in one gather, and `dst` aligns them."""
+    raw window stacks to `dst` in one gather, and `dst` aligns them.  `pixel_format`: as for infer_video_depth (YUV 4:2:0
+    frames [N,3*H0/2,W0] from a video decoder)."""
     from .video_depth import WindowAligner
     rank, world = _world(group)
     if device is None:
         device = torch.device("cuda", torch.cuda.current_device())
     if world == 1:
-        return model.infer_video_depth(frames, target_fps, input_size=input_size, device=device)
+        return model.infer_video_depth(frames, target_fps, input_size=input_size, device=device, pixel_format=pixel_format)
     if _same_host(group):
-        return _infer_two_phase(model, frames, target_fps, input_size, device, dst, group)
-    n, h0, w0 = frames.shape[:3]
+        return _infer_two_phase(model, frames, target_fps, input_size, device, dst, group, pixel_format)
+    n, h0, w0 = video_frame_shape(frames, pixel_format)
     parts = partition_windows(num_windows(n), world)
     counts = [len(p) for p in parts]
     raw = model.infer_video_depth(frames, target_fps, input_size=input_size, device=device,
-                                  window_ids=list(parts[rank]), raw_only=True)         # [k_r,32,h0,w0] on device
+                                  window_ids=list(parts[rank]), raw_only=True, pixel_format=pixel_format)   # [k_r,32,h0,w0]
     allraw = gather_window_depths(raw, counts, dst=dst, group=group)
     if rank != dst:
         return None, target_fps

@@ -26,8 +26,9 @@ from . import ops
 from .engine import Engine
 from .synth import ENCODER_DIMS, synth_state_dict
 from .windows import (INFER_LEN, INTERP_LEN, KEYFRAMES, OVERLAP, aligner_ring_len, aligner_ring_pos, get_resize_hw,
-                      StreamGroupPlan, group_block_layout, group_descriptors, plan_feature_cache, split_group_table,
-                      upload_ring_plan, window_source_indices)
+                      StreamGroupPlan, group_block_layout, group_descriptors, pixel_format_code, plan_feature_cache,
+                      split_group_table, upload_ring_plan, video_frame_shape, window_source_indices, yuv_frame_hw,
+                      yuv_planes)
 
 
 VALIDATION_DTYPE = torch.float16     # operand type of the `fp32=True` path (see _ensure_engine)
@@ -125,7 +126,8 @@ class VideoDepthAnything(nn.Module):
     # ---- long-video driver -------------------------------------------------------------------
     @torch.no_grad()
     def infer_video_depth(self, frames: np.ndarray, target_fps, input_size=518, device="cuda", fp32=False,
-                          window_ids: Optional[Sequence[int]] = None, raw_only=False, reuse_features: bool = True):
+                          window_ids: Optional[Sequence[int]] = None, raw_only=False, reuse_features: bool = True,
+                          pixel_format: str = "rgb"):
         """frames uint8 [N,H0,W0,3] -> (float32 [N,H0,W0], target_fps)   (video_depth.py:166-254).
 
         Everything after the upload of the uint8 frames runs on the device: per-window gather + cv2-style
@@ -141,15 +143,16 @@ class VideoDepthAnything(nn.Module):
         `reuse_features`: the DINOv2 encoder is per-frame and 10 of a window's 32 slots repeat frames of earlier
         windows (:200-201), so each source frame is encoded once and its four tap features are kept on the device
         until no later window needs them (FeatureCache); every kernel is batch-invariant, so the result is
-        bit-identical to `reuse_features=False` (tests/test_forward_gpu.py)."""
+        bit-identical to `reuse_features=False` (tests/test_forward_gpu.py).
+        `pixel_format` "nv12" | "i420": frames are YUV 4:2:0 as video decoders give them, uint8 [N, 3*H0/2, W0] in
+        OpenCV's packed layout (Y rows, then the chroma rows), H0 and W0 even; uploaded at 1.5 bytes per pixel and
+        converted on the device as they are read (BT.601 limited range, nearest chroma): the result is bit-identical to
+        the call on cv2.cvtColor(frame, COLOR_YUV2RGB_NV12 / _I420) of every frame."""
         if torch.device(device).type != "cuda":
             raise RuntimeError("infer_video_depth: the B200 engine has no CPU path (device must be 'cuda')")
-        if frames.ndim != 4 or frames.shape[3] != 3 or frames.dtype != np.uint8:
-            raise ValueError("frames must be uint8 [N,H0,W0,3]")
+        n, h0, w0 = video_frame_shape(frames, pixel_format)          # ValueError: not a video of this pixel format
         self.to(device)
         eng = self._ensure_engine(validation=bool(fp32))
-        n = frames.shape[0]
-        h0, w0 = frames.shape[1:3]
         nh, nw = get_resize_hw(h0, w0, input_size)
         wins = window_source_indices(n)
         ids = list(range(len(wins))) if window_ids is None else list(window_ids)
@@ -160,7 +163,8 @@ class VideoDepthAnything(nn.Module):
             needed = sorted({i for k in ids for i in wins[k]})
             # upload ring: windows in increasing order only; not for the two-phase sharded driver (raw_only), which keeps the
             # raw stacks of all its windows on the device anyway and whose per-rank share shrinks with the rank count
-            up = FrameUploader(frames, needed, self._device, ring=not raw_only and all(a < b for a, b in zip(ids, ids[1:])))
+            up = FrameUploader(frames, needed, self._device, ring=not raw_only and all(a < b for a, b in zip(ids, ids[1:])),
+                               pixel_format=pixel_format)
             # raw stack allocated once: a fresh 34 MB block per window costs a cudaMalloc each (~10 ms at 518x518)
             raws = torch.empty(len(ids), INFER_LEN, h0, w0, dtype=torch.float32, device=self._device) if raw_only else None
             aligner = None if raw_only else WindowAligner(n, h0, w0, self._device, "identity" if self.metric else "affine")
@@ -173,7 +177,7 @@ class VideoDepthAnything(nn.Module):
                 if cache is not None:
                     d = cache.window(j)                                      # [32,nh,nw] fp32 (graph-owned buffer)
                 else:
-                    x = ops.preprocess_frames(up.dev, idx_all[j], nh, nw).unsqueeze(0)  # [1,32,3,nh,nw]   (:197-201)
+                    x = up.preprocess(idx_all[j], nh, nw).unsqueeze(0)                  # [1,32,3,nh,nw]   (:197-201)
                     up.reads_done(wins[k])
                     d = eng.forward(x)[0]                                    # [32,nh,nw] fp32   (:203-205)
                 if (nh, nw) != (h0, w0):
@@ -188,39 +192,112 @@ class VideoDepthAnything(nn.Module):
             return aligner.result(), target_fps
 
     # ---- streaming -----------------------------------------------------------------------------
-    def stream(self, input_size: int = 518, fp32: bool = False, max_frames: int = 16) -> "DepthStream":
+    def stream(self, input_size: int = 518, fp32: bool = False, max_frames: int = 16,
+               pixel_format: str = "rgb") -> "DepthStream":
         """Open a depth stream on this model's device: `push` one uint8 frame, get its depth back at once, or push a stack
         of up to `max_frames` consecutive frames and get their depths as one step.  Each frame attends to frame 0 and the
         30 frames before it (DepthStream).  Streams are independent of each other and of `forward` /
-        `infer_video_depth`; `fp32=True` selects the validation-precision engine as in infer_video_depth."""
-        return DepthStream(self, self._ensure_engine(validation=bool(fp32)), input_size, max_frames)
+        `infer_video_depth`; `fp32=True` selects the validation-precision engine as in infer_video_depth.
+        `pixel_format` "nv12" | "i420": the stream takes YUV 4:2:0 frames (DepthStreamGroup)."""
+        return DepthStream(self, self._ensure_engine(validation=bool(fp32)), input_size, max_frames, pixel_format)
 
     def stream_group(self, max_streams: int = 8, input_size: int = 518, fp32: bool = False,
-                     max_frames: Optional[int] = None) -> "DepthStreamGroup":
+                     max_frames: Optional[int] = None, pixel_format: str = "rgb") -> "DepthStreamGroup":
         """Open a group of up to `max_streams` depth streams (several cameras) on this model's device: each `push` takes
         one frame, or a stack of consecutive frames, of any subset of the group's open streams and runs them as one
         batched step of at most `max_frames` frames (default max(max_streams, 16); DepthStreamGroup).  Every stream
-        behaves as a DepthStream of its own; `fp32=True` selects the validation-precision engine."""
-        return DepthStreamGroup(self, self._ensure_engine(validation=bool(fp32)), max_streams, input_size, max_frames)
+        behaves as a DepthStream of its own; `fp32=True` selects the validation-precision engine.  `pixel_format`
+        "rgb" | "nv12" | "i420" is fixed per group, as the network size is."""
+        return DepthStreamGroup(self, self._ensure_engine(validation=bool(fp32)), max_streams, input_size, max_frames,
+                                pixel_format)
 
     @torch.no_grad()
-    def infer_video_depth_one(self, frame, input_size: int = 518, device="cuda", fp32: bool = False, to_host: bool = True):
+    def infer_video_depth_one(self, frame, input_size: int = 518, device="cuda", fp32: bool = False, to_host: bool = True,
+                              pixel_format: str = "rgb"):
         """Depth of the next frame of the model's own stream (the name of the upstream project's streaming entry
         point): frame uint8 [H0,W0,3] (numpy array or CUDA tensor) -> float32 [H0,W0] (numpy array, or with
         `to_host=False` a CUDA tensor; DepthStream.push).  The stream is opened on the first call and reopened (its
-        temporal context starts over) when `input_size`, `fp32` or the device change or new weights were loaded."""
+        temporal context starts over) when `input_size`, `fp32`, `pixel_format` or the device change or new weights were
+        loaded.  `pixel_format` "nv12" | "i420": one YUV 4:2:0 frame, packed [3*H0/2, W0] or a plane tuple
+        (DepthStreamGroup)."""
         if torch.device(device).type != "cuda":
             raise RuntimeError("infer_video_depth_one: the B200 engine has no CPU path (device must be 'cuda')")
-        if getattr(frame, "ndim", None) != 3:
+        pixel_format_code(pixel_format)
+        if pixel_format == "rgb" and getattr(frame, "ndim", None) != 3:
             raise ValueError("infer_video_depth_one takes one frame uint8 [H0,W0,3]; push stacks through model.stream()")
+        if pixel_format != "rgb" and not (getattr(frame, "ndim", None) == 2 or
+                                          isinstance(frame, (tuple, list)) and all(getattr(t, "ndim", None) == 2 for t in frame)):
+            raise ValueError(f"infer_video_depth_one takes one {pixel_format} frame, packed uint8 [3*H0/2, W0] or a tuple of "
+                             f"[rows, columns] planes; push stacks through model.stream()")
         self.to(device)
         eng = self._ensure_engine(validation=bool(fp32))
         st = self._stream_one
-        if st is None or st.engine is not eng or st.input_size != input_size or st.generation != eng.generation:
+        if st is None or st.engine is not eng or st.input_size != input_size or st.generation != eng.generation or \
+                st.pixel_format != pixel_format:
             if st is not None:
                 st.close()
-            st = self._stream_one = self.stream(input_size, fp32)
+            st = self._stream_one = self.stream(input_size, fp32, pixel_format=pixel_format)
         return st.push(frame, to_host)
+
+
+def check_yuv_frame(f, fmt: str, device, L: int, host: bool = True):
+    """(k, H0, W0) of a YUV 4:2:0 frame of format `fmt` ("nv12" | "i420") for a stream group on `device` (k = None for a
+    single frame, else a stack of 1 <= k <= L frames), ValueError if it is not one.  Forms: a packed frame [3*H0/2, W0]
+    in OpenCV's layout, a numpy array (`host`) or a CUDA tensor whose rows may be pitched (NV12 only: I420's U and V rows
+    are W0/2 bytes apart); or a tuple of CUDA plane tensors, (Y [H0,W0], UV [H0/2,W0]) for NV12, (Y, U [H0/2,W0/2], V)
+    for I420, each with its own row pitch; all with an optional leading k.  H0, W0 even.  Every check a push needs is
+    made here, before anything is planned or launched."""
+    names = "(Y, UV)" if fmt == "nv12" else "(Y, U, V)"
+
+    def check_tensor(t):
+        if t.device != device:                           # (the group's device is a CUDA device)
+            raise ValueError(f"a tensor frame must be a CUDA tensor on the group's device {device}, got {t.device}")
+        if t.dtype != torch.uint8 or t.dim() not in (2, 3):
+            raise ValueError(f"{fmt} planes are uint8 [rows, columns] (or [k, rows, columns]), got {t.dtype} {tuple(t.shape)}")
+        if t.stride(-1) != 1 or t.stride(-2) < t.shape[-1]:
+            raise ValueError(f"a plane's bytes must be contiguous within a row, stride (pitch >= columns = {t.shape[-1]}, 1), "
+                             f"got {t.stride()}")
+
+    if isinstance(f, (tuple, list)):
+        if len(f) != (2 if fmt == "nv12" else 3) or not all(isinstance(t, torch.Tensor) for t in f):
+            raise ValueError(f"an {fmt} plane tuple is {names} of CUDA tensors, got {len(f)} items")
+        for t in f:
+            check_tensor(t)
+        h0, w0 = int(f[0].shape[-2]), int(f[0].shape[-1])
+        if h0 % 2 or w0 % 2 or h0 <= 0 or w0 <= 0:
+            raise ValueError(f"an {fmt} frame has an even size, got a Y plane of {h0}x{w0}")
+        lead = tuple(f[0].shape[:-2])
+        chroma = [(h0 // 2, w0)] if fmt == "nv12" else [(h0 // 2, w0 // 2)] * 2
+        want = [lead + (h0, w0)] + [lead + c for c in chroma]
+        if [tuple(t.shape) for t in f] != want:
+            raise ValueError(f"{fmt} planes {names} must have shapes {want}, got {[tuple(t.shape) for t in f]}")
+        k = lead[0] if lead else None
+    elif isinstance(f, torch.Tensor):
+        check_tensor(f)
+        h0, w0 = yuv_frame_hw(int(f.shape[-2]), int(f.shape[-1]), fmt)
+        yuv_planes(0, f.stride(-2), h0, w0, fmt)         # ValueError: a pitched packed I420 frame
+        k = int(f.shape[0]) if f.dim() == 3 else None
+    elif host and isinstance(f, np.ndarray) and f.dtype == np.uint8 and f.ndim in (2, 3):
+        h0, w0 = yuv_frame_hw(int(f.shape[-2]), int(f.shape[-1]), fmt)
+        k = int(f.shape[0]) if f.ndim == 3 else None
+    else:
+        raise ValueError(f"an {fmt} frame is a uint8 {'numpy array or ' if host else ''}CUDA tensor [3*H0/2, W0] in OpenCV's "
+                         f"packed layout (or a stack [k, 3*H0/2, W0]), or a tuple {names} of CUDA plane tensors; got "
+                         f"{type(f).__name__} {getattr(f, 'dtype', '')} {tuple(getattr(f, 'shape', ()))}")
+    if k is not None and not 1 <= k <= L:
+        raise ValueError(f"a stack holds 1..{L} frames, got {k}")
+    return k, h0, w0
+
+
+def yuv_source(f, j: Optional[int], h0: int, w0: int, fmt: str):
+    """(plane addresses, plane pitches) -- a vda_frame_planes row without its size -- of frame j of a stack (j = None: a
+    single frame) of a CUDA YUV frame that check_yuv_frame accepted."""
+    if isinstance(f, (tuple, list)):
+        ts = [t if j is None else t[j] for t in f]
+        pad = (0,) * (3 - len(ts))
+        return tuple(t.data_ptr() for t in ts) + pad, tuple(t.stride(-2) for t in ts) + pad
+    t = f if j is None else f[j]
+    return yuv_planes(t.data_ptr(), t.stride(-2), h0, w0, fmt)
 
 
 class DepthStreamGroup:
@@ -260,7 +337,9 @@ class DepthStreamGroup:
     today's graph."""
 
     def __init__(self, model: VideoDepthAnything, engine: Engine, max_streams: int = 8, input_size: int = 518,
-                 max_frames: Optional[int] = None):
+                 max_frames: Optional[int] = None, pixel_format: str = "rgb"):
+        pixel_format_code(pixel_format)                  # ValueError for an unknown format
+        self.pixel_format = pixel_format
         self.engine, self.input_size = engine, int(input_size)
         self.device = engine.device
         self.generation = engine.generation
@@ -288,7 +367,7 @@ class DepthStreamGroup:
     def _alloc(self) -> None:
         eng, S, L = self.engine, self.max_streams, self.plan.L
         self.nh, self.nw = self.plan.net
-        nbytes = group_block_layout(self.plan.buckets[-1], L)[2].stop
+        nbytes = group_block_layout(self.plan.buckets[-1], L, self.pixel_format)[2].stop
         with torch.cuda.device(self.device):
             self.pool = eng.stream_pool(S, self.nh // 14, self.nw // 14, L + 1)
             self.meta_dev = torch.zeros(nbytes, dtype=torch.uint8, device=self.device)
@@ -305,18 +384,21 @@ class DepthStreamGroup:
 
     def _step(self, bk: int, causal: bool = False) -> None:
         eng = self.engine
-        fs, os_, ts = group_block_layout(bk, self.plan.L)
+        fs, os_, ts = group_block_layout(bk, self.plan.L, self.pixel_format)
         rows, ctx, _ = split_group_table(self.meta_dev[ts].view(torch.int32), bk, self.plan.L)
         inputs = [self.meta_dev[fs], self.meta_dev[os_], rows, ctx]
+        planes = self.pixel_format != "rgb"
 
         def fn(frame_desc, out_desc, rows, ctx):
-            return eng.stream_group_step(frame_desc, out_desc, rows, ctx, self.pool, self.nh, self.nw, causal)
+            return eng.stream_group_step(frame_desc, out_desc, rows, ctx, self.pool, self.nh, self.nw, causal, planes)
         if eng.use_graphs and ops.PROFILE is None:
             return eng.run_graphed(self.causal_graphs if causal else self.graphs, bk, fn, inputs, adopt=True)
         return fn(*inputs)
 
     def _check_frame(self, f):
         """(k, H0, W0) of a frame (k = None) or of a stack of k frames; ValueError if it is neither."""
+        if self.pixel_format != "rgb":
+            return check_yuv_frame(f, self.pixel_format, self.device, self.plan.L)
         if isinstance(f, torch.Tensor):
             if not f.is_cuda or f.device != self.device:
                 raise ValueError(f"a tensor frame must be a CUDA tensor on the group's device {self.device}, got {f.device}")
@@ -356,7 +438,9 @@ class DepthStreamGroup:
         # batch rows: (item, frame of the item, H0, W0), the frames of a stack on consecutive rows
         rows = [(i, j, h0, w0) for i, (h0, w0) in enumerate(sizes) for j in range(counts[i])]
         host = [r for r, (i, _, _, _) in enumerate(rows) if isinstance(items[i][1], np.ndarray)]
-        packed = np.cumsum([0] + [3 * rows[r][2] * rows[r][3] for r in host]).tolist()      # host frames, packed
+        yuv = self.pixel_format != "rgb"
+        px3 = 3 if not yuv else 1.5                                                          # bytes per pixel
+        packed = np.cumsum([0] + [int(px3 * rows[r][2] * rows[r][3]) for r in host]).tolist()   # host frames, packed
         in_off, in_bytes = dict(zip(host, packed)), packed[-1]
         out_off = np.cumsum([0] + [h0 * w0 for _, _, h0, w0 in rows]).tolist()             # depths, packed
         out_elems = out_off[-1]
@@ -369,11 +453,20 @@ class DepthStreamGroup:
                 for r in host:
                     i, j, h0, w0 = rows[r]
                     f = items[i][1]
-                    np.copyto(ih[in_off[r]:in_off[r] + 3 * h0 * w0].reshape(h0, w0, 3), f[j] if f.ndim == 4 else f)
+                    if yuv:
+                        np.copyto(ih[in_off[r]:in_off[r] + 3 * h0 * w0 // 2].reshape(3 * h0 // 2, w0), f[j] if f.ndim == 3 else f)
+                    else:
+                        np.copyto(ih[in_off[r]:in_off[r] + 3 * h0 * w0].reshape(h0, w0, 3), f[j] if f.ndim == 4 else f)
             srcs = []
             for r, (i, j, h0, w0) in enumerate(rows):
                 f = items[i][1]
-                if isinstance(f, torch.Tensor):
+                if yuv:
+                    if isinstance(f, np.ndarray):
+                        src = yuv_planes(in_dev.data_ptr() + in_off[r], w0, h0, w0, self.pixel_format)
+                    else:
+                        src = yuv_source(f, j if shapes[i][0] is not None else None, h0, w0, self.pixel_format)
+                    srcs.append(src + (h0, w0))
+                elif isinstance(f, torch.Tensor):
                     srcs.append((f[j].data_ptr(), f.stride(1), h0, w0) if f.dim() == 4 else (f.data_ptr(), f.stride(0), h0, w0))
                 else:
                     srcs.append((in_dev.data_ptr() + in_off[r], 3 * w0, h0, w0))
@@ -386,8 +479,8 @@ class DepthStreamGroup:
                 outs = [torch.empty(*((k,) if k else ()), h0, w0, dtype=torch.float32, device=self.device)
                         for k, h0, w0 in shapes]
                 dsts = [outs[i].data_ptr() + 4 * j * h0 * w0 for i, j, h0, w0 in rows]
-            fd, od = group_descriptors(bk, srcs, dsts)
-            fs, os_, ts = group_block_layout(bk, self.plan.L)
+            fd, od = group_descriptors(bk, srcs, dsts, self.pixel_format)
+            fs, os_, ts = group_block_layout(bk, self.plan.L, self.pixel_format)
             mh = self.meta_host.numpy()
             mh[fs], mh[os_], mh[ts] = fd.view(np.uint8), od.view(np.uint8), table.view(np.uint8)
             if host:
@@ -449,15 +542,18 @@ class DepthStream:
     recording or draining a backlog: one batched step of k rows, returning the [k, H0, W0] depths the k one-frame pushes
     would have returned (DepthStreamGroup)."""
 
-    def __init__(self, model: VideoDepthAnything, engine: Engine, input_size: int = 518, max_frames: int = 16):
-        self.group = DepthStreamGroup(model, engine, 1, input_size, max_frames)
+    def __init__(self, model: VideoDepthAnything, engine: Engine, input_size: int = 518, max_frames: int = 16,
+                 pixel_format: str = "rgb"):
+        self.group = DepthStreamGroup(model, engine, 1, input_size, max_frames, pixel_format)
         self.engine, self.input_size, self.generation = engine, self.group.input_size, self.group.generation
+        self.pixel_format = pixel_format
         self.handle = self.group.open()
 
     def push(self, frame, to_host: bool = True):
         """frame uint8 RGB [H0,W0,3] (numpy array, or CUDA tensor on the stream's device, rows may be pitched) -> its
         depth float32 [H0,W0] (>= 0): a fresh numpy array on every call, or with `to_host=False` a fresh CUDA tensor.
-        A stack [k,H0,W0,3] of the next k frames gives their depths [k,H0,W0]."""
+        A stack [k,H0,W0,3] of the next k frames gives their depths [k,H0,W0].  A stream opened with a YUV
+        `pixel_format` takes the frame forms of DepthStreamGroup.push for that format."""
         return self.group.push([(self.handle, frame)], to_host)[self.handle]
 
     def close(self) -> None:
@@ -499,7 +595,7 @@ class FeatureCache:
         eng, P, n = self.eng, self.hp * self.wp, self.n_new[j]
         row = self.table[j]
         if n:
-            x = ops.preprocess_frames(self.up.dev, row[:n], self.nh, self.nw)          # [n,3,nh,nw]   (:197-198)
+            x = self.up.preprocess(row[:n], self.nh, self.nw)                           # [n,3,nh,nw]   (:197-198)
             self.up.reads_done(self.missing[j])
             taps = eng.encode_frames(x)
             for i in range(4):
@@ -552,14 +648,17 @@ class FrameUploader:
     CHUNK = 64
     RING_CHUNKS = 4
 
-    def __init__(self, frames: np.ndarray, needed: List[int], device, ring: bool = True):
+    def __init__(self, frames: np.ndarray, needed: List[int], device, ring: bool = True, pixel_format: str = "rgb"):
+        """frames: uint8 [N,H0,W0,3] (RGB) or [N,3*H0/2,W0] (pixel_format "nv12" / "i420", OpenCV's packed layout): the
+        device slots hold each frame as it comes, 1.5 bytes per pixel for YUV."""
         self.frames, self.needed, self.device = frames, needed, device
+        self.fmt = pixel_format_code(pixel_format)
         self.pos = {i: j for j, i in enumerate(needed)}            # position in upload order
         self.ring, n_slots, slots, self.chunks = upload_ring_plan(len(needed), self.CHUNK, self.RING_CHUNKS if ring else 1 << 30)
         self.slot = {i: slots[j] for i, j in self.pos.items()}     # device slot of every needed source frame
-        h0, w0 = frames.shape[1:3]
-        self.dev = torch.empty(n_slots, h0, w0, 3, dtype=torch.uint8, device=device)
-        self.stage, self._stage_token = _pinned_acquire(("upload", h0, w0), 2, (self.CHUNK, h0, w0, 3), torch.uint8)
+        shape = tuple(frames.shape[1:])
+        self.dev = torch.empty(n_slots, *shape, dtype=torch.uint8, device=device)
+        self.stage, self._stage_token = _pinned_acquire(("upload",) + shape, 2, (self.CHUNK,) + shape, torch.uint8)
         self.stage_free = [None, None]           # event: staging buffer consumed by its H2D copy
         self.read_ev = [None] * (self.RING_CHUNKS if self.ring else 0)   # event: the kernels that read the chunk in this ring region are queued
         self.stream = torch.cuda.Stream(device=device)
@@ -570,6 +669,13 @@ class FrameUploader:
         self.dev.record_stream(self.stream)
         self.uploaded = 0                        # number of `needed` entries issued so far
         self.chunk_no = 0
+
+    def preprocess(self, idx: torch.Tensor, nh: int, nw: int) -> torch.Tensor:
+        """Normalised fp32 [n,3,nh,nw] of the uploaded frames in device slots idx (int32, device): the ingest kernel of
+        the frames' pixel format."""
+        if self.fmt == 0:
+            return ops.preprocess_frames(self.dev, idx, nh, nw)
+        return ops.preprocess_frames_yuv(self.dev, idx, self.fmt, nh, nw)
 
     def _region(self, p: int) -> int:
         """Ring region of upload position p >= 1."""

@@ -294,27 +294,90 @@ def split_group_table(table, bk: int, L: int = STREAM_CONTEXT):
 # include/vda.h vda_frame_desc / vda_out_desc: what the ragged ingest and egress kernels read per batch row
 FRAME_DESC = np.dtype([("src", "<u8"), ("pitch", "<i8"), ("H0", "<i4"), ("W0", "<i4")])
 OUT_DESC = np.dtype([("dst", "<u8"), ("H0", "<i4"), ("W0", "<i4")])
+# include/vda.h vda_frame_planes: the ragged ingest's descriptor of a YUV 4:2:0 frame (64 bytes)
+FRAME_PLANES = np.dtype([("plane", "<u8", (3,)), ("pitch", "<i8", (3,)), ("H0", "<i4"), ("W0", "<i4"), ("format", "<i4"),
+                         ("reserved", "<i4")])
+
+# pixel formats of the ingest: packed uint8 RGB, and the YUV 4:2:0 layouts of video decoders (VDA_PIX_*)
+PIXEL_FORMATS = {"rgb": 0, "nv12": 1, "i420": 2}
 
 
-def group_descriptors(bk: int, frames, dsts):
+def pixel_format_code(pixel_format: str) -> int:
+    """VDA_PIX_* code of a pixel format name ("rgb" -> 0); ValueError for anything else."""
+    if pixel_format not in PIXEL_FORMATS:
+        raise ValueError(f"pixel_format must be one of {sorted(PIXEL_FORMATS)}, got {pixel_format!r}")
+    return PIXEL_FORMATS[pixel_format]
+
+
+def yuv_frame_hw(rows: int, cols: int, pixel_format: str):
+    """(H0, W0) of a YUV 4:2:0 frame packed in OpenCV's layout [3 * H0 / 2, W0] (Y rows, then the chroma rows); ValueError
+    unless H0 and W0 are positive and even."""
+    if rows % 3 or rows <= 0 or cols <= 0 or cols % 2:
+        raise ValueError(f"a packed {pixel_format} frame is uint8 [3*H0/2, W0] with H0, W0 even and positive, "
+                         f"got {rows} x {cols} rows x columns")
+    return 2 * rows // 3, cols
+
+
+def yuv_planes(base: int, pitch: int, h0: int, w0: int, pixel_format: str):
+    """(plane addresses, plane pitches) of a packed YUV 4:2:0 frame at `base` in OpenCV's layout: the chroma follows the
+    H0 luma rows; NV12: one interleaved UV plane of the luma pitch; I420 (pitch == W0): U then V, W0 / 2 bytes per row."""
+    uv = base + h0 * pitch
+    if pixel_format == "nv12":
+        return (base, uv, 0), (pitch, pitch, 0)
+    if pitch != w0:
+        raise ValueError(f"a packed i420 frame's rows must be contiguous (pitch == W0 = {w0}, its U and V rows are W0/2 "
+                         f"bytes apart), got pitch {pitch}: pass a pitched frame as a (Y, U, V) plane tuple")
+    return (base, uv, uv + h0 * w0 // 4), (w0, w0 // 2, w0 // 2)
+
+
+def video_frame_shape(frames: np.ndarray, pixel_format: str = "rgb"):
+    """(N, H0, W0) of a video for infer_video_depth: uint8 [N,H0,W0,3] (RGB) or [N,3*H0/2,W0] (NV12 / I420 in OpenCV's
+    packed layout, H0 and W0 even); ValueError if it is not one."""
+    if pixel_format_code(pixel_format) == 0:
+        if frames.ndim != 4 or frames.shape[3] != 3 or frames.dtype != np.uint8:
+            raise ValueError("frames must be uint8 [N,H0,W0,3]")
+        return tuple(int(x) for x in frames.shape[:3])
+    if frames.ndim != 3 or frames.dtype != np.uint8:
+        raise ValueError(f"{pixel_format} frames must be uint8 [N,3*H0/2,W0] (OpenCV's packed layout)")
+    return (int(frames.shape[0]),) + yuv_frame_hw(int(frames.shape[1]), int(frames.shape[2]), pixel_format)
+
+
+def frame_desc_dtype(pixel_format: str = "rgb") -> np.dtype:
+    """The per-row descriptor the ragged ingest of a pixel format reads: FRAME_DESC (RGB) or FRAME_PLANES (YUV)."""
+    return FRAME_DESC if pixel_format_code(pixel_format) == 0 else FRAME_PLANES
+
+
+def group_descriptors(bk: int, frames, dsts, pixel_format: str = "rgb"):
     """Descriptor arrays of one push: frames = [(device address, row pitch in bytes, H0, W0)] and dsts = [device address
     of the fp32 [H0, W0] output] of the real rows in batch-row order -> (FRAME_DESC [bk], OUT_DESC [bk]).  Pad rows read
-    the first row's frame (any valid frame would do) and write nothing (H0 = W0 = 0)."""
+    the first row's frame (any valid frame would do) and write nothing (H0 = W0 = 0).
+    YUV formats ("nv12" / "i420"): frames = [((address of each plane), (pitch of each plane), H0, W0)] (NV12: Y, UV and
+    an unused third entry; I420: Y, U, V) -> (FRAME_PLANES [bk], OUT_DESC [bk]); ValueError for an odd size or a pitch
+    shorter than its plane's row."""
+    fmt = pixel_format_code(pixel_format)
     if not 1 <= len(frames) <= bk or len(dsts) != len(frames):
         raise ValueError(f"{len(frames)} frames / {len(dsts)} outputs for a bucket of {bk}")
-    fd, od = np.zeros(bk, FRAME_DESC), np.zeros(bk, OUT_DESC)
+    fd, od = np.zeros(bk, frame_desc_dtype(pixel_format)), np.zeros(bk, OUT_DESC)
     for i, ((src, pitch, h0, w0), dst) in enumerate(zip(frames, dsts)):
-        if pitch < 3 * w0:
-            raise ValueError(f"row pitch {pitch} < 3 * W0 = {3 * w0}")
-        fd[i] = (src, pitch, h0, w0)
+        if fmt == 0:
+            if pitch < 3 * w0:
+                raise ValueError(f"row pitch {pitch} < 3 * W0 = {3 * w0}")
+            fd[i] = (src, pitch, h0, w0)
+        else:
+            if h0 % 2 or w0 % 2 or h0 <= 0 or w0 <= 0:
+                raise ValueError(f"a {pixel_format} frame has an even size, got {h0}x{w0}")
+            need = (w0, w0, 0) if pixel_format == "nv12" else (w0, w0 // 2, w0 // 2)
+            if len(src) != 3 or len(pitch) != 3 or any(p < q for p, q in zip(pitch, need)):
+                raise ValueError(f"{pixel_format} plane pitches {tuple(pitch)} shorter than the planes' rows {need}")
+            fd[i] = (src, pitch, h0, w0, fmt, 0)
         od[i] = (dst, h0, w0)
     fd[len(frames):] = fd[0]
     return fd, od
 
 
-def group_block_layout(bk: int, L: int = STREAM_CONTEXT):
+def group_block_layout(bk: int, L: int = STREAM_CONTEXT, pixel_format: str = "rgb"):
     """Byte ranges (frame descriptors, output descriptors, int32 table) of a push's metadata block: everything a push
     uploads besides frame pixels, in one copy.  The descriptors come first, so every part is aligned to its type."""
-    a = bk * FRAME_DESC.itemsize
+    a = bk * frame_desc_dtype(pixel_format).itemsize
     b = a + bk * OUT_DESC.itemsize
     return slice(0, a), slice(a, b), slice(b, b + 4 * bk * (L + 4))
