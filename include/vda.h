@@ -432,6 +432,57 @@ int vda_stream_step_planes(vda_model* m, const vda_frame_planes* frames, const v
                            int B, int causal, void* pool, int S, int nh, int nw, void* workspace, int64_t workspace_bytes,
                            void* stream);
 
+/* ---------------------------------------------------------------------------------------------------------------
+ * Depth frames for displays and encoders: what save_video (utils/dc_utils.py:72-86) does on the host after
+ * infer_video_depth -- normalise by a range, look up a colour table, hand uint8 frames to a writer -- on the device,
+ * with YUV 4:2:0 output for encoders (NVENC takes NV12).  The codec itself is not part of libvda.
+ *
+ * Contract, for one depth d (fp32, finite) and a range (lo, hi):
+ *   level   q = min(255, max(0, trunc(((d - lo) / (hi - lo)) * 255))), every operation IEEE fp32 round-to-nearest in
+ *           this order: the reference's ((depth - d_min) / (d_max - d_min) * 255).astype(np.uint8) on float32 arrays for
+ *           every d in [lo, hi]; the clamp matters only for a fixed range.  hi <= lo: q = 0 everywhere (a constant video).
+ *   colour  (R, G, B) = table[q], table uint8 [256][3] (OpenCV's inferno, or the caller's own, e.g. matplotlib's).
+ *   formats VDA_PIX_RGB   packed [H0][W0][3] at plane[0], rows pitch[0] >= 3 W0 bytes apart;
+ *           VDA_PIX_GRAY  q itself, [H0][W0] at plane[0] (save_video(grayscale=True)); no table needed;
+ *           VDA_PIX_NV12 / VDA_PIX_I420: cv2.cvtColor(COLOR_RGB2YUV_I420) of the RGB frame (BT.601 limited range), with
+ *           the chroma of each 2 x 2 block taken from its top-left pixel, in this integer form (equal to cv2 4.13 on all
+ *           2^24 triples):
+ *             Y = (269484 R + 528482 G + 102760 B + (16 << 20) + (1 << 19)) >> 20
+ *             U = (-155188 R - 305135 G + 460324 B + (128 << 20) + (1 << 19)) >> 20
+ *             V = (460324 R - 385875 G - 74448 B + (128 << 20) + (1 << 19)) >> 20
+ *           planes as vda_frame_planes (NV12: Y, interleaved UV; I420: Y, U, V); H0, W0 even.  Every plane has its own
+ *           pitch, so an encoder surface with its UV plane at Y + pitch * aligned height is written in place.
+ */
+enum { VDA_PIX_RGB = 0, VDA_PIX_GRAY = 3 };
+
+/* An output frame of vda_colorize_depth: vda_frame_planes with writable planes (64 bytes).  H0 == 0 (a pad row) writes
+ * nothing; otherwise H0 x W0 equals the size of the row's depth descriptor, format is a VDA_PIX_*, reserved 0. */
+typedef struct vda_color_planes {
+  uint8_t* plane[3];
+  int64_t pitch[3];
+  int32_t H0, W0, format, reserved;
+} vda_color_planes;
+
+/* The range of the depths (save_video's frames.min(), frames.max()): rows are depth frames fp32 [H0][W0] (vda_out_desc,
+ * the descriptors vda_stream_step writes through; H0 == 0 is an empty row), in device memory.  all_rows == 0: range
+ * fp32 [n][2] = (min, max) of each row ("frame" range; an empty row gives (+inf, -inf)); all_rows != 0: range fp32 [2]
+ * over every row ("video" range).  min and max are exact, so the result does not depend on the order.  scratch: device,
+ * 8-byte aligned, >= vda_depth_range_scratch_bytes(n) = n * VDA_RANGE_PARTIALS * 8 bytes.  Two launches; no allocation
+ * and no synchronisation (graph-capturable).  A range over several calls: the all-rows range of a [k][2] array of ranges
+ * (one row of H0 = k, W0 = 2) is their combined range, since every lo <= its hi. */
+#define VDA_RANGE_PARTIALS 128
+int64_t vda_depth_range_scratch_bytes(int n);
+int vda_depth_range(const vda_out_desc* rows, int n, int all_rows, float* range, void* scratch, void* stream);
+
+/* Colour-map depth frames (dc_utils.py:72-86, the frame loop of save_video): row i reads the depths of src[i] and writes
+ * its frame described by dst[i] (both descriptor arrays in device memory, read by the kernel) with the range
+ * range[2i..2i+1] (range_per_row != 0) or range[0..1] (a shared range), fp32 device memory, e.g. from vda_depth_range.
+ * table: device uint8 [256][3]; may be NULL only when every row is VDA_PIX_GRAY.  One launch, a thread per 2 x 2 pixel
+ * block; reads 4 bytes and writes 1 (grey), 1.5 (YUV) or 3 (RGB) bytes per pixel.  The descriptors are not checked by
+ * the launcher (the Python mirror checks what it writes: windows.color_descriptors). */
+int vda_colorize_depth(const vda_out_desc* src, const vda_color_planes* dst, int n, const float* range, int range_per_row,
+                       const uint8_t* table, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

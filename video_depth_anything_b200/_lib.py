@@ -13,7 +13,7 @@ VDA_BF16, VDA_FP16 = 0, 1
 ACT_NONE, ACT_GELU, ACT_RELU = 0, 1, 2
 EPI_LINEAR, EPI_GEGLU, EPI_CONVT, EPI_TAIL = 0, 1, 2, 3
 A_PLAIN, A_CONV3 = 0, 1
-PIX_NV12, PIX_I420 = 1, 2                  # vda_frame_planes.format (VDA_PIX_*)
+PIX_RGB, PIX_NV12, PIX_I420, PIX_GRAY = 0, 1, 2, 3   # vda_frame_planes / vda_color_planes .format (VDA_PIX_*)
 
 
 class VdaError(RuntimeError):
@@ -103,6 +103,9 @@ _SIGS = {
                                   C.c_int, C.c_int, C.c_void_p, C.c_int64, C.c_void_p]),
     "vda_stream_step_planes": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_int,
                                          C.c_int, C.c_int, C.c_void_p, C.c_int64, C.c_void_p]),
+    "vda_depth_range_scratch_bytes": (C.c_int64, [C.c_int]),
+    "vda_depth_range": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "vda_colorize_depth": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p]),
     "vda_affine_clamp_blend": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int64,
                                          C.c_void_p]),
 }

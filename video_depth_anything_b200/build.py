@@ -8,7 +8,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libvda.so")
-SOURCES = ["capi.cu", "gemm.cu", "attention.cu", "attention_spatial.cu", "norms.cu", "resample.cu", "align.cu", "tail.cu", "preprocess.cu", "evaluate.cu", "model.cu", "stream_plan.cu"]
+SOURCES = ["capi.cu", "gemm.cu", "attention.cu", "attention_spatial.cu", "norms.cu", "resample.cu", "align.cu", "tail.cu", "preprocess.cu", "evaluate.cu", "model.cu", "stream_plan.cu", "colorize.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
               "--use_fast_math", "-Xcompiler", "-fPIC", "-Xcompiler", "-O3"]
 

@@ -15,7 +15,8 @@ from . import _lib
 from ._lib import check
 from .ops import dt_code
 from .video_depth import check_yuv_frame, yuv_source
-from .windows import group_block_layout, group_descriptors, pixel_format_code
+from .windows import (color_args, color_descriptors, color_frame_shape, group_block_layout, group_color_layout,
+                      group_descriptors, pixel_format_code)
 
 
 class CModel:
@@ -143,11 +144,16 @@ class CStreamGroup:
     uint8 CUDA frames: {handle: frame [H0,W0,3] or stack [k,H0,W0,3]} (or pairs) -> {handle: fresh fp32 CUDA depth [H0,W0]
     or [k,H0,W0]}.  Frames are read in place (rows may be pitched).  `graphs=False` runs every step eagerly.
     `pixel_format` "nv12" | "i420": YUV 4:2:0 CUDA frames (packed [3*H0/2, W0] or plane tuples, the CUDA forms of
-    DepthStreamGroup.push) through vda_frame_planes descriptors and vda_stream_step_planes."""
+    DepthStreamGroup.push) through vda_frame_planes descriptors and vda_stream_step_planes.
+    `output_format` "rgb" | "gray" | "nv12" | "i420" (with `colormap`, `value_range`): fresh uint8 CUDA frames of that
+    format instead of depths, the depths going to a device arena; vda_depth_range (for the "frame" range) and
+    vda_colorize_depth run after the step inside the same graph."""
 
     def __init__(self, model: CModel, max_streams: int = 8, input_size: int = 518, max_frames: Optional[int] = None,
-                 graphs: bool = True, pixel_format: str = "rgb"):
+                 graphs: bool = True, pixel_format: str = "rgb", output_format: str = "depth", colormap="inferno",
+                 value_range="frame"):
         pixel_format_code(pixel_format)
+        self.color = color_args(output_format, colormap, value_range, allow_video=False)
         self.pixel_format = pixel_format
         self.model, self.lib, self.device = model, model.lib, model.device
         self.plan = CStreamPlan(max_streams, model.num_frames, input_size, max_frames)
@@ -168,21 +174,40 @@ class CStreamGroup:
         self.ws_bytes = self.lib.vda_stream_workspace_bytes(h, self.plan.buckets[-1], self.nh, self.nw)
         if pool_bytes < 0 or self.ws_bytes < 0:
             raise _lib.VdaError(self.lib.vda_last_error().decode(errors="replace"))
-        nbytes = group_block_layout(self.plan.buckets[-1], self.L, self.pixel_format)[2].stop
+        bk_max = self.plan.buckets[-1]
+        nbytes = group_block_layout(bk_max, self.L, self.pixel_format)[2].stop
+        if self.color[0] is not None:
+            nbytes = group_color_layout(bk_max, self.L, self.pixel_format).stop
         with torch.cuda.device(self.device):
             self.pool = torch.empty(pool_bytes, dtype=torch.uint8, device=self.device)
             self._ws = torch.empty(self.ws_bytes + 1024, dtype=torch.uint8, device=self.device)
             self.meta_dev = torch.zeros(nbytes, dtype=torch.uint8, device=self.device)
             self.meta_host = torch.zeros(nbytes, dtype=torch.uint8).pin_memory()
+            if self.color[0] is not None:
+                _, table, rng = self.color
+                self.color_table = None if table is None else torch.from_numpy(table.copy()).to(self.device)
+                self.range_scratch = torch.empty(self.lib.vda_depth_range_scratch_bytes(bk_max), dtype=torch.uint8,
+                                                 device=self.device)
+                self.color_range = torch.tensor([[float(rng[0]), float(rng[1])]] if rng != "frame" else
+                                                [[0.0, 0.0]] * bk_max, dtype=torch.float32, device=self.device)
         self.ws = -(-self._ws.data_ptr() // 1024) * 1024          # vda_stream_step wants a 1024-byte aligned workspace
 
     def _launch(self, bk: int, causal: bool) -> None:
         fs, os_, ts = group_block_layout(bk, self.L, self.pixel_format)
         m = self.meta_dev.data_ptr()
         step = self.lib.vda_stream_step if self.pixel_format == "rgb" else self.lib.vda_stream_step_planes
+        st = torch.cuda.current_stream().cuda_stream
         check(step(self.model.handle, m + fs.start, m + os_.start, m + ts.start, bk, int(causal),
                                        self.pool.data_ptr(), self.max_streams, self.nh, self.nw, self.ws, self.ws_bytes,
-                                       torch.cuda.current_stream().cuda_stream))
+                                       st))
+        if self.color[0] is not None:
+            per_row = self.color[2] == "frame"
+            if per_row:
+                check(self.lib.vda_depth_range(m + os_.start, bk, 0, self.color_range.data_ptr(),
+                                               self.range_scratch.data_ptr(), st))
+            cs = group_color_layout(bk, self.L, self.pixel_format)
+            check(self.lib.vda_colorize_depth(m + os_.start, m + cs.start, bk, self.color_range.data_ptr(), int(per_row),
+                                              None if self.color_table is None else self.color_table.data_ptr(), st))
 
     def _step(self, bk: int, causal: bool) -> None:
         if not self.use_graphs:
@@ -192,6 +217,7 @@ class CStreamGroup:
             # a step is not idempotent (it writes the pool), so the warm-up and the capture run on pad rows (pool row -1:
             # no pool byte read or written); the push's own table is restored for the replay
             ts = group_block_layout(bk, self.L, self.pixel_format)[2]
+            end = group_color_layout(bk, self.L, self.pixel_format).stop if self.color[0] is not None else ts.stop
             self.meta_dev[ts.start:ts.start + 4 * bk].fill_(255)
             self._launch(bk, causal)                  # warm-up, outside the capture: a new network size's position table
             torch.cuda.current_stream().synchronize()
@@ -199,7 +225,7 @@ class CStreamGroup:
             with torch.cuda.graph(g, capture_error_mode="thread_local"):
                 self._launch(bk, causal)
             self.graphs[(bk, causal)] = g
-            self.meta_dev[:ts.stop].copy_(self.meta_host[:ts.stop], non_blocking=True)
+            self.meta_dev[:end].copy_(self.meta_host[:end], non_blocking=True)
         g.replay()
 
     def _check_frame(self, f):
@@ -218,11 +244,24 @@ class CStreamGroup:
         items = list(frames.items()) if isinstance(frames, dict) else list(frames)
         shapes = [self._check_frame(f) for _, f in items]
         handles = [h for h, _ in items]
+        fmt = self.color[0]
+        if fmt is not None:
+            cshapes = [color_frame_shape(h0, w0, fmt) for _, h0, w0 in shapes]     # ValueError: odd size for YUV output
         bk, table = self.plan.step(handles, [(h0, w0) for _, h0, w0 in shapes], [k or 1 for k, _, _ in shapes])
         if self.pool is None:
             self._alloc()
         with torch.cuda.device(self.device):
-            outs = [torch.empty(*((k,) if k else ()), h0, w0, dtype=torch.float32, device=self.device) for k, h0, w0 in shapes]
+            if fmt is not None:
+                # depths to a device arena (grown on demand: its addresses are in the descriptors), colour frames returned
+                n_px = sum((k or 1) * h0 * w0 for k, h0, w0 in shapes)
+                if getattr(self, "depth_arena", None) is None or self.depth_arena.numel() < n_px:
+                    self.depth_arena = torch.empty(n_px, dtype=torch.float32, device=self.device)
+                depth_base = self.depth_arena.data_ptr()
+                couts = [torch.empty(*((k,) if k else ()), *c, dtype=torch.uint8, device=self.device)
+                         for (k, _, _), c in zip(shapes, cshapes)]
+                cdst = []
+            outs = [torch.empty(*((k,) if k else ()), h0, w0, dtype=torch.float32, device=self.device)
+                    for k, h0, w0 in shapes] if fmt is None else [None] * len(shapes)
             srcs, dsts = [], []
             for (_, f), o, (k, h0, w0) in zip(items, outs, shapes):
                 for j in range(k or 1):
@@ -230,15 +269,26 @@ class CStreamGroup:
                         srcs.append(yuv_source(f, j if k else None, h0, w0, self.pixel_format) + (h0, w0))
                     else:
                         srcs.append((f[j].data_ptr(), f.stride(1), h0, w0) if k else (f.data_ptr(), f.stride(0), h0, w0))
-                    dsts.append(o.data_ptr() + 4 * j * h0 * w0)
+                    if fmt is None:
+                        dsts.append(o.data_ptr() + 4 * j * h0 * w0)
+                    else:
+                        dsts.append(depth_base)
+                        depth_base += 4 * h0 * w0
             fd, od = group_descriptors(bk, srcs, dsts, self.pixel_format)
             fs, os_, ts = group_block_layout(bk, self.L, self.pixel_format)
             mh = self.meta_host.numpy()
             mh[fs], mh[os_], mh[ts] = fd.view(np.uint8), od.view(np.uint8), table.view(np.uint8)
-            self.meta_dev[:ts.stop].copy_(self.meta_host[:ts.stop], non_blocking=True)
+            end = ts.stop
+            if fmt is not None:
+                cs = group_color_layout(bk, self.L, self.pixel_format)
+                for c, (k, h0, w0) in zip(couts, shapes):
+                    cdst += [(c.data_ptr() + j * c[0].numel() if k else c.data_ptr(), h0, w0) for j in range(k or 1)]
+                mh[cs] = color_descriptors(bk, cdst, fmt).view(np.uint8)
+                end = cs.stop
+            self.meta_dev[:end].copy_(self.meta_host[:end], non_blocking=True)
             self._step(bk, max(k or 1 for k, _, _ in shapes) > 1)
             torch.cuda.current_stream().synchronize()
-        return dict(zip(handles, outs))
+        return dict(zip(handles, outs if fmt is None else couts))
 
     def close(self) -> None:
         self.graphs = {}

@@ -15,6 +15,8 @@ from ._lib import (A_CONV3, A_PLAIN, ACT_GELU, ACT_NONE, ACT_RELU, EPI_CONVT, EP
 LSQ_MAX_PARTIALS = 592   # include/vda.h VDA_LSQ_MAX_PARTIALS
 FRAME_DESC_BYTES, OUT_DESC_BYTES = 24, 16   # sizeof(vda_frame_desc), sizeof(vda_out_desc)
 FRAME_PLANES_BYTES = 64                     # sizeof(vda_frame_planes)
+COLOR_PLANES_BYTES = 64                     # sizeof(vda_color_planes)
+RANGE_PARTIALS = 128                        # include/vda.h VDA_RANGE_PARTIALS
 LAUNCHES = 0   # number of libvda kernel launches issued (bench.py reports it as gpu_launches)
 PROFILE = None  # when a list: every op appends (name, info dict, start_event, end_event)   [bench.py / tools]
 _INFO = {}
@@ -428,6 +430,48 @@ def bilinear_f32_ragged(x: torch.Tensor, rows: torch.Tensor) -> None:
     assert x.is_contiguous() and x.dtype == torch.float32
     assert rows.dtype == torch.uint8 and rows.is_contiguous() and rows.numel() == n * OUT_DESC_BYTES
     check(lib.vda_bilinear_f32_ragged(_p(x), _p(rows), n, ih, iw, _stream()))
+    _count()
+
+
+def depth_range_scratch(n: int, device) -> torch.Tensor:
+    """Scratch of depth_range for n rows (vda_depth_range_scratch_bytes)."""
+    return torch.empty(n * RANGE_PARTIALS * 2, dtype=torch.float32, device=device)
+
+
+def depth_range(rows: torch.Tensor, all_rows: bool, out: Optional[torch.Tensor] = None,
+                scratch: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """save_video's frames.min() / frames.max() (utils/dc_utils.py:74-75) on the device: rows = vda_out_desc array (device
+    bytes [n * 16], windows.OUT_DESC) of fp32 depth frames -> fp32 [n, 2] per-row (min, max), or [2] over all rows.
+    Two launches, graph-capturable when `out` and `scratch` are given."""
+    lib = _lib.load()
+    assert rows.dtype == torch.uint8 and rows.is_contiguous() and rows.numel() % OUT_DESC_BYTES == 0
+    n = rows.numel() // OUT_DESC_BYTES
+    if out is None:
+        out = torch.empty((2,) if all_rows else (n, 2), dtype=torch.float32, device=rows.device)
+    if scratch is None:
+        scratch = depth_range_scratch(n, rows.device)
+    assert out.dtype == torch.float32 and out.is_contiguous() and out.numel() >= (2 if all_rows else 2 * n)
+    assert scratch.dtype == torch.float32 and scratch.numel() >= n * RANGE_PARTIALS * 2
+    check(lib.vda_depth_range(_p(rows), n, int(bool(all_rows)), _p(out), _p(scratch), _stream()))
+    _count(2)
+    return out
+
+
+def colorize_depth(src_rows: torch.Tensor, dst_rows: torch.Tensor, value_range: torch.Tensor, range_per_row: bool,
+                   table: Optional[torch.Tensor]) -> None:
+    """The frame loop of save_video (utils/dc_utils.py:76-86) on the device: row i's depths (vda_out_desc src_rows[i]) ->
+    its uint8 frame (vda_color_planes dst_rows[i], windows.COLOR_PLANES) with range value_range[i] (range_per_row) or
+    value_range[0] (fp32 [., 2]) and table uint8 [256, 3] (None: grey rows only).  One launch."""
+    lib = _lib.load()
+    assert src_rows.dtype == torch.uint8 and src_rows.is_contiguous() and src_rows.numel() % OUT_DESC_BYTES == 0
+    n = src_rows.numel() // OUT_DESC_BYTES
+    assert dst_rows.dtype == torch.uint8 and dst_rows.is_contiguous() and dst_rows.numel() == n * COLOR_PLANES_BYTES
+    assert value_range.dtype == torch.float32 and value_range.is_contiguous()
+    assert value_range.numel() >= (2 * n if range_per_row else 2)
+    if table is not None:
+        assert table.dtype == torch.uint8 and table.is_contiguous() and table.numel() == 768
+    check(lib.vda_colorize_depth(_p(src_rows), _p(dst_rows), n, _p(value_range), int(bool(range_per_row)), _p(table),
+                                 _stream()))
     _count()
 
 

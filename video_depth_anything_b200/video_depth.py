@@ -26,7 +26,8 @@ from . import ops
 from .engine import Engine
 from .synth import ENCODER_DIMS, synth_state_dict
 from .windows import (INFER_LEN, INTERP_LEN, KEYFRAMES, OVERLAP, aligner_ring_len, aligner_ring_pos, get_resize_hw,
-                      StreamGroupPlan, group_block_layout, group_descriptors, pixel_format_code, plan_feature_cache,
+                      StreamGroupPlan, color_args, color_descriptors, color_frame_shape, group_block_layout,
+                      group_color_layout, group_descriptors, pixel_format_code, plan_feature_cache,
                       split_group_table, upload_ring_plan, video_frame_shape, window_source_indices, yuv_frame_hw,
                       yuv_planes)
 
@@ -193,36 +194,44 @@ class VideoDepthAnything(nn.Module):
 
     # ---- streaming -----------------------------------------------------------------------------
     def stream(self, input_size: int = 518, fp32: bool = False, max_frames: int = 16,
-               pixel_format: str = "rgb") -> "DepthStream":
+               pixel_format: str = "rgb", output_format: str = "depth", colormap="inferno",
+               value_range="frame") -> "DepthStream":
         """Open a depth stream on this model's device: `push` one uint8 frame, get its depth back at once, or push a stack
         of up to `max_frames` consecutive frames and get their depths as one step.  Each frame attends to frame 0 and the
         30 frames before it (DepthStream).  Streams are independent of each other and of `forward` /
         `infer_video_depth`; `fp32=True` selects the validation-precision engine as in infer_video_depth.
-        `pixel_format` "nv12" | "i420": the stream takes YUV 4:2:0 frames (DepthStreamGroup)."""
-        return DepthStream(self, self._ensure_engine(validation=bool(fp32)), input_size, max_frames, pixel_format)
+        `pixel_format` "nv12" | "i420": the stream takes YUV 4:2:0 frames; `output_format` "rgb" | "gray" | "nv12" |
+        "i420": it returns colour-mapped uint8 frames instead of depths (DepthStreamGroup)."""
+        return DepthStream(self, self._ensure_engine(validation=bool(fp32)), input_size, max_frames, pixel_format,
+                           output_format, colormap, value_range)
 
     def stream_group(self, max_streams: int = 8, input_size: int = 518, fp32: bool = False,
-                     max_frames: Optional[int] = None, pixel_format: str = "rgb") -> "DepthStreamGroup":
+                     max_frames: Optional[int] = None, pixel_format: str = "rgb", output_format: str = "depth",
+                     colormap="inferno", value_range="frame") -> "DepthStreamGroup":
         """Open a group of up to `max_streams` depth streams (several cameras) on this model's device: each `push` takes
         one frame, or a stack of consecutive frames, of any subset of the group's open streams and runs them as one
         batched step of at most `max_frames` frames (default max(max_streams, 16); DepthStreamGroup).  Every stream
         behaves as a DepthStream of its own; `fp32=True` selects the validation-precision engine.  `pixel_format`
-        "rgb" | "nv12" | "i420" is fixed per group, as the network size is."""
+        "rgb" | "nv12" | "i420" is fixed per group, as the network size is; so are `output_format`, `colormap` and
+        `value_range` (DepthStreamGroup: colour-mapped uint8 frames instead of depths)."""
         return DepthStreamGroup(self, self._ensure_engine(validation=bool(fp32)), max_streams, input_size, max_frames,
-                                pixel_format)
+                                pixel_format, output_format, colormap, value_range)
 
     @torch.no_grad()
     def infer_video_depth_one(self, frame, input_size: int = 518, device="cuda", fp32: bool = False, to_host: bool = True,
-                              pixel_format: str = "rgb"):
+                              pixel_format: str = "rgb", output_format: str = "depth", colormap="inferno",
+                              value_range="frame"):
         """Depth of the next frame of the model's own stream (the name of the upstream project's streaming entry
         point): frame uint8 [H0,W0,3] (numpy array or CUDA tensor) -> float32 [H0,W0] (numpy array, or with
         `to_host=False` a CUDA tensor; DepthStream.push).  The stream is opened on the first call and reopened (its
         temporal context starts over) when `input_size`, `fp32`, `pixel_format` or the device change or new weights were
         loaded.  `pixel_format` "nv12" | "i420": one YUV 4:2:0 frame, packed [3*H0/2, W0] or a plane tuple
-        (DepthStreamGroup)."""
+        (DepthStreamGroup).  `output_format` "rgb" | "gray" | "nv12" | "i420" with `colormap` and `value_range`: the
+        frame's colour-mapped uint8 frame instead of its depth (a change of these also reopens the stream)."""
         if torch.device(device).type != "cuda":
             raise RuntimeError("infer_video_depth_one: the B200 engine has no CPU path (device must be 'cuda')")
         pixel_format_code(pixel_format)
+        color = color_args(output_format, colormap, value_range, allow_video=False)
         if pixel_format == "rgb" and getattr(frame, "ndim", None) != 3:
             raise ValueError("infer_video_depth_one takes one frame uint8 [H0,W0,3]; push stacks through model.stream()")
         if pixel_format != "rgb" and not (getattr(frame, "ndim", None) == 2 or
@@ -233,11 +242,18 @@ class VideoDepthAnything(nn.Module):
         eng = self._ensure_engine(validation=bool(fp32))
         st = self._stream_one
         if st is None or st.engine is not eng or st.input_size != input_size or st.generation != eng.generation or \
-                st.pixel_format != pixel_format:
+                st.pixel_format != pixel_format or not _same_color(st.group.color, color):
             if st is not None:
                 st.close()
-            st = self._stream_one = self.stream(input_size, fp32, pixel_format=pixel_format)
+            st = self._stream_one = self.stream(input_size, fp32, pixel_format=pixel_format, output_format=output_format,
+                                                colormap=colormap, value_range=value_range)
         return st.push(frame, to_host)
+
+
+def _same_color(a, b) -> bool:
+    """Whether two windows.color_args results are the same colour mapping."""
+    return a[0] == b[0] and a[2] == b[2] and (a[1] is b[1] or a[1] is not None and b[1] is not None and
+                                              np.array_equal(a[1], b[1]))
 
 
 def check_yuv_frame(f, fmt: str, device, L: int, host: bool = True):
@@ -334,11 +350,23 @@ class DepthStreamGroup:
     max_frames (windows.stream_buckets).  A push that gives any stream k > 1 frames replays the bucket's causal graph
     (captured once per bucket, kept in `causal_graphs`): its temporal attention reads a frame's newer context from the
     push's own rows and writes the cache afterwards (Engine.stream_group_step(causal=True)); any other push replays
-    today's graph."""
+    today's graph.
+
+    Frames for displays and encoders: with `output_format` "rgb" | "gray" | "nv12" | "i420" a push returns each frame's
+    colour-mapped uint8 frame instead of its depth -- [H0, W0, 3], [H0, W0] or [3*H0/2, W0] in OpenCV's packed layout,
+    with a leading k for a stack -- as the display.colorize contract defines it (table `colormap`; `value_range` "frame":
+    each frame's own min / max, or a fixed (lo, hi)).  The depths then go to a device arena, and the range (2 launches,
+    none for a fixed range) and colour (1 launch) kernels run in the same graph as the step, reading a fourth section of
+    the push's metadata block (windows.group_color_layout).  A host output is 1 (grey), 1.5 (YUV) or 3 (RGB) bytes per
+    pixel on the way down instead of 4.  The default "depth" is the depth path unchanged."""
 
     def __init__(self, model: VideoDepthAnything, engine: Engine, max_streams: int = 8, input_size: int = 518,
-                 max_frames: Optional[int] = None, pixel_format: str = "rgb"):
+                 max_frames: Optional[int] = None, pixel_format: str = "rgb", output_format: str = "depth",
+                 colormap="inferno", value_range="frame"):
         pixel_format_code(pixel_format)                  # ValueError for an unknown format
+        # ValueError: unknown output format, bad table, "video" range (no meaning for a live stream), hi <= lo
+        self.color = color_args(output_format, colormap, value_range, allow_video=False)
+        self.output_format = output_format
         self.pixel_format = pixel_format
         self.engine, self.input_size = engine, int(input_size)
         self.device = engine.device
@@ -367,11 +395,20 @@ class DepthStreamGroup:
     def _alloc(self) -> None:
         eng, S, L = self.engine, self.max_streams, self.plan.L
         self.nh, self.nw = self.plan.net
-        nbytes = group_block_layout(self.plan.buckets[-1], L, self.pixel_format)[2].stop
+        bk_max = self.plan.buckets[-1]
+        nbytes = group_block_layout(bk_max, L, self.pixel_format)[2].stop
+        if self.color[0] is not None:
+            nbytes = group_color_layout(bk_max, L, self.pixel_format).stop
         with torch.cuda.device(self.device):
             self.pool = eng.stream_pool(S, self.nh // 14, self.nw // 14, L + 1)
             self.meta_dev = torch.zeros(nbytes, dtype=torch.uint8, device=self.device)
             self.meta_host = torch.zeros(nbytes, dtype=torch.uint8).pin_memory()
+            if self.color[0] is not None:
+                _, table, rng = self.color
+                self.color_table = None if table is None else torch.from_numpy(table.copy()).to(self.device)
+                self.range_scratch = ops.depth_range_scratch(bk_max, self.device)
+                self.color_range = torch.tensor([[float(rng[0]), float(rng[1])]] if rng != "frame" else
+                                                [[0.0, 0.0]] * bk_max, dtype=torch.float32, device=self.device)
 
     def _arena(self, name: str, n: int, dtype, pinned: bool) -> torch.Tensor:
         """Buffer `name` with at least n elements; regrown (in 2 MiB steps) only when a push needs more."""
@@ -389,8 +426,15 @@ class DepthStreamGroup:
         inputs = [self.meta_dev[fs], self.meta_dev[os_], rows, ctx]
         planes = self.pixel_format != "rgb"
 
-        def fn(frame_desc, out_desc, rows, ctx):
-            return eng.stream_group_step(frame_desc, out_desc, rows, ctx, self.pool, self.nh, self.nw, causal, planes)
+        def fn(frame_desc, out_desc, rows, ctx, *color_desc):
+            eng.stream_group_step(frame_desc, out_desc, rows, ctx, self.pool, self.nh, self.nw, causal, planes)
+            if color_desc:
+                per_row = self.color[2] == "frame"
+                if per_row:
+                    ops.depth_range(out_desc, False, self.color_range, self.range_scratch)
+                ops.colorize_depth(out_desc, color_desc[0], self.color_range, per_row, self.color_table)
+        if self.color[0] is not None:
+            inputs.append(self.meta_dev[group_color_layout(bk, self.plan.L, self.pixel_format)])
         if eng.use_graphs and ops.PROFILE is None:
             return eng.run_graphed(self.causal_graphs if causal else self.graphs, bk, fn, inputs, adopt=True)
         return fn(*inputs)
@@ -421,7 +465,9 @@ class DepthStreamGroup:
         """frames: {handle: uint8 RGB [H0,W0,3] numpy array or CUDA tensor, or a stack [k,H0,W0,3] of k consecutive
         frames} (or (handle, frame) pairs) -> {handle: depth [H0,W0] (>= 0), or [k,H0,W0] for a stack}: fresh float32
         numpy arrays, or with `to_host=False` fresh float32 CUDA tensors on the group's device (no device-to-host copy).
-        Returns after the step has finished, so the caller may reuse its frame buffers at once."""
+        With an `output_format` other than "depth", fresh uint8 frames of that format instead (windows.color_frame_shape,
+        with a leading k for a stack).  Returns after the step has finished, so the caller may reuse its frame buffers at
+        once."""
         if self.closed:
             raise RuntimeError("push on a closed DepthStreamGroup")
         if self.engine.generation != self.generation or not self.engine.loaded:
@@ -431,6 +477,9 @@ class DepthStreamGroup:
         sizes = [(h0, w0) for _, h0, w0 in shapes]
         counts = [k or 1 for k, _, _ in shapes]
         handles = [h for h, _ in items]
+        fmt = self.color[0]
+        if fmt is not None:
+            cshapes = [color_frame_shape(h0, w0, fmt) for h0, w0 in sizes]   # ValueError: odd size for YUV output
         # ValueError: empty push, unknown / closed / repeated handle, a frame size the group cannot take, too many frames
         bk, table = self.plan.step(handles, sizes, counts)
         if self.pool is None:
@@ -470,7 +519,21 @@ class DepthStreamGroup:
                     srcs.append((f[j].data_ptr(), f.stride(1), h0, w0) if f.dim() == 4 else (f.data_ptr(), f.stride(0), h0, w0))
                 else:
                     srcs.append((in_dev.data_ptr() + in_off[r], 3 * w0, h0, w0))
-            if to_host:
+            if fmt is not None:
+                # depths to the device arena; the colour frames packed in an arena (to_host) or in the returned tensors
+                out_dev = self._arena("depth_dev", out_elems, torch.float32, False)
+                dsts = [out_dev.data_ptr() + 4 * o for o in out_off[:-1]]
+                csize = [int(np.prod(c)) for c in cshapes]
+                col_off = np.cumsum([0] + [csize[i] for i, _, _, _ in rows]).tolist()
+                if to_host:
+                    col_dev = self._arena("color_dev", col_off[-1], torch.uint8, False)
+                    cdst = [col_dev.data_ptr() + o for o in col_off[:-1]]
+                else:
+                    outs = [torch.empty(*((k,) if k else ()), *c, dtype=torch.uint8, device=self.device)
+                            for (k, _, _), c in zip(shapes, cshapes)]
+                    cdst = [outs[i].data_ptr() + j * csize[i] for i, j, _, _ in rows]
+                cd = color_descriptors(bk, [(a, h0, w0) for a, (_, _, h0, w0) in zip(cdst, rows)], fmt)
+            elif to_host:
                 out_dev = self._arena("out_dev", out_elems, torch.float32, False)
                 dsts = [out_dev.data_ptr() + 4 * o for o in out_off[:-1]]
             else:
@@ -483,9 +546,14 @@ class DepthStreamGroup:
             fs, os_, ts = group_block_layout(bk, self.plan.L, self.pixel_format)
             mh = self.meta_host.numpy()
             mh[fs], mh[os_], mh[ts] = fd.view(np.uint8), od.view(np.uint8), table.view(np.uint8)
+            meta_end = ts.stop
+            if fmt is not None:
+                cs = group_color_layout(bk, self.plan.L, self.pixel_format)
+                mh[cs] = cd.view(np.uint8)
+                meta_end = cs.stop
             if host:
                 in_dev[:in_bytes].copy_(in_host[:in_bytes], non_blocking=True)
-            self.meta_dev[:ts.stop].copy_(self.meta_host[:ts.stop], non_blocking=True)
+            self.meta_dev[:meta_end].copy_(self.meta_host[:meta_end], non_blocking=True)
             causal = max(counts) > 1
             if causal and bk not in self.causal_graphs and self.engine.use_graphs and ops.PROFILE is None:
                 # capturing runs the step twice (warm-up, then the replay), and a causal step is not idempotent: its
@@ -493,14 +561,21 @@ class DepthStreamGroup:
                 # (pool row -1: no pool byte read or written), then the push's own table replays the new graph.
                 self.meta_dev[ts.start:ts.start + 4 * bk].fill_(255)
                 self._step(bk, causal)
-                self.meta_dev[:ts.stop].copy_(self.meta_host[:ts.stop], non_blocking=True)
+                self.meta_dev[:meta_end].copy_(self.meta_host[:meta_end], non_blocking=True)
             self._step(bk, causal)
-            if to_host:
+            if to_host and fmt is not None:
+                col_host = self._arena("color_host", col_off[-1], torch.uint8, True)
+                col_host[:col_off[-1]].copy_(col_dev[:col_off[-1]], non_blocking=True)
+            elif to_host:
                 out_host = self._arena("out_host", out_elems, torch.float32, True)
                 out_host[:out_elems].copy_(out_dev[:out_elems], non_blocking=True)
             torch.cuda.current_stream().synchronize()   # (also: the pinned arenas are free for the next push)
         if not to_host:
             return dict(zip(handles, outs))
+        if fmt is not None:
+            ch = col_host.numpy()
+            return {h: ch[col_off[first[i]]:col_off[first[i + 1]]].reshape(((k,) if k else ()) + cshapes[i]).copy()
+                    for i, (h, (k, _, _)) in enumerate(zip(handles, shapes))}
         oh = out_host.numpy()
         return {h: oh[out_off[first[i]]:out_off[first[i + 1]]].reshape(((k,) if k else ()) + sizes[i]).copy()
                 for i, (h, (k, _, _)) in enumerate(zip(handles, shapes))}
@@ -543,8 +618,9 @@ class DepthStream:
     would have returned (DepthStreamGroup)."""
 
     def __init__(self, model: VideoDepthAnything, engine: Engine, input_size: int = 518, max_frames: int = 16,
-                 pixel_format: str = "rgb"):
-        self.group = DepthStreamGroup(model, engine, 1, input_size, max_frames, pixel_format)
+                 pixel_format: str = "rgb", output_format: str = "depth", colormap="inferno", value_range="frame"):
+        self.group = DepthStreamGroup(model, engine, 1, input_size, max_frames, pixel_format, output_format, colormap,
+                                      value_range)
         self.engine, self.input_size, self.generation = engine, self.group.input_size, self.group.generation
         self.pixel_format = pixel_format
         self.handle = self.group.open()

@@ -381,3 +381,115 @@ def group_block_layout(bk: int, L: int = STREAM_CONTEXT, pixel_format: str = "rg
     a = bk * frame_desc_dtype(pixel_format).itemsize
     b = a + bk * OUT_DESC.itemsize
     return slice(0, a), slice(a, b), slice(b, b + 4 * bk * (L + 4))
+
+
+# ------------------------------------------------------------------------------------------------
+# depth frames for displays and encoders (vda_depth_range / vda_colorize_depth; utils/dc_utils.py:72-86 save_video)
+# ------------------------------------------------------------------------------------------------
+# OpenCV's COLORMAP_INFERNO as RGB, uint8 [256, 3]: cv2.applyColorMap(np.arange(256, dtype=np.uint8)[None],
+# cv2.COLORMAP_INFERNO)[0, :, ::-1] (tests/test_colorize_cpu.py checks it).  matplotlib's table, which the reference
+# truncates where cv2 rounds, differs by up to one level per channel; pass it as a table to reproduce the reference.
+_INFERNO_HEX = (
+    "00000401000501010601010802010a02020c02020e03021004031204031405041706041907051b08051d09061f0a0722"
+    "0b07240c08260d08290e092b10092d110a30120a32140b34150b37160b39180c3c190c3e1b0c411c0c431e0c451f0c48"
+    "210c4a230c4c240c4f260c51280b53290b552b0b572d0b592f0a5b310a5c320a5e340a5f3609613809623909633b0964"
+    "3d09653e0966400a67420a68440a68450a69470b6a490b6a4a0c6b4c0c6b4d0d6c4f0d6c510e6c520e6d540f6d550f6d"
+    "57106e59106e5a116e5c126e5d126e5f136e61136e62146e64156e65156e67166e69166e6a176e6c186e6d186e6f196e"
+    "71196e721a6e741a6e751b6e771c6d781c6d7a1d6d7c1d6d7d1e6d7f1e6c801f6c82206c84206b85216b87216b88226a"
+    "8a226a8c23698d23698f24699025689225689326679526679727669827669a28659b29649d29649f2a63a02a63a22b62"
+    "a32c61a52c60a62d60a82e5fa92e5eab2f5ead305dae305cb0315bb1325ab3325ab43359b63458b73557b93556ba3655"
+    "bc3754bd3853bf3952c03a51c13a50c33b4fc43c4ec63d4dc73e4cc83f4bca404acb4149cc4248ce4347cf4446d04545"
+    "d24644d34743d44842d54a41d74b3fd84c3ed94d3dda4e3cdb503bdd513ade5238df5337e05536e15635e25734e35933"
+    "e45a31e55c30e65d2fe75e2ee8602de9612bea632aeb6429eb6628ec6726ed6925ee6a24ef6c23ef6e21f06f20f1711f"
+    "f1731df2741cf3761bf37819f47918f57b17f57d15f67e14f68013f78212f78410f8850ff8870ef8890cf98b0bf98c0a"
+    "f98e09fa9008fa9207fa9407fb9606fb9706fb9906fb9b06fb9d07fc9f07fca108fca309fca50afca60cfca80dfcaa0f"
+    "fcac11fcae12fcb014fcb216fcb418fbb61afbb81dfbba1ffbbc21fbbe23fac026fac228fac42afac62df9c72ff9c932"
+    "f9cb35f8cd37f8cf3af7d13df7d340f6d543f6d746f5d949f5db4cf4dd4ff4df53f4e156f3e35af3e55df2e661f2e865"
+    "f2ea69f1ec6df1ed71f1ef75f1f179f2f27df2f482f3f586f3f68af4f88ef5f992f6fa96f8fb9af9fc9dfafda1fcffa4"
+)
+INFERNO = np.frombuffer(bytes.fromhex("".join(_INFERNO_HEX)), dtype=np.uint8).reshape(256, 3)
+INFERNO.flags.writeable = False
+
+# output formats of colour-mapped depth frames (VDA_PIX_*); "depth" is the fp32 depth itself
+OUTPUT_FORMATS = {"depth": None, "rgb": 0, "nv12": 1, "i420": 2, "gray": 3}
+# include/vda.h vda_color_planes: vda_frame_planes with writable planes (64 bytes)
+COLOR_PLANES = FRAME_PLANES
+
+
+def color_args(output_format: str = "rgb", colormap="inferno", value_range="video", allow_video: bool = True):
+    """Checked colour-mapping arguments -> (format code or None for "depth", uint8 [256, 3] table or None, range) with range
+    "video" | "frame" | (lo, hi) as float32 values.  ValueError for an unknown format, a bad table (anything but
+    "inferno" or a uint8 [256, 3] array), a table with "gray", "video" where it has no meaning, or a fixed range with
+    hi <= lo."""
+    if output_format not in OUTPUT_FORMATS:
+        raise ValueError(f"output format must be one of {sorted(OUTPUT_FORMATS)}, got {output_format!r}")
+    fmt = OUTPUT_FORMATS[output_format]
+    if isinstance(colormap, str):
+        if colormap != "inferno":
+            raise ValueError(f"the built-in colormap is 'inferno'; pass any other as a uint8 [256, 3] table, got {colormap!r}")
+        table = None if fmt == 3 else INFERNO
+    elif colormap is None and fmt == 3:
+        table = None
+    else:
+        if hasattr(colormap, "detach"):                               # a torch tensor
+            colormap = colormap.detach().cpu().numpy()
+        if not isinstance(colormap, np.ndarray) or colormap.dtype != np.uint8 or colormap.shape != (256, 3):
+            raise ValueError(f"a colour table is uint8 [256, 3] (RGB per level), got "
+                             f"{getattr(colormap, 'dtype', type(colormap).__name__)} {tuple(getattr(colormap, 'shape', ()))}")
+        if fmt == 3:
+            raise ValueError("output format 'gray' writes the 8-bit level itself and takes no colour table")
+        table = np.array(colormap, order="C")                        # a copy: later edits of the caller's do not leak in
+    if isinstance(value_range, str):
+        if value_range not in ("video", "frame"):
+            raise ValueError(f"value_range is 'video', 'frame' or a fixed (lo, hi), got {value_range!r}")
+        if value_range == "video" and not allow_video:
+            raise ValueError("value_range 'video' (one range over all frames) has no meaning for a live stream; "
+                             "use 'frame' or a fixed (lo, hi)")
+        rng = value_range
+    else:
+        try:
+            lo, hi = (np.float32(v) for v in value_range)
+        except (TypeError, ValueError):
+            raise ValueError(f"value_range is 'video', 'frame' or a fixed (lo, hi), got {value_range!r}") from None
+        if not (np.isfinite(lo) and np.isfinite(hi) and hi > lo):
+            raise ValueError(f"a fixed value_range needs finite lo < hi, got {(float(lo), float(hi))}")
+        rng = (lo, hi)
+    return fmt, (None if fmt is None else table), rng
+
+
+def color_frame_shape(h0: int, w0: int, fmt: int):
+    """Shape of one colour-mapped frame of an H0 x W0 depth: RGB [H0, W0, 3], grey [H0, W0], NV12 / I420 packed in
+    OpenCV's layout [3*H0/2, W0]; ValueError for an odd size with a YUV format."""
+    if fmt == 0:
+        return (h0, w0, 3)
+    if fmt == 3:
+        return (h0, w0)
+    if h0 % 2 or w0 % 2:
+        raise ValueError(f"{'nv12' if fmt == 1 else 'i420'} output needs an even frame size, got {h0}x{w0}")
+    return (3 * h0 // 2, w0)
+
+
+def color_descriptors(bk: int, dsts, fmt: int):
+    """COLOR_PLANES [bk] of frames packed in their color_frame_shape at device addresses dsts = [(address, H0, W0)] (real
+    rows in batch-row order); pad rows are all zero (H0 = 0: nothing written)."""
+    if not 1 <= len(dsts) <= bk:
+        raise ValueError(f"{len(dsts)} outputs for a bucket of {bk}")
+    cd = np.zeros(bk, COLOR_PLANES)
+    for i, (base, h0, w0) in enumerate(dsts):
+        color_frame_shape(h0, w0, fmt)
+        if fmt == 0:
+            planes, pitches = (base, 0, 0), (3 * w0, 0, 0)
+        elif fmt == 3:
+            planes, pitches = (base, 0, 0), (w0, 0, 0)
+        else:
+            planes, pitches = yuv_planes(base, w0, h0, w0, "nv12" if fmt == 1 else "i420")
+        cd[i] = (planes, pitches, h0, w0, fmt, 0)
+    return cd
+
+
+def group_color_layout(bk: int, L: int = STREAM_CONTEXT, pixel_format: str = "rgb"):
+    """Byte range of the colour descriptors (COLOR_PLANES [bk]) of a push with an output format other than "depth": one
+    more section of the metadata block, behind group_block_layout's (whose ranges it leaves as they are), 64-byte
+    aligned."""
+    a = -(-group_block_layout(bk, L, pixel_format)[2].stop // 64) * 64
+    return slice(a, a + bk * COLOR_PLANES.itemsize)
